@@ -32,6 +32,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark may run from a read-only tree and leaves it as it found it: no __pycache__ here or in worker processes
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 from physher_b200 import models, synthetic as syn  # noqa: E402
 
@@ -573,9 +576,10 @@ def roofline_record(name, cfg, P, B, kms, kernels, lib_version, cherries=0):
     return hbm
 
 
-def run_config(run, name, cfg, K, W, kernels="auto", strong=False, full_cpu_baseline=False, gate=True):
+def run_config(run, name, cfg, K, W, kernels="auto", strong=False, full_cpu_baseline=False, gate=True, outputs=None):
     """One BASELINE config on this invocation's GPUs: device-resident throughput, end-to-end throughput through the C ABI with host
-    buffers, the live kernel time for the roofline, clocks, and the parity gate against the reference on a bounded sample."""
+    buffers, the live kernel time for the roofline, clocks, and the parity gate against the reference on a bounded sample.
+    outputs[name] receives the arrays the last timed end-to-end step returned to its caller."""
     torch = run.torch
     from physher_b200.treelikelihood import OPT_TIMING
 
@@ -622,6 +626,7 @@ def run_config(run, name, cfg, K, W, kernels="auto", strong=False, full_cpu_base
     tlk = build_tlk(run, cfg, topo, m, rates, props, patterns, weights, kernels)
     ext = torch.cuda.ExternalStream(tlk.stream(), device=torch.device("cuda", run.local_rank))
     rng = np.random.default_rng(7)
+    last = {}
 
     def new_bl():
         # every step sees new branch lengths (host buffer), like an optimiser / VI iteration would produce; the same on every rank
@@ -637,6 +642,7 @@ def run_config(run, name, cfg, K, W, kernels="auto", strong=False, full_cpu_base
         bls[:, topo.root] = 0.0
         bls[:, topo.right[topo.root]] = 0.0
         lnls, grads = tlk.gradient_batch(bls)
+        last.update(lnl=lnls, grad=grads)
         return float(lnls[-1]), grads[-1]
 
     def step_e2e():
@@ -647,8 +653,11 @@ def run_config(run, name, cfg, K, W, kernels="auto", strong=False, full_cpu_base
         tlk.set_branch_lengths(new_bl())
         if world == 1:
             g = tlk.gradient()
-            return tlk.calculate(), g
-        return tlk.gradient_allreduce(run.comm)
+            lnl = tlk.calculate()
+        else:
+            lnl, g = tlk.gradient_allreduce(run.comm)
+        last.update(lnl=lnl, grad=g)
+        return lnl, g
 
     def step_device():
         """Device-resident step: inputs already in HBM, the (reduced) result left on the device; nothing waits on the host."""
@@ -708,15 +717,18 @@ def run_config(run, name, cfg, K, W, kernels="auto", strong=False, full_cpu_base
         "l2": "per-evaluation working set exceeds the 126 MB L2; no explicit flush",
     })
     tlk.close()
+    if outputs is not None:
+        outputs[name] = last
     return rec
 
 
-def run_c1(run, K, W):
+def run_c1(run, K, W, outputs=None):
     """BASELINE config 1 (examples/fluA JC69 strict-clock time tree: 69 taxa x 238 patterns, one rate category): a LATENCY workload.
     (a) single lnL + gradient evaluations through the C ABI with host buffers (what the glue does per model->logP / dlogP);
     (b) the ELBO shape of examples/fluA/JC69-time-ELBO.json: 100 reparameterised tree samples per step through
         phb_tlk_gradient_batch_time (heights, branch lengths, one fused launch, ratio / root-height / clock gradients).
-    The reference's own known answers (tests/test_tree_likelihood.c:28-116, tests/golden/c1_kat.json) gate the record."""
+    The reference's own known answers (tests/test_tree_likelihood.c:28-116, tests/golden/c1_kat.json) gate the record.
+    outputs["c1"] receives what the last timed call of (a) and of (b) returned."""
     phb = run.phb
     gold = os.path.join(ROOT, "tests", "golden")
     z = dict(np.load(os.path.join(gold, "c1_jc69_fluA_tipstates.npz")))
@@ -766,7 +778,7 @@ def run_c1(run, K, W):
     with ClockSampler(run.local_rank) as clocks:
         t0 = time.perf_counter()
         for _ in range(n_single):
-            single()
+            l0, g0 = single()
         tlk.synchronize()
         single_ms = (time.perf_counter() - t0) * 1e3 / n_single
         launches = (tlk.launch_count() - launches0) / (n_single + max(W, 10))
@@ -779,7 +791,7 @@ def run_c1(run, K, W):
             tlk.gradient_batch_time(ratios, rates, include_jacobian=True)
         t0 = time.perf_counter()
         for _ in range(K):
-            lb, _, _, _ = tlk.gradient_batch_time(ratios, rates, include_jacobian=True)
+            lb, ljb, grb, gcb = tlk.gradient_batch_time(ratios, rates, include_jacobian=True)
         batch_ms = (time.perf_counter() - t0) * 1e3 / K
     pn = float(P) * N
     rec.update({
@@ -794,6 +806,8 @@ def run_c1(run, K, W):
         "roofline": {"bound": "latency", "note": "23 kB of tip codes and 137 nodes: launch + copy latency bound, no bandwidth roofline applies"},
     })
     tlk.close()
+    if outputs is not None:
+        outputs["c1"] = dict(lnl=l0, grad=g0, elbo_lnl=lb, elbo_log_jacobian=ljb, elbo_grad_ratios=grb, elbo_grad_rates=gcb)
     try:  # cpu_baseline leg: the reference's own evaluation of the same fixture on one host core
         from oracle import oracle as O
 
@@ -817,6 +831,15 @@ def run_c1(run, K, W):
     return rec
 
 
+def dump_outputs(path, outputs):
+    """outputs {config: {array: values}} -> path/<config>_<array>.npy in float64.  Inputs are seeded, so two builds run with the same
+    arguments can be compared output for output.  Everything is per node or per sample (1.1 MB in all for the default records)."""
+    os.makedirs(path, exist_ok=True)
+    for config, arrays in outputs.items():
+        for key, a in arrays.items():
+            np.save(os.path.join(path, f"{config}_{key}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -826,12 +849,18 @@ def main():
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS), help="headline workload (default: BASELINE configs[1])")
     ap.add_argument("--sub", default=None, help="comma list of further configs reported as sub-records under `configs` "
                                                 "(default: all of c1,c2_1m,c3,c4,c5 for the default headline; 'none' to skip)")
-    ap.add_argument("--sub-steps", type=int, default=5)
+    ap.add_argument("--sub-steps", type=int, default=None, help="timed steps of each sub-record (default: --steps)")
     ap.add_argument("--patterns", type=int, default=0, help="override patterns per GPU of the headline workload")
     ap.add_argument("--kernels", default="auto", choices=["auto", "generic", "fused"])
     ap.add_argument("--strong", action="store_true", help="headline: split --config's patterns over the GPUs instead of weak scaling")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of every record returned (lnL, gradients) as DIR/<config>_<array>.npy, float64")
     args = ap.parse_args()
+    if args.sub_steps is None:
+        args.sub_steps = args.steps
+    if args.steps < 1 or args.sub_steps < 1:
+        ap.error("--steps and --sub-steps must be at least 1")
     cfg = dict(CONFIGS[args.config])
     if args.patterns:
         cfg["patterns"] = args.patterns
@@ -840,8 +869,9 @@ def main():
 
     run = Run()
     W, K = max(args.warmup, 3), args.steps
+    outputs = {}
     head = run_config(run, args.config, cfg, K, W, kernels=args.kernels, strong=args.strong, full_cpu_baseline=(run.world == 1),
-                      gate=not args.no_cpu_baseline)
+                      gate=not args.no_cpu_baseline, outputs=outputs)
     if args.sub is None:
         subs = SUB_CONFIGS if (args.config == "c2" and not args.patterns and args.kernels == "auto") else []
     else:
@@ -852,16 +882,19 @@ def main():
         try:
             if name == "c1":
                 if run.rank == 0:
-                    records[name] = run_c1(run, max(args.sub_steps, 5), W)
+                    records[name] = run_c1(run, args.sub_steps, W, outputs=outputs)
                 run.sync()
             else:
-                records[name] = run_config(run, name, dict(CONFIGS[name]), args.sub_steps, W, strong=True, gate=not args.no_cpu_baseline)
+                records[name] = run_config(run, name, dict(CONFIGS[name]), args.sub_steps, W, strong=True, gate=not args.no_cpu_baseline,
+                                           outputs=outputs)
         except Exception as exc:  # a sub-record must not take the headline down
             records[name] = {"error": repr(exc)}
             if run.world > 1:
                 raise
         if name in records:
             records[name]["wall_s"] = time.perf_counter() - t0
+    if args.dump_outputs and run.rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
     if "error" in head:
         if run.rank == 0:
             print(json.dumps({"metric": METRIC, "value": None, "unit": UNIT, "n_gpus": run.world, "error": head["error"], "parity": head.get("parity")}))
