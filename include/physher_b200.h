@@ -188,6 +188,23 @@ int phb_tlk_update_uppers(phb_tlk *tlk);
 int phb_tlk_calculate_branch(phb_tlk *tlk, int node, int nbl, const double *bl, double *lnl, double *dlnl, double *d2lnl);
 
 /*
+ * phb_tlk_branch_hessian_diagonal: in ONE call, lnL, d lnL / dt_n and d2 lnL / dt_n^2 for the branch above every node n (by node id), at
+ * the current branch lengths -- the value phb_tlk_calculate_branch(tlk, n, 1, &t_n, ...) returns as d2lnl (d2lnldt2_uppper,
+ * treelikelihood.c:2267-2335), for every branch at once (Newton steps over all branch lengths, Laplace approximations, diagonal
+ * preconditioners).  With L_k, L'_k, L"_k the site likelihood and its first two derivatives in t_n (see phb_tlk_calculate_branch):
+ *   hess[n] = sum_k w_k (L"_k / L_k - (L'_k / L_k)^2)
+ * The derivatives are always the exact ones, like those of phb_tlk_calculate_branch: PHB_OPT_INCLUDE_ROOT_FREQS and
+ * PHB_OPT_COMPAT_SCALED_GRADIENT do not apply.  hess[root] = 0 (and grad[root] = 0); with PHB_OPT_UNROOTED the root's right child is 0
+ * in both.  NaN / inf follow phb_tlk_gradient: an infinite lnL switches rescaling on and recomputes once; a lnL still NaN or infinite
+ * NaN-fills grad and hess.  Afterwards the object's cached lnL is *lnl (a following phb_tlk_calculate launches nothing); the
+ * tlk-owned gradient buffer is not refreshed.  4-state models without rescaling run as one fused walk; every other case (20 / 61 /
+ * any state count, rescaling, PHB_KERNELS_GENERIC, tip partials that are not 0/1 vectors, PHB_OPT_INCREMENTAL on) makes every
+ * upper partial resident and switches PHB_OPT_INCREMENTAL on, as phb_tlk_update_uppers does.  grad may be NULL.
+ * PHB_ESTATE with explicit matrices (phb_tlk_set_matrices): the second derivative needs the eigen system.
+ */
+int phb_tlk_branch_hessian_diagonal(phb_tlk *tlk, double *lnl, double *grad /* [N] or NULL */, double *hess /* [N] */);
+
+/*
  * phb_tlk_update_partials == the struct slot tlk->update_partials(tlk, out, p1, m1, p2, m2) (treelikelihood.h:91), for the callers
  * that drive it themselves: update_upper_partials[2] (treelikelihood.c:2129-2190, i.e. the non-virtual
  * SingleTreeLikelihood_update_uppers[2]), the tripod optimisation of SPR (spropt.c:1578-1608).  ONE partial update on the resident

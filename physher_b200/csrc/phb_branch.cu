@@ -9,9 +9,10 @@
 //   L_k(t)  = sum_c prop_c sum_i pi_i U_n[c,k,i] (P(r_c t) L_n[c,k])_i          lnL   = sum_k w_k (log L_k + sf_k)
 //   L'_k(t) = sum_c prop_c r_c   sum_i pi_i U_n[c,k,i] (P'(r_c t) L_n[c,k])_i   lnL'  = sum_k w_k L'_k / L_k
 //   L"_k(t) = sum_c prop_c r_c^2 sum_i pi_i U_n[c,k,i] (P"(r_c t) L_n[c,k])_i   lnL"  = sum_k w_k (L"_k L_k - L'_k^2) / L_k^2
-// The reference evaluates one candidate length per call, each a full pass over two partials buffers; here ONE launch takes a whole
-// vector of candidate lengths (a bracketing step or a line search), so the two buffers are read once per candidate by CTAs that
-// run concurrently and share them through L2.
+// The reference evaluates one candidate length per call, each a full pass over two partials buffers; here ONE launch takes a list
+// of (node, length) items: one node at a vector of candidate lengths (a bracketing step or a line search, whose CTAs read the same
+// two buffers concurrently and share them through L2), or every non-root node at its own length (the diagonal of the
+// branch-length Hessian, phb_tlk_branch_hessian_diagonal, with the gradient and lnL of the same pass).
 //
 // Under rescaling the per-pattern log factor is sf_upper[n] + sf_lower[n] (the factors that were divided out of U_n and L_n);
 // the derivative ratios are scale free.
@@ -21,7 +22,7 @@
 #include <stdlib.h>
 #include <string.h>
 
-// P(t), r P'(t), r^2 P"(t) for every (candidate, category): grid (nbl, C); mats [nbl][C][3][S*S]
+// P(t), r P'(t), r^2 P"(t) for every (item, category): grid (nitems, C); mats [nitems][C][3][S*S]
 // (p_t substmodel.c:518-557 with fabs, dp_dt :695-723, d2p_d2t :801-828; same operation order, no fused multiply-add)
 __global__ void k_branch_matrices(int S, int C, const double *__restrict__ evec, const double *__restrict__ eval, const double *__restrict__ ivec,
                                   const double *__restrict__ bl, const double *__restrict__ rates, const double *__restrict__ ex_host,
@@ -57,16 +58,17 @@ __global__ void k_branch_matrices(int S, int C, const double *__restrict__ evec,
 
 #define BR_THREADS 128
 
-// grid (pattern tiles, nbl); one thread per pattern; partial [nbl][3][tiles]
-__global__ void __launch_bounds__(BR_THREADS) k_branch_lnl(Bufs b, int node, const double *__restrict__ mats, const double *__restrict__ freqs,
-                                                        const double *__restrict__ props, const double *__restrict__ weights, int scale,
-                                                        double *__restrict__ partial) {
+// grid (pattern tiles, nitems); one thread per pattern; item k is the branch above nodes[k]; partial [nitems][3][tiles]
+__global__ void __launch_bounds__(BR_THREADS) k_branch_lnl(Bufs b, const int *__restrict__ nodes, const double *__restrict__ mats,
+                                                        const double *__restrict__ freqs, const double *__restrict__ props,
+                                                        const double *__restrict__ weights, int scale, double *__restrict__ partial) {
 	extern __shared__ double sm[];
 	__shared__ double red[3][BR_THREADS / 32];
 	const int S = b.S, SS = S * S;
 	const int p = blockIdx.x * blockDim.x + threadIdx.x;
 	const bool live = p < b.P;
 	const int k = blockIdx.y;
+	const int node = nodes[k];
 	const bool tip = is_state_tip(b, node);
 	const int s_tip = (tip && live) ? b.tip_states[(size_t)node * b.P + p] : 0;
 	double L = 0.0, dL = 0.0, d2L = 0.0;
@@ -107,8 +109,11 @@ __global__ void __launch_bounds__(BR_THREADS) k_branch_lnl(Bufs b, int node, con
 			if (!tip) plk += b.sf[(size_t)node * b.P + p];
 		}
 		v[0] = plk * w;
-		v[1] = dL / L * w;
-		v[2] = (d2L * L - dL * dL) / (L * L) * w;  // treelikelihood.c:2331
+		const double r1 = dL / L;
+		v[1] = r1 * w;
+		// treelikelihood.c:2331 forms (L" L - L'^2) / L^2, which underflows to 0 / 0 once L_k < 1e-154 -- site likelihoods a tree of a
+		// thousand taxa reaches without rescaling; the ratio form is the same value and stays finite
+		v[2] = (d2L / L - r1 * r1) * w;
 	}
 	for (int q = 0; q < 3; q++) {
 		const double s = phb_warp_sum(v[q]);
@@ -138,26 +143,36 @@ __global__ void k_branch_sum(const double *__restrict__ partial, int n, double *
 	}
 }
 
-// out_host [nbl][3]: lnL, d lnL / dt, d2 lnL / dt2 of the branch above `node` at each candidate length; U_node and L_node must be resident
-extern "C" int phbc_branch_lnl(phbc_ctx *ctx, const phbc_eval_opts *o, int node, int nbl, const double *bl_host, const double *ex_host, double *out_host) {
+// out_host [nitems][3]: lnL, d lnL / dt, d2 lnL / dt2 of the branch above nodes[k] at length bl[k]; U and L of every listed node must be
+// resident.  One node repeated: candidate lengths of one branch; distinct nodes: one entry per branch.
+extern "C" int phbc_branch_lnl(phbc_ctx *ctx, const phbc_eval_opts *o, int nitems, const int *nodes_host, const double *bl_host, const double *ex_host,
+                               double *out_host) {
 	PHBC_CHECK(cudaSetDevice(ctx->device));
 	const size_t S = ctx->S, C = ctx->C, P = ctx->P;
-	if (node < 0 || node >= ctx->N || node == ctx->root || nbl < 1) {
-		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "branch %d (root %d), %d candidate lengths: out of range", node, ctx->root, nbl);
+	if (nitems < 1 || nitems > 65535) {
+		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "%d branch items: out of range (1 .. 65535 per launch)", nitems);
 		return -1;
 	}
 	if (!ctx->have_eigen || o->explicit_matrices) {
 		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "the single-branch path needs the eigen system (explicit matrices cannot be re-evaluated at a new length)");
 		return -4;
 	}
-	if (!ctx->d_upper || (node >= ctx->T && !ctx->d_lower) || (o->scale && !ctx->d_sf) ||
-	    (node < ctx->T && ctx->tip_kind != PHBC_TIP_STATES && !ctx->d_tip_partials)) {
-		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "upper / lower partials are not resident");
-		return -4;
+	for (int k = 0; k < nitems; k++) {
+		const int node = nodes_host[k];
+		if (node < 0 || node >= ctx->N || node == ctx->root) {
+			snprintf(phbc_errbuf, sizeof(phbc_errbuf), "branch %d (root %d): out of range", node, ctx->root);
+			return -1;
+		}
+		if (!ctx->d_upper || (node >= ctx->T && !ctx->d_lower) || (o->scale && !ctx->d_sf) ||
+		    (node < ctx->T && ctx->tip_kind != PHBC_TIP_STATES && !ctx->d_tip_partials)) {
+			snprintf(phbc_errbuf, sizeof(phbc_errbuf), "upper / lower partials are not resident");
+			return -4;
+		}
 	}
+	const size_t n = (size_t)nitems;
 	const size_t tiles = (P + BR_THREADS - 1) / BR_THREADS;
-	// scratch: bl [nbl] | results [nbl][3] | matrices [nbl][C][3][S*S] | partial [nbl][3][tiles] | host exponentials [nbl][C][S]
-	const size_t need = ((size_t)nbl * (4 + C * 3 * S * S + 3 * tiles + C * S)) * sizeof(double);
+	// scratch: bl [n] | results [n][3] | matrices [n][C][3][S*S] | partial [n][3][tiles] | host exponentials [n][C][S] | nodes [n] (int)
+	const size_t need = (n * (4 + C * 3 * S * S + 3 * tiles + C * S) + (n + 1) / 2) * sizeof(double);
 	if (need > ctx->branch_bytes) {
 		PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
 		if (ctx->d_branch) cudaFree(ctx->d_branch);
@@ -166,21 +181,25 @@ extern "C" int phbc_branch_lnl(phbc_ctx *ctx, const phbc_eval_opts *o, int node,
 		PHBC_CHECK(cudaMalloc((void **)&ctx->d_branch, need));
 		ctx->branch_bytes = need;
 	}
-	double *d_bl = ctx->d_branch, *d_out = d_bl + nbl, *d_mats = d_out + 3 * (size_t)nbl, *d_part = d_mats + (size_t)nbl * C * 3 * S * S;
-	double *d_ex = ex_host ? d_part + (size_t)nbl * 3 * tiles : NULL;
-	PHBC_CHECK(cudaMemcpyAsync(d_bl, bl_host, nbl * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-	if (ex_host) PHBC_CHECK(cudaMemcpyAsync(d_ex, ex_host, (size_t)nbl * C * S * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+	double *d_bl = ctx->d_branch, *d_out = d_bl + n, *d_mats = d_out + 3 * n, *d_part = d_mats + n * C * 3 * S * S;
+	double *d_exbuf = d_part + n * 3 * tiles;
+	double *d_ex = ex_host ? d_exbuf : NULL;
+	int *d_nodes = reinterpret_cast<int *>(d_exbuf + n * C * S);
+	PHBC_CHECK(cudaMemcpyAsync(d_bl, bl_host, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+	PHBC_CHECK(cudaMemcpyAsync(d_nodes, nodes_host, n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+	if (ex_host) PHBC_CHECK(cudaMemcpyAsync(d_ex, ex_host, n * C * S * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
 	const int mthreads = S * S >= 256 ? 256 : (S * S >= 64 ? 64 : 32);
-	k_branch_matrices<<<dim3(nbl, (unsigned)C), mthreads, 3 * S * sizeof(double), ctx->stream>>>((int)S, (int)C, ctx->d_evec, ctx->d_eval, ctx->d_ivec, d_bl,
-	                                                                                        ctx->d_rates, d_ex, d_mats);
+	k_branch_matrices<<<dim3((unsigned)n, (unsigned)C), mthreads, 3 * S * sizeof(double), ctx->stream>>>((int)S, (int)C, ctx->d_evec, ctx->d_eval, ctx->d_ivec,
+	                                                                                                d_bl, ctx->d_rates, d_ex, d_mats);
 	const size_t smem = 3 * S * S * sizeof(double);
 	if (smem > 48 * 1024) PHBC_CHECK(cudaFuncSetAttribute(k_branch_lnl, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 	Bufs b = phbc_make_bufs(ctx);
-	k_branch_lnl<<<dim3((unsigned)tiles, nbl), BR_THREADS, smem, ctx->stream>>>(b, node, d_mats, ctx->d_freqs, ctx->d_props, ctx->d_weights, o->scale, d_part);
-	k_branch_sum<<<3 * nbl, 256, 0, ctx->stream>>>(d_part, (int)tiles, d_out);
+	k_branch_lnl<<<dim3((unsigned)tiles, (unsigned)n), BR_THREADS, smem, ctx->stream>>>(b, d_nodes, d_mats, ctx->d_freqs, ctx->d_props, ctx->d_weights,
+	                                                                                   o->scale, d_part);
+	k_branch_sum<<<(unsigned)(3 * n), 256, 0, ctx->stream>>>(d_part, (int)tiles, d_out);
 	ctx->launches += 3;
 	PHBC_CHECK(cudaGetLastError());
-	PHBC_CHECK(cudaMemcpyAsync(out_host, d_out, 3 * (size_t)nbl * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+	PHBC_CHECK(cudaMemcpyAsync(out_host, d_out, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
 	PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
 	return 0;
 }

@@ -65,6 +65,9 @@ struct phbc_ctx {
 	size_t walk_gstat_bytes;
 	double *d_nuc4_G;        // [N][C][16] summed statistics; the root's entry holds the root term of the frequency gradient
 	bool nuc4_G_valid;       // d_nuc4_G belongs to the current inputs (cleared by every other evaluation)
+	double *d_walk_hacc;     // per-(CTA, warp) Hessian-diagonal rows [grid][warps][N] (GRAD = 3 walks)
+	size_t walk_hacc_bytes;
+	double *d_nuc4_hess;     // [N] summed Hessian diagonal of the last GRAD = 3 walk
 	double *h_freqs, *h_qmat;  // host copies of small model constants (kernel parameter bank)
 
 	// outputs

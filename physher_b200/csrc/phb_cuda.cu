@@ -102,7 +102,7 @@ extern "C" void phbc_destroy(phbc_ctx *ctx) {
 	                ctx->d_freqs, ctx->d_rates, ctx->d_props, ctx->d_bl, ctx->d_P, ctx->d_dP, ctx->d_lower, ctx->d_upper,
 	                ctx->d_sf, ctx->d_lower_ops, ctx->d_upper_ops, ctx->d_parent_ops, ctx->d_post_ops, ctx->d_pre_ops, ctx->d_walk_mats,
 	                ctx->d_walk_lower, ctx->d_walk_gacc, ctx->d_pattern_lnl, ctx->d_result, ctx->d_cat_grad, ctx->d_scratch,
-	                ctx->d_nuc4_codes, ctx->d_nuc4_bad, ctx->d_nuc4_cta_lnl, ctx->d_walk_gstat, ctx->d_nuc4_G, ctx->d_ex, ctx->d_post_tip_order, ctx->d_pre_tip_order, ctx->d_dmma_img, ctx->d_tt_lowers, ctx->d_tt_topo, ctx->d_tt_bad,
+	                ctx->d_nuc4_codes, ctx->d_nuc4_bad, ctx->d_nuc4_cta_lnl, ctx->d_walk_gstat, ctx->d_nuc4_G, ctx->d_walk_hacc, ctx->d_nuc4_hess, ctx->d_ex, ctx->d_post_tip_order, ctx->d_pre_tip_order, ctx->d_dmma_img, ctx->d_tt_lowers, ctx->d_tt_topo, ctx->d_tt_bad,
 	                ctx->d_tt_ratios, ctx->d_tt_rates, ctx->d_tt_heights, ctx->d_tt_adj, ctx->d_tt_out, ctx->d_reduce,
 	                ctx->d_dw_post, ctx->d_dw_pre, ctx->d_dw_codes, ctx->d_dw_bad, ctx->d_dw_spill, ctx->d_enc_states, ctx->d_rowmax, ctx->d_upper_slot, ctx->d_cherry_tab, ctx->d_cherry_ops, ctx->d_cherry_enum, ctx->d_cherry_pairmax};
 	for (size_t i = 0; i < sizeof(bufs) / sizeof(bufs[0]); i++)

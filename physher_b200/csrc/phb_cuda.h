@@ -128,7 +128,7 @@ typedef struct phbc_eval_opts {
 	double scaling_threshold;
 	int include_root_freqs;
 	int compat_scaled_gradient;
-	int want_gradient;
+	int want_gradient;           /* 0 lnL, 1 + branch gradients, 2 + transition statistics, 3 + Hessian diagonal (fused 4-state walk only) */
 	int explicit_matrices;       /* matrices were uploaded, do not rebuild them from the eigen system */
 	int batch_index;             /* which uploaded branch-length vector (the first one of a batch)  */
 	int materialize_uppers;      /* tensor-core path: store every upper partial (tips included) and reduce with the generic K9/K10 */
@@ -164,9 +164,14 @@ int phbc_root_frequency_gradient(phbc_ctx *ctx, double *out /* [S] */);
 int phbc_root_category_gradient(phbc_ctx *ctx, double *out /* [C] */);
 /* K9 / K10 / A11 over every branch from resident upper and lower partials (results in slot 0; lnL slot untouched) */
 int phbc_resident_gradient(phbc_ctx *ctx, const phbc_eval_opts *o);
-/* single-branch fast path (phb_branch.cu): out [nbl][3] = lnL, d lnL/dt, d2 lnL/dt2 at each candidate length of the branch above node */
-/* ex (may be NULL): [nbl][C][S] exp(eval * bl * rate) from the host's libm */
-int phbc_branch_lnl(phbc_ctx *ctx, const phbc_eval_opts *o, int node, int nbl, const double *bl, const double *ex, double *out);
+/* single-branch fast path (phb_branch.cu) on resident upper / lower partials: out [nitems][3] = lnL, d lnL/dt, d2 lnL/dt2 of the branch
+ * above nodes[k] at length bl[k] -- one node repeated (candidate lengths) or every non-root node at its own length (Hessian diagonal) */
+/* ex (may be NULL): [nitems][C][S] exp(eval * bl * rate) from the host's libm */
+int phbc_branch_lnl(phbc_ctx *ctx, const phbc_eval_opts *o, int nitems, const int *nodes, const double *bl, const double *ex, double *out);
+/* lnL, d lnL / d bl [N] and d2 lnL / d bl2 [N] (exact form, root entries 0, no unrooted convention) from ONE unscaled fused 4-state
+ * walk (want_gradient = 3, phb_nuc4.cu); grad may be NULL.  Returns 1 (declined, nothing done) when the walk cannot serve the request:
+ * not 4 states, a shape phbc_nuc4_supported refuses, rescaling, PHB_KERNELS_GENERIC, tip partials that are not 0/1 vectors, a batch. */
+int phbc_nuc4_hessian(phbc_ctx *ctx, const phbc_eval_opts *o, double *lnl, double *grad, double *hess);
 int phbc_matrix_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, int nsets, const double *M_host, int skip_node, double *lnl, double *out_host);
 /* time-tree chain, batched (phb_timetree.cu) */
 int phbc_set_time_tree(phbc_ctx *ctx, const double *lowers, const int *parent, const int *preorder, const int *postorder);

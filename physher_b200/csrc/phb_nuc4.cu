@@ -26,7 +26,10 @@
 //     shuffle rounds) and accumulated with no-return reductions into warp-private rows, which a second
 //     tiny kernel sums in a fixed order (deterministic);
 //   * GRAD = 2 additionally accumulates the 4 x 4 transition statistics of every branch (gstat_add), from which the
-//     substitution-model parameter gradients of calculate_dlnl_dQ (treelikelihood.c:2337-2583) are 16-element contractions.
+//     substitution-model parameter gradients of calculate_dlnl_dQ (treelikelihood.c:2337-2583) are 16-element contractions;
+//   * GRAD = 3 (unscaled, exact form) additionally accumulates the diagonal of the branch-length Hessian: d2P/dt2 L = Q^2 (P L)
+//     is one more product with a constant matrix (diag(pi) Q^2 in the parameter bank), and the (L'/L)^2 term takes each pattern's
+//     L' summed over the categories through a shared-memory exchange per op.
 //
 // CTAs are persistent: grid = min(tiles, resident CTAs), each CTA loops over pattern tiles and owns
 // its scratch, so device memory is independent of the pattern count.
@@ -66,6 +69,10 @@ struct Nuc4Params {
 	double fq[4];     // weights of the gradient numerator: pi, or 1 when the root frequencies are folded into the uppers
 	double wroot[4];  // upper message entering the root's children: 1, or pi (tlk->include_root_freqs)
 	double FQ[16];    // diag(fq) Q: row i of the rate matrix times the weight of state i in the gradient numerator
+	// GRAD == 3 only (appended: the layout above is that of the other variants)
+	double FQ2[16];        // diag(pi) Q^2: weights of the second-derivative numerator
+	const double *rates;   // [C] category rates
+	double *hacc;          // [grid][warps][N] Hessian-diagonal rows
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -212,14 +219,17 @@ __device__ __forceinline__ void matvec_smem_n(const double *__restrict__ M, cons
 
 // A thread owns PPT (pattern, category) cells of the tile: category c and patterns pl0 + u * PBT (PBT = PB / PPT), i.e. cell
 // index c * PB + pl0 + u * PBT in every [half][NUC4_NT] cell array (slots, lower rows) -- the layouts do not depend on PPT.
-// GRAD: 0 lnL only, 1 + branch gradients, 2 + expected-transition statistics per branch (substitution-model gradients)
+// GRAD: 0 lnL only, 1 + branch gradients, 2 + expected-transition statistics per branch (substitution-model gradients),
+// 3 + the diagonal of the branch-length Hessian (unscaled only; the extra accumulators do not fit the 168 / 80-register budgets of
+// three CTAs per SM: two CTAs at PPT = 2, one at PPT = 1, so that nothing spills)
 template <int C, bool SCALE, int GRAD, int PPT>
-__global__ void __launch_bounds__(NUC4_NT / PPT, 3) k_nuc4_walk(const Nuc4Params prm) {
+__global__ void __launch_bounds__(NUC4_NT / PPT, GRAD == 3 ? (PPT == 1 ? 1 : 2) : 3) k_nuc4_walk(const Nuc4Params prm) {
 	extern __shared__ __align__(128) unsigned char smem_raw[];
 	constexpr int PB = NUC4_NT / C;      // patterns per tile
 	constexpr int NTHR = NUC4_NT / PPT;  // threads per CTA
 	constexpr int PBT = PB / PPT;        // patterns per u-plane
 	static_assert(PBT % 32 == 0 || PPT == 1, "a warp must not mix categories");
+	static_assert(GRAD != 3 || !SCALE, "the Hessian walk is unscaled (rescaled evaluations take the resident-partials route)");
 	constexpr bool RECOMP = GRAD == 1 && !SCALE;  // cherry recomputation (phb_cuda.h): the descriptors' flags are honoured by this variant only
 	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 	const int c = tid / PBT, pl0 = tid - c * PBT;
@@ -229,7 +239,7 @@ __global__ void __launch_bounds__(NUC4_NT / PPT, 3) k_nuc4_walk(const Nuc4Params
 	unsigned char *stage0 = smem_raw;
 	unsigned char *slot_cell = stage0 + 2 * lay.bytes + cell0 * 16;  // this thread's first cell in slot 0
 	double *xch = reinterpret_cast<double *>(stage0 + 2 * lay.bytes + (size_t)prm.nslots * NUC4_SLOT_BYTES);
-	double *invLw = xch + (SCALE ? (GRAD == 2 ? 5 : 4) : 1) * C * PB;
+	double *invLw = xch + (SCALE ? (GRAD == 2 ? 5 : 4) : (GRAD == 3 ? 2 : 1)) * C * PB;  // GRAD == 3: 1 / L_k follows at invLw + PB
 	double *sfslot = invLw + PB;  // [nslots][NT] thread-private copies (SCALE only)
 	const uint32_t my_mat = lay.mat_off + c * 128;  // this thread's category inside a staged matrix group
 	const uint32_t my_code = lay.code_off + pl0;
@@ -247,6 +257,8 @@ __global__ void __launch_bounds__(NUC4_NT / PPT, 3) k_nuc4_walk(const Nuc4Params
 	unsigned char *row_cell = GRAD ? reinterpret_cast<unsigned char *>(prm.lower) + (size_t)blockIdx.x * prm.n_post * NUC4_ROW_BYTES + cell0 * 16 : nullptr;
 	double *my_gacc = nullptr;
 	double *my_gstat = GRAD == 2 ? prm.gstat + ((size_t)blockIdx.x * (NTHR / 32) + warp) * prm.N * 16 : nullptr;  // single sample only
+	double *my_hacc = GRAD == 3 ? prm.hacc + ((size_t)blockIdx.x * (NTHR / 32) + warp) * prm.N : nullptr;          // single sample only
+	const double rate_c = GRAD == 3 ? prm.rates[c] : 0.0;
 
 	// L2 prefetch lanes of the pre-order pass (see pre_op): lane -> (row a | b, plane, half, 128-byte line)
 	constexpr int PF_LPR = PPT * 2 * 4;  // lines per message row and warp
@@ -407,6 +419,7 @@ __global__ void __launch_bounds__(NUC4_NT / PPT, 3) k_nuc4_walk(const Nuc4Params
 					const double w = live ? prm.weights[p] : 0.0;
 					if (live && prm.nbatch == 1) prm.pattern_lnl[p] = plk;
 					invLw[pl] = w / L;  // unscaled path: w_k / L_k; scaled paths use ratios instead
+					if (GRAD == 3) invLw[PB + pl] = 1.0 / L;
 					v += live ? plk * w : 0.0;
 				}
 				v = phb_warp_sum(v);
@@ -417,13 +430,14 @@ __global__ void __launch_bounds__(NUC4_NT / PPT, 3) k_nuc4_walk(const Nuc4Params
 
 		// ------------------------------------------------------------------ pre-order + gradients
 		if (GRAD) {
-			double sgrad[PPT], wk[PPT];
+			double sgrad[PPT], wk[PPT], rinv[PPT];
 #pragma unroll
 			for (int u = 0; u < PPT; u++) {
 				const int pl = pl0 + u * PBT;
 				const int p = tile * PB + pl;
 				sgrad[u] = invLw[pl];
 				wk[u] = p < prm.P ? prm.weights[p] : 0.0;
+				rinv[u] = GRAD == 3 ? invLw[PB + pl] : 0.0;
 			}
 			if (GRAD == 2) {
 				// root entry of the statistics: sum_k w_k / L_k L_root[c, k, i] (the root term of the frequency parameters,
@@ -464,12 +478,13 @@ __global__ void __launch_bounds__(NUC4_NT / PPT, 3) k_nuc4_walk(const Nuc4Params
 			// thing this op does is to issue the loads of the NEXT op's rows into the other register set (na / nb), a full op ahead
 			// of their use -- the two sets alternate between consecutive ops, no copies, and nothing tempts ptxas to sink the loads
 			// towards their consumer.  The statistics variant (GRAD = 2) has no registers to spare for a second set: it copies its
-			// operands out and refills the same set (na / nb alias xa / xb).  Returns the two gradient terms.
+			// operands out and refills the same set (na / nb alias xa / xb).  Returns the two gradient terms (and with GRAD == 3 the two
+			// Hessian terms in ha / hb).
 			constexpr bool ALT = GRAD != 2;
 			constexpr bool L2PF = NUC4_L2PF && GRAD != 2;  // the statistics variant is issue-bound: the hints cost it more than they return
 			auto pre_op = [&](const phbc_pre_op *desc, const unsigned char *mats, const uint8_t *cds, int j, int cnt, bool more_chunks,
 			                  double (&xa)[PPT][4], double (&xb)[PPT][4], double (&na_)[PPT][4], double (&nb_)[PPT][4], double (&ureg)[PPT][4],
-			                  double &va, double &vb) {
+			                  double &va, double &vb, double &ha, double &hb) {
 				const phbc_pre_op *d = desc + j;
 				const int kind = d->kind;
 				auto prefetch = [&]() {
@@ -566,6 +581,47 @@ __global__ void __launch_bounds__(NUC4_NT / PPT, 3) k_nuc4_walk(const Nuc4Params
 				if (!SCALE) {
 #pragma unroll
 					for (int u = 0; u < PPT; u++) va = fma(na[u], sgrad[u], va), vb = fma(nb[u], sgrad[u], vb);
+					if (GRAD == 3) {
+						// row of category c, scaled by prop_c r_c in k_nuc4_finalize: w_k / L_k (r_c s_c - (L'_k / L_k) n_c) with s_c = sum_i
+						// pi_i U[i] (Q^2 m)[i] and n_c = sum_i pi_i U[i] (Q m)[i]; summed over the categories that is
+						// w_k (L"_k / L_k - (L'_k / L_k)^2), d2lnldt2_uppper (treelikelihood.c:2331)
+						double lpa[PPT], lpb[PPT];
+						if (C == 1) {
+#pragma unroll
+							for (int u = 0; u < PPT; u++) lpa[u] = rate_c * na[u] * rinv[u], lpb[u] = rate_c * nb[u] * rinv[u];
+						} else {  // L'_k sums over the categories: exchange through two shared planes
+							const double pr = prm.props[c] * rate_c;
+							__syncthreads();  // previous op's readers are done
+#pragma unroll
+							for (int u = 0; u < PPT; u++) {
+								const int ci = cell0 + u * PBT;
+								xch[ci] = na[u] * pr;
+								xch[C * PB + ci] = nb[u] * pr;
+							}
+							__syncthreads();
+#pragma unroll
+							for (int u = 0; u < PPT; u++) {
+								const int pl = pl0 + u * PBT;
+								double sa = 0.0, sb = 0.0;
+								for (int cc = 0; cc < C; cc++) sa += xch[cc * PB + pl], sb += xch[C * PB + cc * PB + pl];
+								lpa[u] = sa * rinv[u], lpb[u] = sb * rinv[u];
+							}
+						}
+						ha = hb = 0.0;
+#pragma unroll
+						for (int u = 0; u < PPT; u++) {
+							double sa = 0.0, sb = 0.0;
+#pragma unroll
+							for (int i = 0; i < 4; i++) {
+								const double qa = fma(prm.FQ2[4 * i], ma[u][0], fma(prm.FQ2[4 * i + 1], ma[u][1], fma(prm.FQ2[4 * i + 2], ma[u][2], prm.FQ2[4 * i + 3] * ma[u][3])));
+								const double qb = fma(prm.FQ2[4 * i], mb[u][0], fma(prm.FQ2[4 * i + 1], mb[u][1], fma(prm.FQ2[4 * i + 2], mb[u][2], prm.FQ2[4 * i + 3] * mb[u][3])));
+								sa = fma(ua[u][i], qa, sa);
+								sb = fma(ub[u][i], qb, sb);
+							}
+							ha = fma(sgrad[u], rate_c * sa - lpa[u] * na[u], ha);
+							hb = fma(sgrad[u], rate_c * sb - lpb[u] * nb[u], hb);
+						}
+					}
 				} else {
 					// rescale the upper partials like the reference (their scale cancels in the ratios below)
 					double *plane = xch;  // planes: max_a, max_b, den_a, den_b [, den_p]
@@ -708,19 +764,31 @@ __global__ void __launch_bounds__(NUC4_NT / PPT, 3) k_nuc4_walk(const Nuc4Params
 				for (int j = 0; j < cnt; j += 2) {
 					// two ops (four branches) share one warp butterfly; partial sums go to warp-private rows
 					double v0, v1, v2 = 0.0, v3 = 0.0;
-					if (ALT) pre_op(desc, mats, cds, j, cnt, more, xa, xb, ya, yb, ureg, v0, v1);
-					else pre_op(desc, mats, cds, j, cnt, more, xa, xb, xa, xb, ureg, v0, v1);
+					double h0 = 0.0, h1 = 0.0, h2 = 0.0, h3 = 0.0;  // GRAD == 3 only
+					if (ALT) pre_op(desc, mats, cds, j, cnt, more, xa, xb, ya, yb, ureg, v0, v1, h0, h1);
+					else pre_op(desc, mats, cds, j, cnt, more, xa, xb, xa, xb, ureg, v0, v1, h0, h1);
 					if (j + 1 < cnt) {
-						if (ALT) pre_op(desc, mats, cds, j + 1, cnt, more, ya, yb, xa, xb, ureg, v2, v3);
-						else pre_op(desc, mats, cds, j + 1, cnt, more, xa, xb, xa, xb, ureg, v2, v3);
+						if (ALT) pre_op(desc, mats, cds, j + 1, cnt, more, ya, yb, xa, xb, ureg, v2, v3, h2, h3);
+						else pre_op(desc, mats, cds, j + 1, cnt, more, xa, xb, xa, xb, ureg, v2, v3, h2, h3);
 						const double r = butterfly4(v0, v1, v2, v3, lane);
 						if ((lane & 7) == 0) {
 							const phbc_pre_op *d = desc + j + ((lane >> 3) & 1);
 							red_add_f64(my_gacc + ((lane & 16) ? d->b_node : d->a_node), r);
 						}
+						if (GRAD == 3) {
+							const double rh = butterfly4(h0, h1, h2, h3, lane);
+							if ((lane & 7) == 0) {
+								const phbc_pre_op *d = desc + j + ((lane >> 3) & 1);
+								red_add_f64(my_hacc + ((lane & 16) ? d->b_node : d->a_node), rh);
+							}
+						}
 					} else {
 						const double r = butterfly2(v0, v1, lane);
 						if ((lane & 15) == 0) red_add_f64(my_gacc + ((lane & 16) ? desc[j].b_node : desc[j].a_node), r);
+						if (GRAD == 3) {
+							const double rh = butterfly2(h0, h1, lane);
+							if ((lane & 15) == 0) red_add_f64(my_hacc + ((lane & 16) ? desc[j].b_node : desc[j].a_node), rh);
+						}
 					}
 				}
 				loads++;
@@ -827,7 +895,8 @@ __global__ void k_nuc4_encode_tips(int T, int P, int PB, int ntiles, int tip_kin
 __global__ void __launch_bounds__(32 * NUC4_FY) k_nuc4_finalize(int N, int C, int nw /* warps per walk CTA */, int grid, int phases, int ntiles, int nbatch, int root,
                                                                 const double *__restrict__ cta_lnl, const double *__restrict__ gacc, int want_grad,
                                                                 const double *__restrict__ props, const double *__restrict__ rates,
-                                                                double *__restrict__ cat_grad, double *__restrict__ result) {
+                                                                double *__restrict__ cat_grad, double *__restrict__ result,
+                                                                const double *__restrict__ hacc, double *__restrict__ hess) {
 	constexpr int warps = NUC4_NT / 32;  // upper bound of nw
 	__shared__ double red[NUC4_FY][warps][33];
 	const int wpc = nw / C;  // warps per category
@@ -869,37 +938,44 @@ __global__ void __launch_bounds__(32 * NUC4_FY) k_nuc4_finalize(int N, int C, in
 	}
 	if (!want_grad) return;
 	const int n = blockIdx.x * 32 + tx;
-	double s8[warps];
+	// row set 0: gradient rows -> cat_grad, result[1 + n]; row set 1 (hacc != NULL, single sample): Hessian-diagonal rows -> hess[n],
+	// the category rows weighted like the gradient's (the kernel folded the second rate factor in)
+	for (int set = 0; set < (hacc ? 2 : 1); set++) {
+		const double *rows = set ? hacc : gacc;
+		double s8[warps];
 #pragma unroll
-	for (int w = 0; w < warps; w++) s8[w] = 0.0;
-	if (n < N && n != root)
-		for (int cta = c_lo + ty; cta < c_hi; cta += NUC4_FY) {
-			const int ph = phase_of(cta);
-			if (ph < 0) continue;
-			const double *base = gacc + ((size_t)cta * phases + ph) * nw * N + n;
+		for (int w = 0; w < warps; w++) s8[w] = 0.0;
+		if (n < N && n != root)
+			for (int cta = c_lo + ty; cta < c_hi; cta += NUC4_FY) {
+				const int ph = phase_of(cta);
+				if (ph < 0) continue;
+				const double *base = rows + ((size_t)cta * phases + ph) * nw * N + n;
 #pragma unroll
-			for (int w = 0; w < warps; w++)
-				if (w < nw) s8[w] += base[(size_t)w * N];  // independent loads in flight
-		}
+				for (int w = 0; w < warps; w++)
+					if (w < nw) s8[w] += base[(size_t)w * N];  // independent loads in flight
+			}
 #pragma unroll
-	for (int w = 0; w < warps; w++) red[ty][w][tx] = s8[w];
-	__syncthreads();
-	if (ty < nw) {  // thread row w sums warp-row w over the CTA slices, fixed order
-		double tot = 0.0;
-		for (int k = 0; k < NUC4_FY; k++) tot += red[k][ty][tx];
-		red[0][ty][tx] = tot;  // slice 0 of row ty is read only by this thread above
-	}
-	__syncthreads();
-	if (ty == 0 && n < N) {
-		double g = 0.0;
-		for (int c = 0; c < C; c++) {
+		for (int w = 0; w < warps; w++) red[ty][w][tx] = s8[w];
+		__syncthreads();
+		if (ty < nw) {  // thread row w sums warp-row w over the CTA slices, fixed order
 			double tot = 0.0;
-			for (int w = 0; w < wpc; w++) tot += red[0][c * wpc + w][tx];
-			cat_grad[(size_t)n * C + c] = tot;
-			if (C == 1) g = tot;
-			else g = c == 0 ? tot * props[0] * rates[0] : g + tot * props[c] * rates[c];
+			for (int k = 0; k < NUC4_FY; k++) tot += red[k][ty][tx];
+			red[0][ty][tx] = tot;  // slice 0 of row ty is read only by this thread above
 		}
-		result[1 + n] = g;
+		__syncthreads();
+		if (ty == 0 && n < N) {
+			double g = 0.0;
+			for (int c = 0; c < C; c++) {
+				double tot = 0.0;
+				for (int w = 0; w < wpc; w++) tot += red[0][c * wpc + w][tx];
+				if (set == 0) cat_grad[(size_t)n * C + c] = tot;
+				if (C == 1) g = tot;
+				else g = c == 0 ? tot * props[0] * rates[0] : g + tot * props[c] * rates[c];
+			}
+			if (set == 0) result[1 + n] = g;
+			else hess[n] = C == 1 ? g * rates[0] : g;  // C == 1: the weighting above leaves the rate factor out
+		}
+		__syncthreads();  // red is reused by the next row set
 	}
 }
 
@@ -961,9 +1037,11 @@ __global__ void k_nuc4_gstat_contract(int N, int C, int root, int skip, const do
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-static size_t nuc4_smem_bytes(int C, int PB, int nslots, bool scale, bool stat) {
+// grad: phbc_eval_opts.want_gradient (2: statistics planes under rescaling; 3: two exchange planes and 1 / L_k, unscaled only)
+static size_t nuc4_smem_bytes(int C, int PB, int nslots, bool scale, int grad) {
+	const bool stat = grad == 2, hess = grad == 3 && !scale;
 	return 2 * (size_t)nuc4_stage_layout(C, PB).bytes + (size_t)nslots * NUC4_SLOT_BYTES +
-	       (size_t)((scale ? (stat ? 5 : 4) : 1) * C * PB + PB + (scale ? nslots * NUC4_NT : 0)) * sizeof(double);
+	       (size_t)((scale ? (stat ? 5 : 4) : (hess ? 2 : 1)) * C * PB + (hess ? 2 : 1) * PB + (scale ? nslots * NUC4_NT : 0)) * sizeof(double);
 }
 
 static int pattern_block(int C) {
@@ -976,7 +1054,7 @@ bool phbc_nuc4_supported(const phbc_ctx *ctx, const phbc_eval_opts *o) {
 	if (ctx->C != 1 && ctx->C != 2 && ctx->C != 4 && ctx->C != 8) return false;  // categories must tile the CTA exactly
 	const int PB = pattern_block(ctx->C);
 	const int nslots = ctx->post_slots > ctx->pre_slots ? ctx->post_slots : ctx->pre_slots;
-	if (nuc4_smem_bytes(ctx->C, PB, nslots, o->scale != 0, o->want_gradient == 2) > ctx->smem_optin) return false;
+	if (nuc4_smem_bytes(ctx->C, PB, nslots, o->scale != 0, o->want_gradient) > ctx->smem_optin) return false;
 	return true;
 }
 
@@ -988,7 +1066,7 @@ int phbc_nuc4_evaluate(phbc_ctx *ctx, const phbc_eval_opts *o) {
 	const int C = ctx->C, N = ctx->N, T = ctx->T, P = ctx->P;
 	const int PB = pattern_block(C);
 	const int nslots = ctx->post_slots > ctx->pre_slots ? ctx->post_slots : ctx->pre_slots;
-	const size_t smem = nuc4_smem_bytes(C, PB, nslots, o->scale != 0, o->want_gradient == 2);
+	const size_t smem = nuc4_smem_bytes(C, PB, nslots, o->scale != 0, o->want_gradient);
 	const int ntiles = (P + PB - 1) / PB;
 	// tip codes in walk order (once per tip upload / schedule change)
 	{
@@ -1022,14 +1100,21 @@ int phbc_nuc4_evaluate(phbc_ctx *ctx, const phbc_eval_opts *o) {
 	                                         {k_nuc4_walk<2, false, 2, 2>, k_nuc4_walk<2, true, 2, 2>},
 	                                         {k_nuc4_walk<4, false, 2, 2>, k_nuc4_walk<4, true, 2, 2>},
 	                                         {k_nuc4_walk<8, false, 2, 1>, k_nuc4_walk<8, true, 2, 1>}};
+	// unscaled walks that also accumulate the diagonal of the branch-length Hessian (phbc_nuc4_hessian)
+	static const walk_fn table_hess[4] = {k_nuc4_walk<1, false, 3, 2>, k_nuc4_walk<2, false, 3, 2>, k_nuc4_walk<4, false, 3, 2>,
+	                                      k_nuc4_walk<8, false, 3, 1>};
 	const int ppt = C == 8 ? 1 : 2, nthr = NUC4_NT / ppt;
 	const int ci = C == 1 ? 0 : (C == 2 ? 1 : (C == 4 ? 2 : 3));
-	const bool want_stat = o->want_gradient == 2;
+	const bool want_stat = o->want_gradient == 2, want_hess = o->want_gradient == 3;
 	if (want_stat && o->batch_count > 1) {
 		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "nuc4 walk: transition statistics need a single-sample evaluation");
 		return -1;
 	}
-	walk_fn kern = want_stat ? table_stat[ci][o->scale ? 1 : 0] : table[ci][o->scale ? 1 : 0][o->want_gradient ? 1 : 0];
+	if (want_hess && (o->batch_count > 1 || o->scale)) {
+		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "nuc4 walk: the Hessian diagonal needs a single unscaled evaluation");
+		return -1;
+	}
+	walk_fn kern = want_hess ? table_hess[ci] : want_stat ? table_stat[ci][o->scale ? 1 : 0] : table[ci][o->scale ? 1 : 0][o->want_gradient ? 1 : 0];
 	ctx->nuc4_G_valid = false;
 	PHBC_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 	int per_sm = 0;
@@ -1097,6 +1182,19 @@ int phbc_nuc4_evaluate(phbc_ctx *ctx, const phbc_eval_opts *o) {
 		if (!ctx->d_nuc4_G) PHBC_CHECK(cudaMalloc((void **)&ctx->d_nuc4_G, (size_t)N * C * 16 * sizeof(double)));
 		PHBC_CHECK(cudaMemsetAsync(ctx->d_walk_gstat, 0, gstat_bytes, ctx->stream));
 	}
+	if (want_hess) {
+		const size_t hacc_bytes = (size_t)grid * warps * N * sizeof(double);
+		if (hacc_bytes > ctx->walk_hacc_bytes) {
+			PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
+			if (ctx->d_walk_hacc) cudaFree(ctx->d_walk_hacc);
+			ctx->d_walk_hacc = NULL;
+			ctx->walk_hacc_bytes = 0;
+			PHBC_CHECK(cudaMalloc((void **)&ctx->d_walk_hacc, hacc_bytes));
+			ctx->walk_hacc_bytes = hacc_bytes;
+		}
+		if (!ctx->d_nuc4_hess) PHBC_CHECK(cudaMalloc((void **)&ctx->d_nuc4_hess, (size_t)N * sizeof(double)));
+		PHBC_CHECK(cudaMemsetAsync(ctx->d_walk_hacc, 0, hacc_bytes, ctx->stream));
+	}
 	if (!ctx->d_nuc4_cta_lnl || ctx->nuc4_grid < grid * phases) {
 		PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
 		if (ctx->d_nuc4_cta_lnl) cudaFree(ctx->d_nuc4_cta_lnl);
@@ -1144,10 +1242,21 @@ int phbc_nuc4_evaluate(phbc_ctx *ctx, const phbc_eval_opts *o) {
 	prm.cta_lnl = ctx->d_nuc4_cta_lnl;
 	prm.pattern_lnl = ctx->d_pattern_lnl;
 	memcpy(prm.freqs, ctx->h_freqs, sizeof(prm.freqs));  // small model constants travel in the kernel parameter bank
+	const bool irf = o->include_root_freqs && !want_hess;  // the Hessian diagonal is always in the exact form
 	for (int i = 0; i < 4; i++) {
-		prm.fq[i] = o->include_root_freqs ? 1.0 : ctx->h_freqs[i];
-		prm.wroot[i] = o->include_root_freqs ? ctx->h_freqs[i] : 1.0;
+		prm.fq[i] = irf ? 1.0 : ctx->h_freqs[i];
+		prm.wroot[i] = irf ? ctx->h_freqs[i] : 1.0;
 		for (int j = 0; j < 4; j++) prm.FQ[4 * i + j] = prm.fq[i] * ctx->h_qmat[4 * i + j];
+	}
+	if (want_hess) {
+		for (int i = 0; i < 4; i++)
+			for (int j = 0; j < 4; j++) {
+				double q2 = 0.0;
+				for (int k = 0; k < 4; k++) q2 += ctx->h_qmat[4 * i + k] * ctx->h_qmat[4 * k + j];
+				prm.FQ2[4 * i + j] = ctx->h_freqs[i] * q2;
+			}
+		prm.rates = ctx->d_rates;
+		prm.hacc = ctx->d_walk_hacc;
 	}
 	int trc;
 	if ((trc = phbc_time_begin(ctx))) return trc;
@@ -1157,7 +1266,8 @@ int phbc_nuc4_evaluate(phbc_ctx *ctx, const phbc_eval_opts *o) {
 	double *result = ctx->d_result + (size_t)o->batch_index * (1 + N);
 	k_nuc4_finalize<<<dim3((N + 31) / 32, nbatch), dim3(32, NUC4_FY), 0, ctx->stream>>>(N, C, warps, grid, phases, ntiles, nbatch, ctx->root, ctx->d_nuc4_cta_lnl,
 	                                                                         ctx->d_walk_gacc, o->want_gradient, ctx->d_props, ctx->d_rates,
-	                                                                         ctx->d_cat_grad, result);
+	                                                                         ctx->d_cat_grad, result, want_hess ? ctx->d_walk_hacc : NULL,
+	                                                                         want_hess ? ctx->d_nuc4_hess : NULL);
 	ctx->launches++;
 	if (want_stat) {
 		k_nuc4_gstat_sum<<<(N * C * 16 + 63) / 64, dim3(64, NUC4_GY), 0, ctx->stream>>>(N, C, warps, grid, ctx->d_walk_gstat, ctx->d_nuc4_G);
@@ -1236,6 +1346,25 @@ int phbc_nuc4_matrix_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, int nsets,
 	if (lnl) PHBC_CHECK(cudaMemcpyAsync(lnl, ctx->d_result + (size_t)e.batch_index * (1 + N), sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
 	PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
 	PHBC_CHECK(cudaGetLastError());
+	return 0;
+}
+
+// Diagonal of the branch-length Hessian on the fused walk: one GRAD = 3 launch, then lnL, gradient and hess[N] to the host.  Returns 1
+// (declined, nothing done) when the walk cannot serve it (see phb_cuda.h); the caller then takes the resident-partials route.
+int phbc_nuc4_hessian(phbc_ctx *ctx, const phbc_eval_opts *o, double *lnl, double *grad, double *hess) {
+	phbc_eval_opts e = *o;
+	e.want_gradient = 3;
+	e.batch_count = 1;
+	e.include_root_freqs = 0;
+	e.compat_scaled_gradient = 0;
+	if (o->kernels == 1 || o->scale || o->batch_count > 1 || !phbc_nuc4_supported(ctx, &e)) return 1;
+	PHBC_CHECK(cudaSetDevice(ctx->device));
+	int usable = 0, rc;
+	if ((rc = nuc4_prepare_codes(ctx, &usable))) return rc;
+	if (!usable) return 1;
+	if ((rc = phbc_nuc4_evaluate(ctx, &e))) return rc;
+	PHBC_CHECK(cudaMemcpyAsync(hess, ctx->d_nuc4_hess, (size_t)ctx->N * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+	if ((rc = phbc_download_results(ctx, 1, lnl, grad))) return rc;  // synchronises the stream
 	return 0;
 }
 

@@ -1280,6 +1280,23 @@ static int phb_tlk_update_uppers_impl(phb_tlk *t) {
 	return resident_uppers(t, -1, 0);
 }
 
+/* lnL, d lnL/dt, d2 lnL/dt2 [nitems][3] of the branch above nodes[k] at length bl[k]; the uppers and lowers of those nodes are resident */
+static int branch_items(phb_tlk *t, int nitems, const int *nodes, const double *bl, double *out) {
+	phbc_eval_opts o;
+	fill_opts_resident(t, &o, 1);
+	double *ex = NULL;
+	if (wants_host_exp(t)) { /* the item lengths get the host's exponentials like every other matrix of this model */
+		ex = (double *)malloc(sizeof(double) * (size_t)nitems * t->C * t->S);
+		if (!ex) return fail(PHB_ENOMEM, "out of memory");
+		for (int k = 0; k < nitems; k++)
+			for (int c = 0; c < t->C; c++)
+				for (int q = 0; q < t->S; q++) ex[((size_t)k * t->C + c) * t->S + q] = exp(t->h_eval[q] * (bl[k] * t->h_rates[c]));
+	}
+	const int rc = phbc_branch_lnl(t->ctx, &o, nitems, nodes, bl, ex, out);
+	free(ex);
+	return rc ? dev_fail(rc) : PHB_OK;
+}
+
 /* _calculate_uppper + calculate_dldt_uppper + d2lnldt2_uppper (treelikelihood.c:2592-2686, 2195-2335) at nbl candidate lengths */
 static int phb_tlk_calculate_branch_impl(phb_tlk *t, int node, int nbl, const double *bl, double *lnl, double *dlnl, double *d2lnl) {
 	if (node < 0 || node >= t->N || node == t->root) return fail(PHB_EINVAL, "calculate_branch: node %d is not a branch (root %d)", node, t->root);
@@ -1303,23 +1320,16 @@ static int phb_tlk_calculate_branch_impl(phb_tlk *t, int node, int nbl, const do
 		return PHB_OK;
 	}
 	if ((rc = resident_uppers(t, node, 0))) return rc;
+	int *nodes = (int *)malloc(sizeof(int) * (size_t)nbl);
+	if (!nodes) return fail(PHB_ENOMEM, "out of memory");
+	for (int k = 0; k < nbl; k++) nodes[k] = node;
 	double *out = (double *)malloc(sizeof(double) * 3 * (size_t)nbl);
-	if (!out) return fail(PHB_ENOMEM, "out of memory");
-	phbc_eval_opts o;
-	fill_opts_resident(t, &o, 1);
-	double *ex = NULL;
-	if (wants_host_exp(t)) { /* the candidate lengths get the host's exponentials like every other matrix of this model */
-		ex = (double *)malloc(sizeof(double) * (size_t)nbl * t->C * t->S);
-		if (!ex) {
-			free(out);
-			return fail(PHB_ENOMEM, "out of memory");
-		}
-		for (int k = 0; k < nbl; k++)
-			for (int c = 0; c < t->C; c++)
-				for (int q = 0; q < t->S; q++) ex[((size_t)k * t->C + c) * t->S + q] = exp(t->h_eval[q] * (bl[k] * t->h_rates[c]));
+	if (!out) {
+		free(nodes);
+		return fail(PHB_ENOMEM, "out of memory");
 	}
-	rc = phbc_branch_lnl(t->ctx, &o, node, nbl, bl, ex, out);
-	free(ex);
+	rc = branch_items(t, nbl, nodes, bl, out);
+	free(nodes);
 	if (!rc)
 		for (int k = 0; k < nbl; k++) {
 			if (lnl) lnl[k] = out[3 * k];
@@ -1327,7 +1337,91 @@ static int phb_tlk_calculate_branch_impl(phb_tlk *t, int node, int nbl, const do
 			if (d2lnl) d2lnl[k] = out[3 * k + 2];
 		}
 	free(out);
-	if (rc) return dev_fail(rc);
+	return rc;
+}
+
+static void apply_unrooted(const phb_tlk *t, double *g);
+
+/*
+ * Diagonal of the branch-length Hessian (d2lnldt2_uppper, treelikelihood.c:2267-2335, for every branch at its current length), with
+ * lnL and the gradient of the same pass.  Route 1: one unscaled fused 4-state walk that forms d2P/dt2 L = Q (Q m) next to the gradient
+ * terms (phbc_nuc4_hessian).  Route 2, for everything the walk declines: lowers and uppers made resident (PHB_OPT_INCREMENTAL on, as
+ * update_uppers does) and one launch of the single-branch kernels over the list (n, bl[n]) of every non-root node.
+ */
+static int phb_tlk_branch_hessian_diagonal_impl(phb_tlk *t, double *lnl, double *grad, double *hess) {
+	if (!lnl || !hess) return fail(PHB_EINVAL, "branch_hessian_diagonal: lnl and hess are required");
+	if (t->have_matrices) return fail(PHB_ESTATE, "branch_hessian_diagonal needs the eigen system: explicit matrices cannot be differentiated twice");
+	int rc = check_ready(t);
+	if (rc) return rc;
+	const int N = t->N;
+	double cur = 0.0;
+	int done = 0;
+	if (!t->incremental && !t->scale && t->kernels != PHB_KERNELS_GENERIC) {
+		if ((rc = upload_bl(t))) return dev_fail(rc);
+		t->bl_dirty = 0;
+		t->sweep_valid = 0;
+		phbc_eval_opts o;
+		fill_opts(t, &o, 3, 0);
+		rc = phbc_nuc4_hessian(t->ctx, &o, &cur, grad, hess);
+		if (rc < 0) return dev_fail(rc);
+		if (rc == 0) {
+			if (isinf(cur)) { /* treelikelihood.c:1496-1519: rescaling on, recompute once -- on route 2, the walk route is unscaled */
+				t->scale = 1;
+				t->all_dirty = 1;
+			} else {
+				done = 1;
+				t->lk = cur;
+				if (isnan(cur)) {
+					phb_tlk_update_all_nodes(t); /* :1489-1495 */
+				} else {
+					memset(t->update_nodes, 0, N);
+					t->update = 0;
+					t->update_upper = 1; /* the tlk-owned gradient buffer is not refreshed here */
+				}
+			}
+		}
+	}
+	if (!done) {
+		if (!t->incremental) {
+			t->incremental = 1;
+			t->resident = 0;
+		}
+		if ((rc = resident_calculate(t, &cur))) return rc; /* retries with rescaling on itself */
+		if (!isnan(cur) && !isinf(cur)) {
+			if ((rc = resident_uppers(t, -1, 0))) return rc;
+			int *nodes = (int *)malloc(sizeof(int) * (size_t)N);
+			double *bl = (double *)malloc(sizeof(double) * (size_t)N);
+			double *out = (double *)malloc(sizeof(double) * 3 * (size_t)N);
+			if (!nodes || !bl || !out) {
+				free(nodes), free(bl), free(out);
+				return fail(PHB_ENOMEM, "out of memory");
+			}
+			int n_items = 0;
+			for (int n = 0; n < N; n++)
+				if (n != t->root) nodes[n_items] = n, bl[n_items++] = t->bl[n];
+			rc = branch_items(t, n_items, nodes, bl, out);
+			if (!rc) {
+				for (int k = 0; k < n_items; k++) {
+					if (grad) grad[nodes[k]] = out[3 * k + 1];
+					hess[nodes[k]] = out[3 * k + 2];
+				}
+				if (grad) grad[t->root] = 0.0;
+				hess[t->root] = 0.0;
+			}
+			free(nodes), free(bl), free(out);
+			if (rc) return rc;
+		}
+	}
+	*lnl = cur;
+	if (isnan(cur) || isinf(cur)) { /* as phb_tlk_gradient, :328-332 */
+		for (int n = 0; n < N; n++) {
+			if (grad) grad[n] = NAN;
+			hess[n] = NAN;
+		}
+		return PHB_OK;
+	}
+	if (grad) apply_unrooted(t, grad);
+	apply_unrooted(t, hess);
 	return PHB_OK;
 }
 
@@ -1971,6 +2065,13 @@ int phb_tlk_matrix_gradient(phb_tlk *t, int nsets, const double *M, double *out)
 int phb_tlk_calculate_branch(phb_tlk *t, int node, int nbl, const double *bl, double *lnl, double *dlnl, double *d2lnl) {
 	nvtxRangePushA("phb_tlk_calculate_branch");
 	const int rc = phb_tlk_calculate_branch_impl(t, node, nbl, bl, lnl, dlnl, d2lnl);
+	nvtxRangePop();
+	return rc;
+}
+
+int phb_tlk_branch_hessian_diagonal(phb_tlk *t, double *lnl, double *grad, double *hess) {
+	nvtxRangePushA("phb_tlk_branch_hessian_diagonal");
+	const int rc = phb_tlk_branch_hessian_diagonal_impl(t, lnl, grad, hess);
 	nvtxRangePop();
 	return rc;
 }

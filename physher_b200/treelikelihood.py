@@ -70,6 +70,7 @@ SYMBOLS = [
     ("phb_tlk_category_gradient", C.c_int, [C.c_void_p, _dp]),
     ("phb_tlk_update_uppers", C.c_int, [C.c_void_p]),
     ("phb_tlk_calculate_branch", C.c_int, [C.c_void_p, C.c_int, C.c_int, _dp, _dp, _dp, _dp]),
+    ("phb_tlk_branch_hessian_diagonal", C.c_int, [C.c_void_p, _dp, _dp, _dp]),
     ("phb_tlk_update_partials", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _dp]),
     ("phb_tlk_get_partials", C.c_int, [C.c_void_p, C.c_int, _dp]),
     ("phb_tlk_get_matrices", C.c_int, [C.c_void_p, _dp, _dp]),
@@ -452,6 +453,14 @@ class SingleTreeLikelihood:
         self._check(self.lib.phb_tlk_calculate_branch(self.h, int(node), int(a.size), a.ctypes.data_as(_dp), lnl.ctypes.data_as(_dp),
                                                       d1.ctypes.data_as(_dp), d2.ctypes.data_as(_dp)))
         return lnl, d1, d2
+
+    def branch_hessian_diagonal(self):
+        """lnL, d lnL/dt_n and d2 lnL/dt_n^2 of every branch (by node id) at the current lengths, in one call: (lnl, grad[N], hess[N]).
+        hess[n] is what calculate_branch(n, [t_n]) returns as d2 lnL/dt2 (d2lnldt2_uppper, treelikelihood.c:2267-2335)."""
+        lnl = C.c_double(0.0)
+        grad, hess = np.zeros(self.N), np.zeros(self.N)
+        self._check(self.lib.phb_tlk_branch_hessian_diagonal(self.h, C.byref(lnl), grad.ctypes.data_as(_dp), hess.ctypes.data_as(_dp)))
+        return lnl.value, grad, hess
 
     def update_partials(self, out, p1, m1, p2=-1, m2=-1, mirror=True):
         """tlk->update_partials(tlk, out, p1, m1, p2, m2) (treelikelihood.h:91) on the resident device buffers; returns the result."""
