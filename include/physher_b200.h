@@ -205,6 +205,39 @@ int phb_tlk_calculate_branch(phb_tlk *tlk, int node, int nbl, const double *bl, 
 int phb_tlk_branch_hessian_diagonal(phb_tlk *tlk, double *lnl, double *grad /* [N] or NULL */, double *hess /* [N] */);
 
 /*
+ * Nearest-neighbour interchanges (the NNI neighbourhood the tree-search drivers score, nniopt.c:301-334).  Move (x, y): exchange the
+ * subtree rooted at node x with the subtree rooted at node y.  With v = parent[y] (v internal, v != root) a move is valid in exactly
+ * two cases:
+ *   (R) x is the sibling of v                    -- rooted NNI across the branch above v;
+ *   (C) parent[v] is the root, the other child w of the root is internal and parent[x] == w
+ *                                                  -- NNI across the root edge of the unrooted tree.
+ * The exchanged tree: x takes y's slot (same side) under v, y takes x's slot under parent[x].  Branch lengths stay with node ids, as
+ * in phb_tlk_set_topology.  The "central branch" of a move is the branch above v.
+ *
+ * phb_tlk_nni_moves enumerates the neighbourhood into moves [count][2] (may be NULL) and returns the count.  With PHB_OPT_UNROOTED
+ * (default): (sibling(v), left[v]) and (sibling(v), right[v]) for every internal v whose parent is not the root, plus the two moves
+ * across the root (left[r1], left[r2]) and (left[r1], right[r2]) when both root children r1, r2 are internal -- 2(T - 3) moves, one
+ * per neighbour of the unrooted tree.  Without it: both moves of every internal non-root v, 2(T - 2).
+ *
+ * phb_tlk_nni_scores: out[k] = {lnL, d lnL / dt_v, d2 lnL / dt_v2} of the tree move k produces, its central branch at t_central[k]
+ * (NULL: the current t_v) and every other branch at its current length, from resident partials in one pass -- no topology change.
+ * With M_n = P_n L_n, p = parent[v], keep the child of v that stays, W_p = P_p U_p (1 when p is the root):
+ *   (R)  L_k = sum_c prop_c sum_i pi_i [W_p o M_y]_i (P_v (M_keep o M_x))_i
+ *   (C)  the upper side is P_w (M_keep_w o M_y), keep_w the child of w that stays
+ * and the derivatives replace P_v by r_c P'_v and r_c^2 P"_v, in the form sum w (L"/L - (L'/L)^2).  They are the exact ones:
+ * PHB_OPT_INCLUDE_ROOT_FREQS and PHB_OPT_COMPAT_SCALED_GRADIENT do not apply.  Under rescaling the per-pattern log factor is the sum
+ * of the cumulative factors of the four operands.  Like phb_tlk_branch_hessian_diagonal's resident route the call switches
+ * PHB_OPT_INCREMENTAL on and leaves every partial resident; the cached lnL of the current tree is *lnl (may be NULL; a following
+ * phb_tlk_calculate launches nothing).  An infinite lnL of the current tree, or a move whose unscaled site likelihood is 0 or not
+ * finite, switches rescaling on and recomputes once; a lnL still NaN or infinite NaN-fills out.  PHB_EINVAL: an invalid move (the
+ * message names its index), nmoves < 1, a negative t_central, NULL moves / out.  PHB_ESTATE with explicit matrices.  PHB_ENOMEM when
+ * the device cannot hold the resident partials; the object stays usable.
+ */
+int phb_tlk_nni_moves(phb_tlk *tlk, int *moves /* [count][2] or NULL */);
+int phb_tlk_nni_scores(phb_tlk *tlk, int nmoves, const int *moves /* [nmoves][2] */, const double *t_central /* [nmoves] or NULL */,
+                       double *lnl, double *out /* [nmoves][3] */);
+
+/*
  * phb_tlk_update_partials == the struct slot tlk->update_partials(tlk, out, p1, m1, p2, m2) (treelikelihood.h:91), for the callers
  * that drive it themselves: update_upper_partials[2] (treelikelihood.c:2129-2190, i.e. the non-virtual
  * SingleTreeLikelihood_update_uppers[2]), the tripod optimisation of SPR (spropt.c:1578-1608).  ONE partial update on the resident

@@ -172,6 +172,24 @@ int phbc_branch_lnl(phbc_ctx *ctx, const phbc_eval_opts *o, int nitems, const in
  * walk (want_gradient = 3, phb_nuc4.cu); grad may be NULL.  Returns 1 (declined, nothing done) when the walk cannot serve the request:
  * not 4 states, a shape phbc_nuc4_supported refuses, rescaling, PHB_KERNELS_GENERIC, tip partials that are not 0/1 vectors, a batch. */
 int phbc_nuc4_hessian(phbc_ctx *ctx, const phbc_eval_opts *o, double *lnl, double *grad, double *hess);
+/* One nearest-neighbour interchange (phb_nni.cu): x and y exchanged across the branch above v = parent[y].  Buffer indices as in
+ * phbc_op; matrix indices are entries of the call's matrix table (node n at its current length = entry n, move k's central length =
+ * entry N + k). */
+typedef struct phbc_nni_move {
+	int x, y, keep; /* the exchanged subtrees and the child of v that stays                                          */
+	int a, a_mat;   /* second factor of the upper side: N + p (U_p, matrix P_p) for an NNI below p, the child of w that stays
+	                   for one across the root, a = -1 (a vector of ones) when p is the root                            */
+	int w;          /* across the root: the root child w whose matrix closes the upper side; -1 otherwise               */
+	int cmat;       /* table entry of the central branch (P, P', P")                                                   */
+	int out;        /* output row                                                                                      */
+} phbc_nni_move;
+/* device buffers the scores read, allocated before the resident evaluation: -3 when the device cannot hold them */
+int phbc_nni_reserve(phbc_ctx *ctx, int scale);
+/* out [nmoves][3] = lnL, d lnL/dt_v, d2 lnL/dt_v2 of each exchanged tree from resident upper / lower partials; bl [N + nmoves] the matrix
+ * table's lengths, ex (may be NULL) their exponentials [N + nmoves][C][S]; groups [ngroups][2] move pairs sharing (v, x), -1 = none
+ * (the 4-state kernel's work items) */
+int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmoves, const phbc_nni_move *moves, int ngroups, const int *groups,
+                    const double *bl, const double *ex, double *out);
 int phbc_matrix_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, int nsets, const double *M_host, int skip_node, double *lnl, double *out_host);
 /* time-tree chain, batched (phb_timetree.cu) */
 int phbc_set_time_tree(phbc_ctx *ctx, const double *lowers, const int *parent, const int *preorder, const int *postorder);

@@ -1426,6 +1426,152 @@ static int phb_tlk_branch_hessian_diagonal_impl(phb_tlk *t, double *lnl, double 
 }
 
 /*
+ * Nearest-neighbour interchanges (nniopt.c:301-334): move (x, y) exchanges the subtrees rooted at x and y across the branch above
+ * v = parent[y].  Kind R (0): x is the sibling of v.  Kind C (1): v and w are the two children of the root, w is internal and x a child
+ * of w -- the NNI across the root edge of the unrooted tree.  -1: not a move.
+ */
+static int sibling_of(const phb_tlk *t, int n) {
+	const int p = t->parent[n];
+	return t->left[p] == n ? t->right[p] : t->left[p];
+}
+
+static int nni_kind(const phb_tlk *t, int x, int y) {
+	const int N = t->N;
+	if (x < 0 || x >= N || y < 0 || y >= N || x == y) return -1;
+	const int v = t->parent[y];
+	if (v < 0 || v == t->root) return -1;
+	const int p = t->parent[v];
+	if (t->parent[x] == p && x != v) return 0;
+	if (p == t->root) {
+		const int w = sibling_of(t, v);
+		if (!is_tip(t, w) && t->parent[x] == w) return 1;
+	}
+	return -1;
+}
+
+static int phb_tlk_nni_moves_impl(phb_tlk *t, int *moves) {
+	int n = 0;
+	for (int v = 0; v < t->N; v++) {
+		if (is_tip(t, v) || v == t->root || (t->unrooted && t->parent[v] == t->root)) continue;
+		const int s = sibling_of(t, v);
+		if (moves) moves[2 * n] = s, moves[2 * n + 1] = t->left[v], moves[2 * n + 2] = s, moves[2 * n + 3] = t->right[v];
+		n += 2;
+	}
+	const int r1 = t->left[t->root], r2 = t->right[t->root];
+	if (t->unrooted && r1 >= 0 && !is_tip(t, r1) && !is_tip(t, r2)) {
+		if (moves) moves[2 * n] = t->left[r1], moves[2 * n + 1] = t->left[r2], moves[2 * n + 2] = t->left[r1], moves[2 * n + 3] = t->right[r2];
+		n += 2;
+	}
+	return n;
+}
+
+/* launch order of the 4-state kernel's work items: by parent of v, so that the groups of two siblings are neighbours (U_p from L2) */
+static _Thread_local const phb_tlk *g_nni_tlk;
+static _Thread_local const int *g_nni_moves;
+static int nni_order(const void *pa, const void *pb) {
+	const int a = *(const int *)pa, b = *(const int *)pb;
+	const phb_tlk *t = g_nni_tlk;
+	const int va = t->parent[g_nni_moves[2 * a + 1]], vb = t->parent[g_nni_moves[2 * b + 1]];
+	const int ka[4] = {t->parent[va], va, g_nni_moves[2 * a], a}, kb[4] = {t->parent[vb], vb, g_nni_moves[2 * b], b};
+	for (int i = 0; i < 4; i++)
+		if (ka[i] != kb[i]) return ka[i] < kb[i] ? -1 : 1;
+	return 0;
+}
+
+/* one pass of the scores on resident partials: the move descriptors, the (v, x) pairs, the matrix table and its lengths */
+static int nni_pass(phb_tlk *t, int nmoves, const int *moves, const double *t_central, double *out) {
+	const int N = t->N, C = t->C, S = t->S;
+	const size_t items = (size_t)N + nmoves;
+	phbc_nni_move *desc = (phbc_nni_move *)malloc(sizeof(phbc_nni_move) * (size_t)nmoves);
+	int *order = (int *)malloc(sizeof(int) * (size_t)nmoves);
+	int *groups = (int *)malloc(sizeof(int) * 2 * (size_t)nmoves);
+	double *bl = (double *)malloc(sizeof(double) * items);
+	double *ex = wants_host_exp(t) ? (double *)malloc(sizeof(double) * items * C * S) : NULL;
+	int rc = PHB_OK;
+	if (!desc || !order || !groups || !bl || (wants_host_exp(t) && !ex)) {
+		rc = fail(PHB_ENOMEM, "out of memory");
+		goto done;
+	}
+	for (int n = 0; n < N; n++) bl[n] = n == t->root ? 0.0 : t->bl[n];
+	for (int k = 0; k < nmoves; k++) {
+		const int x = moves[2 * k], y = moves[2 * k + 1], v = t->parent[y];
+		phbc_nni_move *m = &desc[k];
+		m->x = x, m->y = y, m->keep = sibling_of(t, y);
+		if (nni_kind(t, x, y) == 0) {
+			const int p = t->parent[v];
+			m->a = p == t->root ? -1 : N + p, m->a_mat = p, m->w = -1;
+		} else {
+			m->w = t->parent[x];
+			m->a = m->a_mat = sibling_of(t, x);
+		}
+		m->cmat = N + k, m->out = k;
+		bl[N + k] = t_central ? t_central[k] : t->bl[v];
+		order[k] = k;
+	}
+	g_nni_tlk = t, g_nni_moves = moves;
+	qsort(order, (size_t)nmoves, sizeof(int), nni_order);
+	int ngroups = 0;
+	for (int i = 0; i < nmoves; ngroups++) {
+		const int a = order[i], b = i + 1 < nmoves ? order[i + 1] : -1;
+		const int pair = b >= 0 && moves[2 * a] == moves[2 * b] && t->parent[moves[2 * a + 1]] == t->parent[moves[2 * b + 1]];
+		groups[2 * ngroups] = a, groups[2 * ngroups + 1] = pair ? b : -1;
+		i += pair ? 2 : 1;
+	}
+	if (ex)
+		for (size_t k = 0; k < items; k++)
+			for (int c = 0; c < C; c++)
+				for (int q = 0; q < S; q++) ex[(k * C + c) * S + q] = exp(t->h_eval[q] * (bl[k] * t->h_rates[c]));
+	phbc_eval_opts o;
+	fill_opts_resident(t, &o, 1);
+	if ((rc = phbc_nni_scores(t->ctx, &o, nmoves, desc, ngroups, groups, bl, ex, out))) rc = dev_fail(rc);
+done:
+	free(desc), free(order), free(groups), free(bl), free(ex);
+	return rc;
+}
+
+/*
+ * lnL and central-branch derivatives of every listed NNI neighbour from resident partials: lowers and uppers made resident
+ * (PHB_OPT_INCREMENTAL on, as phb_tlk_branch_hessian_diagonal's resident route), then one pass over them (phb_nni.cu).  NaN / inf as
+ * treelikelihood.c:1496-1519: an infinite lnL of the current tree, or a move whose unscaled site likelihood underflows, switches
+ * rescaling on and recomputes once.
+ */
+static int phb_tlk_nni_scores_impl(phb_tlk *t, int nmoves, const int *moves, const double *t_central, double *lnl, double *out) {
+	if (!moves || !out) return fail(PHB_EINVAL, "nni_scores: moves and out are required");
+	if (nmoves < 1) return fail(PHB_EINVAL, "nni_scores: %d moves (at least one is needed)", nmoves);
+	for (int k = 0; k < nmoves; k++) {
+		if (nni_kind(t, moves[2 * k], moves[2 * k + 1]) < 0)
+			return fail(PHB_EINVAL, "nni_scores: move %d (%d, %d) is not a nearest-neighbour interchange of the current tree", k, moves[2 * k],
+			            moves[2 * k + 1]);
+		if (t_central && !(t_central[k] >= 0))
+			return fail(PHB_EINVAL, "nni_scores: move %d central branch length = %E", k, t_central[k]);
+	}
+	if (t->have_matrices) return fail(PHB_ESTATE, "nni_scores needs the eigen system: explicit matrices cannot be re-evaluated at a new length");
+	int rc = check_ready(t);
+	if (rc) return rc;
+	if ((rc = phbc_nni_reserve(t->ctx, t->scale))) return dev_fail(rc);
+	if (!t->incremental) {
+		t->incremental = 1;
+		t->resident = 0;
+	}
+	double cur = 0.0;
+	for (int attempt = 0; attempt < 2; attempt++) {
+		if ((rc = resident_calculate(t, &cur))) return rc; /* retries with rescaling on itself */
+		if (isnan(cur) || isinf(cur)) break;
+		if ((rc = resident_uppers(t, -1, 0))) return rc;
+		if ((rc = nni_pass(t, nmoves, moves, t_central, out))) return rc;
+		int finite = 1;
+		for (int k = 0; k < 3 * nmoves; k++) finite &= isfinite(out[k]) != 0;
+		if (finite || t->scale) break;
+		t->scale = 1; /* a move's site likelihood underflowed unscaled: rescale everything and score again */
+		t->all_dirty = 1;
+	}
+	if (lnl) *lnl = cur;
+	if (isnan(cur) || isinf(cur))
+		for (int k = 0; k < 3 * nmoves; k++) out[k] = NAN;
+	return PHB_OK;
+}
+
+/*
  * tlk->update_partials(tlk, out, p1, m1, p2, m2) (treelikelihood.h:91; treelikelihoodX.c:1207 and friends): ONE partial update on the
  * resident buffers, by index like the reference's slot -- out = (P[m1] x[p1]) o (P[m2] x[p2]), p2 < 0: single child (the upper partial of
  * a child of the root, treelikelihood.c:2147).  Indices: < T tips, T..N-1 lower partials, N + node upper partials
@@ -2072,6 +2218,15 @@ int phb_tlk_calculate_branch(phb_tlk *t, int node, int nbl, const double *bl, do
 int phb_tlk_branch_hessian_diagonal(phb_tlk *t, double *lnl, double *grad, double *hess) {
 	nvtxRangePushA("phb_tlk_branch_hessian_diagonal");
 	const int rc = phb_tlk_branch_hessian_diagonal_impl(t, lnl, grad, hess);
+	nvtxRangePop();
+	return rc;
+}
+
+int phb_tlk_nni_moves(phb_tlk *t, int *moves) { return phb_tlk_nni_moves_impl(t, moves); }
+
+int phb_tlk_nni_scores(phb_tlk *t, int nmoves, const int *moves, const double *t_central, double *lnl, double *out) {
+	nvtxRangePushA("phb_tlk_nni_scores");
+	const int rc = phb_tlk_nni_scores_impl(t, nmoves, moves, t_central, lnl, out);
 	nvtxRangePop();
 	return rc;
 }

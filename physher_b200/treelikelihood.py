@@ -71,6 +71,8 @@ SYMBOLS = [
     ("phb_tlk_update_uppers", C.c_int, [C.c_void_p]),
     ("phb_tlk_calculate_branch", C.c_int, [C.c_void_p, C.c_int, C.c_int, _dp, _dp, _dp, _dp]),
     ("phb_tlk_branch_hessian_diagonal", C.c_int, [C.c_void_p, _dp, _dp, _dp]),
+    ("phb_tlk_nni_moves", C.c_int, [C.c_void_p, _ip]),
+    ("phb_tlk_nni_scores", C.c_int, [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp]),
     ("phb_tlk_update_partials", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _dp]),
     ("phb_tlk_get_partials", C.c_int, [C.c_void_p, C.c_int, _dp]),
     ("phb_tlk_get_matrices", C.c_int, [C.c_void_p, _dp, _dp]),
@@ -461,6 +463,31 @@ class SingleTreeLikelihood:
         grad, hess = np.zeros(self.N), np.zeros(self.N)
         self._check(self.lib.phb_tlk_branch_hessian_diagonal(self.h, C.byref(lnl), grad.ctypes.data_as(_dp), hess.ctypes.data_as(_dp)))
         return lnl.value, grad, hess
+
+    def nni_moves(self):
+        """The NNI neighbourhood of the current tree as moves (x, y), int32 [n, 2] (see phb_tlk_nni_moves; PHB_OPT_UNROOTED decides
+        whether the moves across the root replace the rooted moves at the root's children)."""
+        n = self.lib.phb_tlk_nni_moves(self.h, None)
+        if n < 0:
+            self._check(n)
+        moves = np.zeros((n, 2), dtype=np.int32)
+        if n:
+            self.lib.phb_tlk_nni_moves(self.h, moves.ctypes.data_as(_ip))
+        return moves
+
+    def nni_scores(self, moves=None, t_central=None):
+        """lnL, d lnL/dt_v and d2 lnL/dt_v2 of the tree each move (x, y) produces, its central branch (above v = parent[y]) at
+        t_central[k] (None: the current length), in one call on resident partials: (lnl of the current tree, out[n, 3]).
+        moves=None scores the whole neighbourhood, nni_moves()."""
+        m = self.nni_moves() if moves is None else np.ascontiguousarray(moves, dtype=np.int32).reshape(-1, 2)
+        tc = None if t_central is None else np.ascontiguousarray(t_central, dtype=np.float64).reshape(-1)
+        if tc is not None and tc.shape[0] != m.shape[0]:
+            raise ValueError("t_central needs one length per move")
+        out = np.zeros((m.shape[0], 3))
+        lnl = C.c_double(0.0)
+        self._check(self.lib.phb_tlk_nni_scores(self.h, int(m.shape[0]), m.ctypes.data_as(_ip), None if tc is None else tc.ctypes.data_as(_dp),
+                                                C.byref(lnl), out.ctypes.data_as(_dp)))
+        return lnl.value, out
 
     def update_partials(self, out, p1, m1, p2=-1, m2=-1, mirror=True):
         """tlk->update_partials(tlk, out, p1, m1, p2, m2) (treelikelihood.h:91) on the resident device buffers; returns the result."""
