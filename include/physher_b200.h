@@ -238,6 +238,41 @@ int phb_tlk_nni_scores(phb_tlk *tlk, int nmoves, const int *moves /* [nmoves][2]
                        double *lnl, double *out /* [nmoves][3] */);
 
 /*
+ * Subtree prune and regraft (the SPR moves the tree-search drivers score, spropt.c:1548-1615).  s is the root of the subtree to prune;
+ * neither s nor p = parent[s] may be the root.  b is the sibling of s, g = parent[p] and q the sibling of p.
+ *   pruned tree      p and the subtree of s removed; b takes p's slot (same side) under g.
+ *   target e         any node outside the subtree of s (s included) other than p and the root.
+ *   regrafted tree   from the pruned tree: p takes e's slot under e's pruned parent, e takes the slot of p that is not s's, s keeps its
+ *                    side under p.  Branch lengths stay with node ids, as in phb_tlk_set_topology.  e = b gives back the current tree,
+ *                    e = q the NNI move (q, b).
+ *
+ * phb_tlk_spr_targets writes the regraft targets of s into targets [count] (may be NULL) and returns the count, or PHB_EINVAL for an s
+ * that cannot be pruned.  With k tips below s: without PHB_OPT_UNROOTED every target but b, 2(T - k) - 3; with it (default) one target
+ * per distinct unrooted neighbour, 2(T - k) - 4 -- b, q when g is the root (b - q is then the current edge), and the right child of the
+ * root otherwise (the pruned tree's two root-child branches are one unrooted edge) are left out.
+ *
+ * phb_tlk_spr_scores: out[k] = {lnL, d lnL / dt_s, d2 lnL / dt_s2} of the tree regrafted on targets[k] (any valid target, b included),
+ * its pendant branch (above s) at t_pendant[k] (NULL: the current t_s) and every other branch at its current length, from one pass over
+ * the pruned tree -- no topology change.  With the pruned tree's upper and lower partials U~_e and L~_e (U~_e at the top of branch e;
+ * P_sib L~_sib when e's pruned parent is the root):
+ *   L_k = sum_c prop_c sum_i pi_i [(P_p U~_e) o (P_e L~_e)]_i (P_s L_s)_i
+ * and the derivatives replace P_s by r_c P'_s and r_c^2 P"_s, in the form sum w (L"/L - (L'/L)^2).  They are the exact ones:
+ * PHB_OPT_INCLUDE_ROOT_FREQS and PHB_OPT_COMPAT_SCALED_GRADIENT do not apply.  Under rescaling the per-pattern log factor is
+ * sf(U~_e) + sf(L~_e) + sf(L_s) (tips carry none).  *lnl (may be NULL) is the lnL of the current tree.
+ * The call switches PHB_OPT_INCREMENTAL on and writes the pruned tree's partials over the resident ones: the lowers of g and its
+ * ancestors below the root and the uppers of every node outside p and the subtree of s are marked invalid (the uppers of p and of the
+ * subtree of s stay valid).  The cached lnL of the current tree is unchanged: a following phb_tlk_calculate returns it bit for bit, and
+ * the next call that needs the lowers recomputes those of that path.  An infinite lnL of the current tree, or a target whose unscaled
+ * site likelihood is 0 or not finite, switches rescaling on and scores once more; a lnL still NaN or infinite NaN-fills out.
+ * PHB_EINVAL: an s that cannot be pruned, an invalid target (the message names its index), ntargets < 1, a negative t_pendant, NULL
+ * targets / out.  PHB_ESTATE with explicit matrices.  PHB_ENOMEM when the device cannot hold the resident partials or the call's
+ * matrix table; both are allocated before anything is overwritten, and the object stays usable.
+ */
+int phb_tlk_spr_targets(phb_tlk *tlk, int s, int *targets /* [count] or NULL */);
+int phb_tlk_spr_scores(phb_tlk *tlk, int s, int ntargets, const int *targets, const double *t_pendant /* [ntargets] or NULL */,
+                       double *lnl, double *out /* [ntargets][3] */);
+
+/*
  * phb_tlk_update_partials == the struct slot tlk->update_partials(tlk, out, p1, m1, p2, m2) (treelikelihood.h:91), for the callers
  * that drive it themselves: update_upper_partials[2] (treelikelihood.c:2129-2190, i.e. the non-virtual
  * SingleTreeLikelihood_update_uppers[2]), the tripod optimisation of SPR (spropt.c:1578-1608).  ONE partial update on the resident

@@ -10,7 +10,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libphysher_b200.so")
 
-CUDA_SOURCES = ["phb_cuda.cu", "phb_nuc4.cu", "phb_dmma.cu", "phb_dwalk.cu", "phb_timetree.cu", "phb_patterns.cu", "phb_branch.cu", "phb_nni.cu"]
+CUDA_SOURCES = ["phb_cuda.cu", "phb_nuc4.cu", "phb_dmma.cu", "phb_dwalk.cu", "phb_timetree.cu", "phb_patterns.cu", "phb_branch.cu", "phb_nni.cu",
+                "phb_spr.cu"]
 C_SOURCES = ["phb_treelikelihood.c", "phb_group.c", "phb_nccl.c"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

@@ -190,6 +190,15 @@ int phbc_nni_reserve(phbc_ctx *ctx, int scale);
  * (the 4-state kernel's work items) */
 int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmoves, const phbc_nni_move *moves, int ngroups, const int *groups,
                     const double *bl, const double *ex, double *out);
+/* Subtree prune and regraft (phb_spr.cu): out [ntargets][3] = lnL, d lnL/dt_s, d2 lnL/dt_s2 of the subtree of s (p = parent[s])
+ * regrafted on the branch above each target node, from the pruned tree's partials the caller left in the resident buffers (U~_e at
+ * N + e, L~_e at e); bl [N + ntargets] the matrix table's lengths (node n = entry n, target k's pendant length = entry N + k), ex (may
+ * be NULL) their exponentials [N + ntargets][C][S].  The resident buffers are those of phbc_nni_reserve. */
+/* the call's matrix table and sums, allocated before the pruned pass changes anything: -1 when the state count needs more shared
+ * memory than a CTA may have, -3 when the device cannot hold them */
+int phbc_spr_reserve(phbc_ctx *ctx, int ntargets);
+int phbc_spr_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int s, int p, int ntargets, const int *targets, const double *bl, const double *ex,
+                    double *out);
 int phbc_matrix_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, int nsets, const double *M_host, int skip_node, double *lnl, double *out_host);
 /* time-tree chain, batched (phb_timetree.cu) */
 int phbc_set_time_tree(phbc_ctx *ctx, const double *lowers, const int *parent, const int *preorder, const int *postorder);

@@ -1572,6 +1572,195 @@ static int phb_tlk_nni_scores_impl(phb_tlk *t, int nmoves, const int *moves, con
 }
 
 /*
+ * Subtree prune and regraft (spropt.c:1548-1615): the subtree of s is pruned together with p = parent[s] -- the sibling b of s takes
+ * p's slot under g = parent[p] -- and regrafted on the branch above a target e of the pruned tree: p takes e's slot, e the slot of p
+ * that is not s's.  s may be neither the root nor a child of the root; a target is any node outside the subtree of s other than p and
+ * the root.  Regrafting on b gives back the current tree.
+ */
+static int spr_check_prune(const phb_tlk *t, const char *fn, int s) {
+	if (s < 0 || s >= t->N || s == t->root || t->parent[s] == t->root)
+		return fail(PHB_EINVAL, "%s: node %d cannot be pruned (it must be neither the root %d nor a child of the root)", fn, s, t->root);
+	return PHB_OK;
+}
+
+/* mark [N] = 1 on the subtree of s, 0 elsewhere; stack [N] scratch */
+static void mark_subtree(const phb_tlk *t, int s, unsigned char *mark, int *stack) {
+	memset(mark, 0, t->N);
+	int sp = 0;
+	stack[sp++] = s;
+	while (sp) {
+		const int x = stack[--sp];
+		mark[x] = 1;
+		if (!is_tip(t, x)) stack[sp++] = t->left[x], stack[sp++] = t->right[x];
+	}
+}
+
+static int phb_tlk_spr_targets_impl(phb_tlk *t, int s, int *targets) {
+	int rc = spr_check_prune(t, "spr_targets", s);
+	if (rc) return rc;
+	unsigned char *mark = (unsigned char *)malloc(t->N);
+	int *stack = (int *)malloc(sizeof(int) * t->N);
+	if (!mark || !stack) {
+		free(mark), free(stack);
+		return fail(PHB_ENOMEM, "out of memory");
+	}
+	mark_subtree(t, s, mark, stack);
+	const int p = t->parent[s], g = t->parent[p], b = sibling_of(t, s);
+	/* unrooted: regrafting on q = sibling(p) when g is the root gives the current tree again (b and q then hang from the root, one
+	 * unrooted edge), and the pruned tree's two root-child branches are one unrooted edge otherwise -- drop the right one */
+	const int twin = !t->unrooted ? -1 : (g == t->root ? sibling_of(t, p) : t->right[t->root]);
+	int n = 0;
+	for (int e = 0; e < t->N; e++) {
+		if (e == t->root || e == p || mark[e] || e == b || e == twin) continue;
+		if (targets) targets[n] = e;
+		n++;
+	}
+	free(mark), free(stack);
+	return n;
+}
+
+/*
+ * One pass of the SPR scores: the pruned tree's partials over the resident buffers, then the contraction of every target (phb_spr.cu).
+ *   lowers  g's op becomes (b, b) o (q, q) on the side p had, every ancestor of g below the root takes its usual op (nothing when g is
+ *           the root; the root's own lower partial is never written);
+ *   uppers  the pruned tree's upper op of every node outside {p} and the subtree of s, grouped by their depth in the pruned tree.
+ * Current matrices (no rebuild), no root integration.  The validity maps lose exactly what the pass overwrites: lower_ok of g and its
+ * ancestors below the root (lower_stale: the next evaluation recomputes them, and the cached lnL stays that of the current tree) and
+ * upper_ok of every node it wrote; the uppers of p and of the subtree of s are untouched.
+ */
+static int spr_pass(phb_tlk *t, int s, int ntargets, const int *targets, const double *t_pendant, double *out) {
+	const int N = t->N, C = t->C, S = t->S, root = t->root;
+	const int p = t->parent[s], g = t->parent[p], b = sibling_of(t, s);
+	const size_t items = (size_t)N + ntargets;
+	int *queue = (int *)malloc(sizeof(int) * N);
+	int *depth = (int *)malloc(sizeof(int) * N);
+	double *bl = (double *)malloc(sizeof(double) * items);
+	double *ex = wants_host_exp(t) ? (double *)malloc(sizeof(double) * items * C * S) : NULL;
+	int rc = PHB_OK;
+	if (!queue || !depth || !bl || (wants_host_exp(t) && !ex)) {
+		rc = fail(PHB_ENOMEM, "out of memory");
+		goto done;
+	}
+	t->sweep_valid = 0;
+	phbc_eval_opts o;
+	int nops = 0;
+	for (int x = g; x != root; x = t->parent[x]) { /* one level each, children before parents */
+		int l = t->left[x], r = t->right[x];
+		if (x == g) *(l == p ? &l : &r) = b;
+		phbc_op *op = &t->sub_ops[nops];
+		op->out = x, op->a = op->a_mat = l, op->b = op->b_mat = r, op->flags = 0;
+		t->sub_level_off[nops] = nops;
+		nops++;
+		t->lower_ok[x] = 0;
+	}
+	t->sub_level_off[nops] = nops;
+	if (nops) {
+		t->lower_stale = 1;
+		fill_opts_resident(t, &o, 0);
+		if ((rc = phbc_run_ops(t->ctx, &o, nops, t->sub_ops, nops, t->sub_level_off, 0, 0, NULL))) {
+			rc = dev_fail(rc);
+			goto done;
+		}
+	}
+	/* uppers: breadth first over the pruned tree (p replaced by b), so that the ops come grouped by depth */
+	int head = 0, tail = 0, nlevels = 0;
+	nops = 0;
+	queue[tail++] = root;
+	depth[root] = 0;
+	while (head < tail) {
+		const int n = queue[head++];
+		if (is_tip(t, n)) continue;
+		int ch[2] = {t->left[n], t->right[n]};
+		for (int j = 0; j < 2; j++)
+			if (ch[j] == p) ch[j] = b;
+		for (int j = 0; j < 2; j++) {
+			const int x = ch[j], sib = ch[1 - j];
+			phbc_op *op = &t->sub_ops[nops++];
+			op->out = N + x;
+			if (n != root) /* u_x = (P_n u_n) o (P_sib L_sib) */
+				op->a = N + n, op->a_mat = n, op->b = op->b_mat = sib, op->flags = 0;
+			else /* u_x = P_sib L_sib */
+				op->a = op->a_mat = sib, op->b = op->b_mat = -1, op->flags = 1;
+			depth[x] = depth[n] + 1;
+			queue[tail++] = x;
+			t->upper_ok[x] = 0;
+		}
+	}
+	for (int k = 0; k < nops; k++)
+		if (k == 0 || depth[t->sub_ops[k].out - N] != depth[t->sub_ops[k - 1].out - N]) t->sub_level_off[nlevels++] = k;
+	t->sub_level_off[nlevels] = nops;
+	fill_opts_resident(t, &o, 1);
+	o.include_root_freqs = 0;
+	if ((rc = phbc_run_ops(t->ctx, &o, nops, t->sub_ops, nlevels, t->sub_level_off, 0, 0, NULL))) {
+		rc = dev_fail(rc);
+		goto done;
+	}
+	/* the matrix table: every node at its current length, then each target's pendant length */
+	for (int n = 0; n < N; n++) bl[n] = n == root ? 0.0 : t->bl[n];
+	for (int k = 0; k < ntargets; k++) bl[N + k] = t_pendant ? t_pendant[k] : t->bl[s];
+	if (ex)
+		for (size_t k = 0; k < items; k++)
+			for (int c = 0; c < C; c++)
+				for (int q = 0; q < S; q++) ex[(k * C + c) * S + q] = exp(t->h_eval[q] * (bl[k] * t->h_rates[c]));
+	fill_opts_resident(t, &o, 1);
+	if ((rc = phbc_spr_scores(t->ctx, &o, s, p, ntargets, targets, bl, ex, out))) rc = dev_fail(rc);
+done:
+	free(queue), free(depth), free(bl), free(ex);
+	return rc;
+}
+
+/*
+ * lnL and pendant-branch derivatives of the subtree of s regrafted on each listed target, from one pass over the pruned tree: lowers
+ * made resident (PHB_OPT_INCREMENTAL on), then spr_pass.  NaN / inf as phb_tlk_nni_scores: an infinite lnL of the current tree, or a
+ * target whose unscaled site likelihood underflows, switches rescaling on and scores once more.
+ */
+static int phb_tlk_spr_scores_impl(phb_tlk *t, int s, int ntargets, const int *targets, const double *t_pendant, double *lnl, double *out) {
+	int rc = spr_check_prune(t, "spr_scores", s);
+	if (rc) return rc;
+	if (!targets || !out) return fail(PHB_EINVAL, "spr_scores: targets and out are required");
+	if (ntargets < 1) return fail(PHB_EINVAL, "spr_scores: %d targets (at least one is needed)", ntargets);
+	unsigned char *mark = (unsigned char *)malloc(t->N);
+	int *stack = (int *)malloc(sizeof(int) * t->N);
+	if (!mark || !stack) {
+		free(mark), free(stack);
+		return fail(PHB_ENOMEM, "out of memory");
+	}
+	mark_subtree(t, s, mark, stack);
+	const int p = t->parent[s];
+	for (int k = 0; k < ntargets && !rc; k++) {
+		const int e = targets[k];
+		if (e < 0 || e >= t->N || e == t->root || e == p || mark[e])
+			rc = fail(PHB_EINVAL, "spr_scores: target %d (node %d) is not a regraft position of the subtree of %d", k, e, s);
+		else if (t_pendant && !(t_pendant[k] >= 0))
+			rc = fail(PHB_EINVAL, "spr_scores: target %d pendant branch length = %E", k, t_pendant[k]);
+	}
+	free(mark), free(stack);
+	if (rc) return rc;
+	if (t->have_matrices) return fail(PHB_ESTATE, "spr_scores needs the eigen system: explicit matrices cannot be re-evaluated at a new length");
+	if ((rc = check_ready(t))) return rc;
+	if ((rc = phbc_nni_reserve(t->ctx, t->scale)) || (rc = phbc_spr_reserve(t->ctx, ntargets))) return dev_fail(rc);
+	if (!t->incremental) {
+		t->incremental = 1;
+		t->resident = 0;
+	}
+	double cur = 0.0;
+	for (int attempt = 0; attempt < 2; attempt++) {
+		if ((rc = resident_calculate(t, &cur))) return rc; /* retries with rescaling on itself */
+		if (isnan(cur) || isinf(cur)) break;
+		if ((rc = spr_pass(t, s, ntargets, targets, t_pendant, out))) return rc;
+		int finite = 1;
+		for (int k = 0; k < 3 * ntargets; k++) finite &= isfinite(out[k]) != 0;
+		if (finite || t->scale) break;
+		t->scale = 1; /* a target's site likelihood underflowed unscaled: rescale everything and score again */
+		t->all_dirty = 1;
+	}
+	if (lnl) *lnl = cur;
+	if (isnan(cur) || isinf(cur))
+		for (int k = 0; k < 3 * ntargets; k++) out[k] = NAN;
+	return PHB_OK;
+}
+
+/*
  * tlk->update_partials(tlk, out, p1, m1, p2, m2) (treelikelihood.h:91; treelikelihoodX.c:1207 and friends): ONE partial update on the
  * resident buffers, by index like the reference's slot -- out = (P[m1] x[p1]) o (P[m2] x[p2]), p2 < 0: single child (the upper partial of
  * a child of the root, treelikelihood.c:2147).  Indices: < T tips, T..N-1 lower partials, N + node upper partials
@@ -2227,6 +2416,15 @@ int phb_tlk_nni_moves(phb_tlk *t, int *moves) { return phb_tlk_nni_moves_impl(t,
 int phb_tlk_nni_scores(phb_tlk *t, int nmoves, const int *moves, const double *t_central, double *lnl, double *out) {
 	nvtxRangePushA("phb_tlk_nni_scores");
 	const int rc = phb_tlk_nni_scores_impl(t, nmoves, moves, t_central, lnl, out);
+	nvtxRangePop();
+	return rc;
+}
+
+int phb_tlk_spr_targets(phb_tlk *t, int s, int *targets) { return phb_tlk_spr_targets_impl(t, s, targets); }
+
+int phb_tlk_spr_scores(phb_tlk *t, int s, int ntargets, const int *targets, const double *t_pendant, double *lnl, double *out) {
+	nvtxRangePushA("phb_tlk_spr_scores");
+	const int rc = phb_tlk_spr_scores_impl(t, s, ntargets, targets, t_pendant, lnl, out);
 	nvtxRangePop();
 	return rc;
 }

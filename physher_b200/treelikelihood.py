@@ -73,6 +73,8 @@ SYMBOLS = [
     ("phb_tlk_branch_hessian_diagonal", C.c_int, [C.c_void_p, _dp, _dp, _dp]),
     ("phb_tlk_nni_moves", C.c_int, [C.c_void_p, _ip]),
     ("phb_tlk_nni_scores", C.c_int, [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp]),
+    ("phb_tlk_spr_targets", C.c_int, [C.c_void_p, C.c_int, _ip]),
+    ("phb_tlk_spr_scores", C.c_int, [C.c_void_p, C.c_int, C.c_int, _ip, _dp, _dp, _dp]),
     ("phb_tlk_update_partials", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _dp]),
     ("phb_tlk_get_partials", C.c_int, [C.c_void_p, C.c_int, _dp]),
     ("phb_tlk_get_matrices", C.c_int, [C.c_void_p, _dp, _dp]),
@@ -487,6 +489,31 @@ class SingleTreeLikelihood:
         lnl = C.c_double(0.0)
         self._check(self.lib.phb_tlk_nni_scores(self.h, int(m.shape[0]), m.ctypes.data_as(_ip), None if tc is None else tc.ctypes.data_as(_dp),
                                                 C.byref(lnl), out.ctypes.data_as(_dp)))
+        return lnl.value, out
+
+    def spr_targets(self, s):
+        """The regraft targets of the subtree of s, int32 [n] (see phb_tlk_spr_targets; PHB_OPT_UNROOTED decides whether targets that
+        give the same unrooted tree are listed once)."""
+        n = self.lib.phb_tlk_spr_targets(self.h, int(s), None)
+        if n < 0:
+            self._check(n)
+        targets = np.zeros(n, dtype=np.int32)
+        if n:
+            self.lib.phb_tlk_spr_targets(self.h, int(s), targets.ctypes.data_as(_ip))
+        return targets
+
+    def spr_scores(self, s, targets=None, t_pendant=None):
+        """lnL, d lnL/dt_s and d2 lnL/dt_s2 of the tree the subtree of s (pruned with its parent) regrafted on the branch above each
+        target gives, its pendant branch (above s) at t_pendant[k] (None: the current length), in one call on resident partials:
+        (lnl of the current tree, out[n, 3]).  targets=None scores every target of spr_targets(s)."""
+        tg = self.spr_targets(s) if targets is None else np.ascontiguousarray(targets, dtype=np.int32).reshape(-1)
+        tp = None if t_pendant is None else np.ascontiguousarray(t_pendant, dtype=np.float64).reshape(-1)
+        if tp is not None and tp.shape[0] != tg.shape[0]:
+            raise ValueError("t_pendant needs one length per target")
+        out = np.zeros((tg.shape[0], 3))
+        lnl = C.c_double(0.0)
+        self._check(self.lib.phb_tlk_spr_scores(self.h, int(s), int(tg.shape[0]), tg.ctypes.data_as(_ip),
+                                                None if tp is None else tp.ctypes.data_as(_dp), C.byref(lnl), out.ctypes.data_as(_dp)))
         return lnl.value, out
 
     def update_partials(self, out, p1, m1, p2=-1, m2=-1, mirror=True):
