@@ -179,8 +179,9 @@ int phb_tlk_category_gradient(phb_tlk *tlk, double *out /* [C] */);
  *
  * phb_tlk_calculate_branch == _calculate_uppper (treelikelihood.c:2592-2686) + calculate_dldt_uppper (:2195-2262) +
  * d2lnldt2_uppper (:2267-2335): lnL and its first and second derivative with respect to the length of the branch above `node`,
- * at `nbl` candidate lengths in ONE launch, from the upper partial of `node`, its lower partial and fresh P, P', P" -- every other
+ * at `nbl` candidate lengths in ONE pass, from the upper partial of `node`, its lower partial and fresh P, P', P" -- every other
  * branch at its current length (pending set_branch_length changes are applied first, recomputing only the partials they reach).
+ * The number of candidate lengths is not limited (past 65,535 the score kernel takes one more launch per 65,535).
  * The object's own branch lengths are not changed; the caller keeps the length it chooses with phb_tlk_set_branch_length.
  * Output pointers may be NULL.
  */

@@ -1,4 +1,4 @@
-// phb_branch.cu -- single-branch fast path on resident upper / lower partials.
+// phb_branch.cu -- single-branch fast path on resident upper / lower partials, and the frame every score pass shares (phb_score.cuh).
 //
 // Replaces, for one branch at a time, the reference's "upper likelihood" functions used by Brent / Newton branch optimisation,
 // NNI / SPR and Model.d2logP:
@@ -9,14 +9,15 @@
 //   L_k(t)  = sum_c prop_c sum_i pi_i U_n[c,k,i] (P(r_c t) L_n[c,k])_i          lnL   = sum_k w_k (log L_k + sf_k)
 //   L'_k(t) = sum_c prop_c r_c   sum_i pi_i U_n[c,k,i] (P'(r_c t) L_n[c,k])_i   lnL'  = sum_k w_k L'_k / L_k
 //   L"_k(t) = sum_c prop_c r_c^2 sum_i pi_i U_n[c,k,i] (P"(r_c t) L_n[c,k])_i   lnL"  = sum_k w_k (L"_k L_k - L'_k^2) / L_k^2
-// The reference evaluates one candidate length per call, each a full pass over two partials buffers; here ONE launch takes a list
+// The reference evaluates one candidate length per call, each a full pass over two partials buffers; here ONE pass takes a list
 // of (node, length) items: one node at a vector of candidate lengths (a bracketing step or a line search, whose CTAs read the same
 // two buffers concurrently and share them through L2), or every non-root node at its own length (the diagonal of the
-// branch-length Hessian, phb_tlk_branch_hessian_diagonal, with the gradient and lnL of the same pass).
+// branch-length Hessian, phb_tlk_branch_hessian_diagonal, with the gradient and lnL of the same pass).  Items go on grid.y in
+// launches of at most 65,535, so any number of them works.
 //
 // Under rescaling the per-pattern log factor is sf_upper[n] + sf_lower[n] (the factors that were divided out of U_n and L_n);
 // the derivative ratios are scale free.
-#include "phb_ctx.cuh"
+#include "phb_score.cuh"
 
 #include <math.h>
 #include <stdlib.h>
@@ -108,23 +109,9 @@ __global__ void __launch_bounds__(BR_THREADS) k_branch_lnl(Bufs b, const int *__
 			plk += b.sf[(size_t)(b.N + node) * b.P + p];
 			if (!tip) plk += b.sf[(size_t)node * b.P + p];
 		}
-		v[0] = plk * w;
-		const double r1 = dL / L;
-		v[1] = r1 * w;
-		// treelikelihood.c:2331 forms (L" L - L'^2) / L^2, which underflows to 0 / 0 once L_k < 1e-154 -- site likelihoods a tree of a
-		// thousand taxa reaches without rescaling; the ratio form is the same value and stays finite
-		v[2] = (d2L / L - r1 * r1) * w;
+		score_terms(plk, L, dL, d2L, w, v);
 	}
-	for (int q = 0; q < 3; q++) {
-		const double s = phb_warp_sum(v[q]);
-		if ((threadIdx.x & 31) == 0) red[q][threadIdx.x >> 5] = s;
-	}
-	__syncthreads();
-	if (threadIdx.x < 3) {
-		double s = 0.0;
-		for (int w = 0; w < BR_THREADS / 32; w++) s += red[threadIdx.x][w];
-		partial[((size_t)k * 3 + threadIdx.x) * gridDim.x + blockIdx.x] = s;
-	}
+	score_block_sum(red, v, BR_THREADS / 32, k, partial);
 }
 
 // out[row] = sum of partial[row][0..n): one CTA per row, fixed order
@@ -143,14 +130,65 @@ __global__ void k_branch_sum(const double *__restrict__ partial, int n, double *
 	}
 }
 
+int phbc_score_resident(const phbc_ctx *ctx, const phbc_eval_opts *o) {
+	if (!ctx->d_upper || !ctx->d_lower || (o->scale && !ctx->d_sf) || (ctx->tip_kind != PHBC_TIP_STATES && !ctx->d_tip_partials)) {
+		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "upper / lower partials are not resident");
+		return -4;
+	}
+	return 0;
+}
+
+// grows ctx->d_branch to the pass's layout (the stream is drained before the old buffer goes) and carves it
+int phbc_score_scratch(phbc_ctx *ctx, size_t items, size_t nout, size_t tiles, size_t desc_bytes, ScoreScratch *sc) {
+	const size_t S = ctx->S, C = ctx->C;
+	const size_t need = (items * (1 + C * 3 * S * S + C * S) + nout * (3 + 3 * tiles) + (desc_bytes + 7) / 8) * sizeof(double);
+	if (need > ctx->branch_bytes) {
+		PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
+		if (ctx->d_branch) cudaFree(ctx->d_branch);
+		ctx->d_branch = NULL;
+		ctx->branch_bytes = 0;
+		int rc = phbc_alloc(ctx, &ctx->d_branch, need / sizeof(double), false);
+		if (rc) return rc;
+		ctx->branch_bytes = need;
+	}
+	sc->bl = ctx->d_branch;
+	sc->out = sc->bl + items;
+	sc->mats = sc->out + 3 * nout;
+	sc->part = sc->mats + items * C * 3 * S * S;
+	sc->ex = sc->part + nout * 3 * tiles;
+	sc->desc = sc->ex + items * C * S;
+	return 0;
+}
+
+// the matrix table: items lengths (and, ex_host not NULL, their exponentials [items][C][S]) up, P, r P', r^2 P" of each
+int phbc_score_matrices(phbc_ctx *ctx, const ScoreScratch &sc, size_t items, const double *bl_host, const double *ex_host) {
+	const int S = ctx->S, C = ctx->C;
+	PHBC_CHECK(cudaMemcpyAsync(sc.bl, bl_host, items * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+	if (ex_host) PHBC_CHECK(cudaMemcpyAsync(sc.ex, ex_host, items * C * S * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+	const int threads = S * S >= 256 ? 256 : (S * S >= 64 ? 64 : 32);
+	k_branch_matrices<<<dim3((unsigned)items, (unsigned)C), threads, 3 * S * sizeof(double), ctx->stream>>>(S, C, ctx->d_evec, ctx->d_eval, ctx->d_ivec, sc.bl,
+	                                                                                                  ctx->d_rates, ex_host ? sc.ex : NULL, sc.mats);
+	ctx->launches++;
+	return 0;
+}
+
+// out_host [nout][3] = the per-CTA sums [nout][3][tiles] summed in a fixed order; synchronous
+int phbc_score_finish(phbc_ctx *ctx, const ScoreScratch &sc, size_t nout, size_t tiles, double *out_host) {
+	k_branch_sum<<<(unsigned)(3 * nout), 256, 0, ctx->stream>>>(sc.part, (int)tiles, sc.out);
+	ctx->launches++;
+	PHBC_CHECK(cudaGetLastError());
+	PHBC_CHECK(cudaMemcpyAsync(out_host, sc.out, 3 * nout * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+	PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
+	return 0;
+}
+
 // out_host [nitems][3]: lnL, d lnL / dt, d2 lnL / dt2 of the branch above nodes[k] at length bl[k]; U and L of every listed node must be
 // resident.  One node repeated: candidate lengths of one branch; distinct nodes: one entry per branch.
 extern "C" int phbc_branch_lnl(phbc_ctx *ctx, const phbc_eval_opts *o, int nitems, const int *nodes_host, const double *bl_host, const double *ex_host,
                                double *out_host) {
 	PHBC_CHECK(cudaSetDevice(ctx->device));
-	const size_t S = ctx->S, C = ctx->C, P = ctx->P;
-	if (nitems < 1 || nitems > 65535) {
-		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "%d branch items: out of range (1 .. 65535 per launch)", nitems);
+	if (nitems < 1) {
+		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "%d branch items: at least one is needed", nitems);
 		return -1;
 	}
 	if (!ctx->have_eigen || o->explicit_matrices) {
@@ -163,43 +201,26 @@ extern "C" int phbc_branch_lnl(phbc_ctx *ctx, const phbc_eval_opts *o, int nitem
 			snprintf(phbc_errbuf, sizeof(phbc_errbuf), "branch %d (root %d): out of range", node, ctx->root);
 			return -1;
 		}
-		if (!ctx->d_upper || (node >= ctx->T && !ctx->d_lower) || (o->scale && !ctx->d_sf) ||
-		    (node < ctx->T && ctx->tip_kind != PHBC_TIP_STATES && !ctx->d_tip_partials)) {
-			snprintf(phbc_errbuf, sizeof(phbc_errbuf), "upper / lower partials are not resident");
-			return -4;
-		}
 	}
-	const size_t n = (size_t)nitems;
-	const size_t tiles = (P + BR_THREADS - 1) / BR_THREADS;
-	// scratch: bl [n] | results [n][3] | matrices [n][C][3][S*S] | partial [n][3][tiles] | host exponentials [n][C][S] | nodes [n] (int)
-	const size_t need = (n * (4 + C * 3 * S * S + 3 * tiles + C * S) + (n + 1) / 2) * sizeof(double);
-	if (need > ctx->branch_bytes) {
-		PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
-		if (ctx->d_branch) cudaFree(ctx->d_branch);
-		ctx->d_branch = NULL;
-		ctx->branch_bytes = 0;
-		PHBC_CHECK(cudaMalloc((void **)&ctx->d_branch, need));
-		ctx->branch_bytes = need;
-	}
-	double *d_bl = ctx->d_branch, *d_out = d_bl + n, *d_mats = d_out + 3 * n, *d_part = d_mats + n * C * 3 * S * S;
-	double *d_exbuf = d_part + n * 3 * tiles;
-	double *d_ex = ex_host ? d_exbuf : NULL;
-	int *d_nodes = reinterpret_cast<int *>(d_exbuf + n * C * S);
-	PHBC_CHECK(cudaMemcpyAsync(d_bl, bl_host, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-	PHBC_CHECK(cudaMemcpyAsync(d_nodes, nodes_host, n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-	if (ex_host) PHBC_CHECK(cudaMemcpyAsync(d_ex, ex_host, n * C * S * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-	const int mthreads = S * S >= 256 ? 256 : (S * S >= 64 ? 64 : 32);
-	k_branch_matrices<<<dim3((unsigned)n, (unsigned)C), mthreads, 3 * S * sizeof(double), ctx->stream>>>((int)S, (int)C, ctx->d_evec, ctx->d_eval, ctx->d_ivec,
-	                                                                                                d_bl, ctx->d_rates, d_ex, d_mats);
+	int rc;
+	if ((rc = phbc_score_resident(ctx, o))) return rc;
+	const size_t S = ctx->S, C = ctx->C, n = (size_t)nitems;
+	const size_t tiles = ((size_t)ctx->P + BR_THREADS - 1) / BR_THREADS;
+	ScoreScratch sc;
+	if ((rc = phbc_score_scratch(ctx, n, n, tiles, n * sizeof(int), &sc))) return rc;
+	const int *d_nodes = static_cast<int *>(sc.desc);
+	PHBC_CHECK(cudaMemcpyAsync(sc.desc, nodes_host, n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+	if ((rc = phbc_score_matrices(ctx, sc, n, bl_host, ex_host))) return rc;
 	const size_t smem = 3 * S * S * sizeof(double);
 	if (smem > 48 * 1024) PHBC_CHECK(cudaFuncSetAttribute(k_branch_lnl, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 	Bufs b = phbc_make_bufs(ctx);
-	k_branch_lnl<<<dim3((unsigned)tiles, (unsigned)n), BR_THREADS, smem, ctx->stream>>>(b, d_nodes, d_mats, ctx->d_freqs, ctx->d_props, ctx->d_weights,
-	                                                                                   o->scale, d_part);
-	k_branch_sum<<<(unsigned)(3 * n), 256, 0, ctx->stream>>>(d_part, (int)tiles, d_out);
-	ctx->launches += 3;
-	PHBC_CHECK(cudaGetLastError());
-	PHBC_CHECK(cudaMemcpyAsync(out_host, d_out, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-	PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
-	return 0;
+	if ((rc = phbc_time_begin(ctx))) return rc;
+	for (size_t k0 = 0; k0 < n; k0 += 65535) {  // items k0 .. k0 + cnt - 1: their nodes, matrices and sums
+		const unsigned cnt = (unsigned)(n - k0 < 65535 ? n - k0 : 65535);
+		k_branch_lnl<<<dim3((unsigned)tiles, cnt), BR_THREADS, smem, ctx->stream>>>(b, d_nodes + k0, sc.mats + k0 * C * 3 * S * S, ctx->d_freqs,
+		                                                                           ctx->d_props, ctx->d_weights, o->scale, sc.part + k0 * 3 * tiles);
+		ctx->launches++;
+	}
+	if ((rc = phbc_time_end(ctx))) return rc;
+	return phbc_score_finish(ctx, sc, n, tiles, out_host);
 }

@@ -38,7 +38,7 @@ struct phbc_ctx {
 	phbc_op *d_lower_ops, *d_upper_ops;
 	phbc_op *d_sub_ops;      // op list of a partial re-evaluation (phbc_run_ops)
 	int sub_ops_cap;
-	double *d_branch;        // single-branch scratch: candidate lengths, matrices, per-CTA sums, results (phb_branch.cu)
+	double *d_branch;        // score-pass scratch: matrix-table lengths, matrices, per-CTA sums, results, descriptors (phb_score.cuh)
 	size_t branch_bytes;
 	phbc_parent_op *d_parent_ops;
 	int n_lower_ops, n_upper_ops, n_parent_ops;
@@ -144,6 +144,8 @@ extern thread_local char phbc_errbuf[512];
 	} while (0)
 
 int phbc_ensure_scratch(phbc_ctx *ctx, size_t bytes);
+// cudaMalloc of count doubles (zero: cleared on the stream); device exhaustion is -3, with the error it leaves cleared
+int phbc_alloc(phbc_ctx *ctx, double **p, size_t count, bool zero);
 
 // generic node-at-a-time path (phb_cuda.cu)
 int phbc_generic_evaluate(phbc_ctx *ctx, const phbc_eval_opts *o);
@@ -158,7 +160,6 @@ struct Bufs {
 };
 Bufs phbc_make_bufs(phbc_ctx *ctx);
 int phbc_generic_prepare(phbc_ctx *ctx, const phbc_eval_opts *o);                       // buffers + transition matrices
-int phbc_generic_buffers(phbc_ctx *ctx, const phbc_eval_opts *o);                       // buffers only (lazy)
 int phbc_generic_scale_ops(phbc_ctx *ctx, const phbc_op *d_ops, int count, double threshold);  // K5 on one level
 int phbc_generic_root(phbc_ctx *ctx, const phbc_eval_opts *o, double *result);           // K6, K7 -> result[0]
 int phbc_generic_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, double *result);       // K9, K10, A11 from materialised uppers

@@ -714,6 +714,19 @@ static int phbc_launch_transition_matrices(phbc_ctx *ctx, int batch_index) {
 	return 0;
 }
 
+int phbc_alloc(phbc_ctx *ctx, double **p, size_t count, bool zero) {
+	const cudaError_t e = cudaMalloc((void **)p, count * sizeof(double));
+	if (e == cudaErrorMemoryAllocation) {
+		(void)cudaGetLastError();
+		*p = NULL;
+		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "out of device memory: %.2f GB requested", count * 8.0 / 1e9);
+		return -3;
+	}
+	PHBC_CHECK(e);
+	if (zero) PHBC_CHECK(cudaMemsetAsync(*p, 0, count * sizeof(double), ctx->stream));
+	return 0;
+}
+
 // buffers of the node-at-a-time paths (lazy) and the per-node transition matrices
 int phbc_generic_buffers(phbc_ctx *ctx, const phbc_eval_opts *o) {
 	PHBC_CHECK(cudaSetDevice(ctx->device));
@@ -722,18 +735,10 @@ int phbc_generic_buffers(phbc_ctx *ctx, const phbc_eval_opts *o) {
 	// zero-initialised, with a zeroed tail: the tensor-core kernels stage whole k-chunks without predicates and may read a few
 	// doubles past a row (into the next row / block) -- always finite values that meet zero-padded matrix columns
 	const size_t tail = 64;
-	if (!ctx->d_lower) {
-		PHBC_CHECK(cudaMalloc((void **)&ctx->d_lower, ((N - T) * psize + tail) * sizeof(double)));
-		PHBC_CHECK(cudaMemsetAsync(ctx->d_lower, 0, ((N - T) * psize + tail) * sizeof(double), ctx->stream));
-	}
-	if (o->want_gradient && !ctx->d_upper) {
-		PHBC_CHECK(cudaMalloc((void **)&ctx->d_upper, (N * psize + tail) * sizeof(double)));
-		PHBC_CHECK(cudaMemsetAsync(ctx->d_upper, 0, (N * psize + tail) * sizeof(double), ctx->stream));
-	}
-	if (o->scale && !ctx->d_sf) {
-		PHBC_CHECK(cudaMalloc((void **)&ctx->d_sf, 2 * N * P * sizeof(double)));
-		PHBC_CHECK(cudaMemsetAsync(ctx->d_sf, 0, 2 * N * P * sizeof(double), ctx->stream));
-	}
+	int rc;
+	if (!ctx->d_lower && (rc = phbc_alloc(ctx, &ctx->d_lower, (N - T) * psize + tail, true))) return rc;
+	if (o->want_gradient && !ctx->d_upper && (rc = phbc_alloc(ctx, &ctx->d_upper, N * psize + tail, true))) return rc;
+	if (o->scale && !ctx->d_sf && (rc = phbc_alloc(ctx, &ctx->d_sf, 2 * N * P, true))) return rc;
 	return 0;
 }
 

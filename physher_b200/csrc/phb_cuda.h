@@ -162,6 +162,9 @@ int phbc_run_ops(phbc_ctx *ctx, const phbc_eval_opts *o, int nops, const phbc_op
 int phbc_root_frequency_gradient(phbc_ctx *ctx, double *out /* [S] */);
 /* d lnL / d prop_c at fixed conditional likelihoods, from the same root partial (root term of gradient_pinv_sitemodel, treelikelihood.c:2943-3001) */
 int phbc_root_category_gradient(phbc_ctx *ctx, double *out /* [C] */);
+/* the node-at-a-time buffers, allocated lazily (zero-filled): lowers, uppers with want_gradient, scale factors with scale; -3 when the
+ * device cannot hold them */
+int phbc_generic_buffers(phbc_ctx *ctx, const phbc_eval_opts *o);
 /* K9 / K10 / A11 over every branch from resident upper and lower partials (results in slot 0; lnL slot untouched) */
 int phbc_resident_gradient(phbc_ctx *ctx, const phbc_eval_opts *o);
 /* single-branch fast path (phb_branch.cu) on resident upper / lower partials: out [nitems][3] = lnL, d lnL/dt, d2 lnL/dt2 of the branch
@@ -183,8 +186,6 @@ typedef struct phbc_nni_move {
 	int cmat;       /* table entry of the central branch (P, P', P")                                                   */
 	int out;        /* output row                                                                                      */
 } phbc_nni_move;
-/* device buffers the scores read, allocated before the resident evaluation: -3 when the device cannot hold them */
-int phbc_nni_reserve(phbc_ctx *ctx, int scale);
 /* out [nmoves][3] = lnL, d lnL/dt_v, d2 lnL/dt_v2 of each exchanged tree from resident upper / lower partials; bl [N + nmoves] the matrix
  * table's lengths, ex (may be NULL) their exponentials [N + nmoves][C][S]; groups [ngroups][2] move pairs sharing (v, x), -1 = none
  * (the 4-state kernel's work items) */
@@ -193,7 +194,7 @@ int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmoves, const ph
 /* Subtree prune and regraft (phb_spr.cu): out [ntargets][3] = lnL, d lnL/dt_s, d2 lnL/dt_s2 of the subtree of s (p = parent[s])
  * regrafted on the branch above each target node, from the pruned tree's partials the caller left in the resident buffers (U~_e at
  * N + e, L~_e at e); bl [N + ntargets] the matrix table's lengths (node n = entry n, target k's pendant length = entry N + k), ex (may
- * be NULL) their exponentials [N + ntargets][C][S].  The resident buffers are those of phbc_nni_reserve. */
+ * be NULL) their exponentials [N + ntargets][C][S]. */
 /* the call's matrix table and sums, allocated before the pruned pass changes anything: -1 when the state count needs more shared
  * memory than a CTA may have, -3 when the device cannot hold them */
 int phbc_spr_reserve(phbc_ctx *ctx, int ntargets);

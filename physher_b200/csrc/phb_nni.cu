@@ -13,17 +13,11 @@
 //              operand messages stay in registers, the group's matrices of one category are staged in shared memory;
 //   any S      k_nni_operands writes A o M_y and M_keep o M_x of a chunk of moves to scratch, k_nni_contract contracts them.
 // Per-CTA partial sums [move][3][tile] go through k_branch_sum (phb_branch.cu): fixed order, bit-identical from run to run.
-#include "phb_ctx.cuh"
+#include "phb_score.cuh"
 
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
-
-// phb_branch.cu
-__global__ void k_branch_matrices(int S, int C, const double *__restrict__ evec, const double *__restrict__ eval, const double *__restrict__ ivec,
-                                  const double *__restrict__ bl, const double *__restrict__ rates, const double *__restrict__ ex_host,
-                                  double *__restrict__ mats);
-__global__ void k_branch_sum(const double *__restrict__ partial, int n, double *__restrict__ out);
 
 #define NNI_THREADS 128
 #define NNI_SLOTS 11  // matrices of a group and category: P_x, P_y0, P_keep0, P_A, P_w, then P, P', P" of each of the two moves
@@ -158,9 +152,10 @@ __global__ void __launch_bounds__(NNI_THREADS) k_nni_score(Bufs b, const int2 *_
 			const double r1 = acc[j][1] / L;
 			v[3 * j] = plk * w;
 			v[3 * j + 1] = r1 * w;
-			v[3 * j + 2] = (acc[j][2] / L - r1 * r1) * w;
+			v[3 * j + 2] = (acc[j][2] / L - r1 * r1) * w;  // the ratio form of score_terms
 		}
 	}
+	// the block sum of score_block_sum, six terms into two rows (written out: the shared helpers change this kernel's code)
 	for (int q = 0; q < 6; q++) {
 		const double s = phb_warp_sum(v[q]);
 		if ((threadIdx.x & 31) == 0) red[q][threadIdx.x >> 5] = s;
@@ -253,48 +248,9 @@ __global__ void __launch_bounds__(NNI_THREADS) k_nni_contract(Bufs b, const phbc
 		const double w = weights[p];
 		double plk = log(L);
 		if (scale) plk += nni_log_factor(b, m, p);
-		v[0] = plk * w;
-		const double r1 = dL / L;
-		v[1] = r1 * w;
-		v[2] = (d2L / L - r1 * r1) * w;
+		score_terms(plk, L, dL, d2L, w, v);
 	}
-	for (int q = 0; q < 3; q++) {
-		const double s = phb_warp_sum(v[q]);
-		if ((threadIdx.x & 31) == 0) red[q][threadIdx.x >> 5] = s;
-	}
-	__syncthreads();
-	if (threadIdx.x < 3) {
-		double s = 0.0;
-		for (int w = 0; w < NNI_THREADS / 32; w++) s += red[threadIdx.x][w];
-		partial[((size_t)m.out * 3 + threadIdx.x) * gridDim.x + blockIdx.x] = s;
-	}
-}
-
-// device allocation that reports exhaustion as -3 (and clears the error it leaves) instead of a CUDA failure
-static int nni_alloc(phbc_ctx *ctx, double **p, size_t count, bool zero) {
-	const cudaError_t e = cudaMalloc((void **)p, count * sizeof(double));
-	if (e == cudaErrorMemoryAllocation) {
-		(void)cudaGetLastError();
-		*p = NULL;
-		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "out of device memory: %.1f GB for resident partials or NNI scratch", count * 8.0 / 1e9);
-		return -3;
-	}
-	PHBC_CHECK(e);
-	if (zero) PHBC_CHECK(cudaMemsetAsync(*p, 0, count * sizeof(double), ctx->stream));
-	return 0;
-}
-
-// the resident node-at-a-time buffers the scores read, allocated up front (as phbc_generic_buffers lays them out) so that a device too
-// small for them is reported as -3 before anything changes
-extern "C" int phbc_nni_reserve(phbc_ctx *ctx, int scale) {
-	PHBC_CHECK(cudaSetDevice(ctx->device));
-	const size_t S = ctx->S, C = ctx->C, P = ctx->P, N = ctx->N, T = ctx->T;
-	const size_t psize = C * P * S, tail = 64;
-	int rc;
-	if (!ctx->d_lower && (rc = nni_alloc(ctx, &ctx->d_lower, (N - T) * psize + tail, true))) return rc;
-	if (!ctx->d_upper && (rc = nni_alloc(ctx, &ctx->d_upper, N * psize + tail, true))) return rc;
-	if (scale && !ctx->d_sf && (rc = nni_alloc(ctx, &ctx->d_sf, 2 * N * P, true))) return rc;
-	return 0;
+	score_block_sum(red, v, NNI_THREADS / 32, m.out, partial);
 }
 
 // out_host [nmoves][3]; bl_host [N + nmoves]: every node's length (root entry unused), then each move's central length; ex_host
@@ -311,45 +267,23 @@ extern "C" int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmove
 		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "NNI scores need the eigen system (explicit matrices cannot be re-evaluated at a new length)");
 		return -4;
 	}
-	if (!ctx->d_upper || !ctx->d_lower || (o->scale && !ctx->d_sf) || (ctx->tip_kind != PHBC_TIP_STATES && !ctx->d_tip_partials)) {
-		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "upper / lower partials are not resident");
-		return -4;
-	}
+	int rc;
+	if ((rc = phbc_score_resident(ctx, o))) return rc;
 	const size_t n = (size_t)nmoves, items = N + n;
 	const size_t tiles = (P + NNI_THREADS - 1) / NNI_THREADS;
-	const size_t desc = (n * sizeof(phbc_nni_move) + 2 * (size_t)ngroups * sizeof(int) + 7) / 8;
-	// scratch: bl [items] | results [n][3] | matrices [items][C][3][S*S] | partial [n][3][tiles] | host exponentials [items][C][S] |
-	// groups and move descriptors
-	const size_t need = (items * (1 + C * 3 * S * S + C * S) + n * (3 + 3 * tiles) + desc) * sizeof(double);
-	if (need > ctx->branch_bytes) {
-		PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
-		if (ctx->d_branch) cudaFree(ctx->d_branch);
-		ctx->d_branch = NULL;
-		ctx->branch_bytes = 0;
-		int rc = nni_alloc(ctx, &ctx->d_branch, need / sizeof(double), false);
-		if (rc) return rc;
-		ctx->branch_bytes = need;
-	}
-	double *d_bl = ctx->d_branch, *d_out = d_bl + items, *d_mats = d_out + 3 * n, *d_part = d_mats + items * C * 3 * S * S;
-	double *d_exbuf = d_part + n * 3 * tiles;
-	double *d_ex = ex_host ? d_exbuf : NULL;
-	int2 *d_groups = reinterpret_cast<int2 *>(d_exbuf + items * C * S);  // 8-byte aligned; the 32-byte descriptors follow
+	ScoreScratch sc;
+	if ((rc = phbc_score_scratch(ctx, items, n, tiles, 2 * (size_t)ngroups * sizeof(int) + n * sizeof(phbc_nni_move), &sc))) return rc;
+	int2 *d_groups = static_cast<int2 *>(sc.desc);  // the 32-byte descriptors follow
 	phbc_nni_move *d_moves = reinterpret_cast<phbc_nni_move *>(d_groups + ngroups);
-	PHBC_CHECK(cudaMemcpyAsync(d_bl, bl_host, items * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
 	PHBC_CHECK(cudaMemcpyAsync(d_moves, moves_host, n * sizeof(phbc_nni_move), cudaMemcpyHostToDevice, ctx->stream));
 	if (ngroups > 0) PHBC_CHECK(cudaMemcpyAsync(d_groups, groups_host, 2 * (size_t)ngroups * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-	if (ex_host) PHBC_CHECK(cudaMemcpyAsync(d_ex, ex_host, items * C * S * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-	const int mthreads = S * S >= 256 ? 256 : (S * S >= 64 ? 64 : 32);
-	k_branch_matrices<<<dim3((unsigned)items, (unsigned)C), mthreads, 3 * S * sizeof(double), ctx->stream>>>((int)S, (int)C, ctx->d_evec, ctx->d_eval,
-	                                                                                                    ctx->d_ivec, d_bl, ctx->d_rates, d_ex, d_mats);
-	ctx->launches++;
+	if ((rc = phbc_score_matrices(ctx, sc, items, bl_host, ex_host))) return rc;
 	Bufs b = phbc_make_bufs(ctx);
 	// any S: operand scratch of a chunk of moves, e and d [chunk][C][P][S], at most a quarter of the free memory and 4 GiB, allocated
 	// before the timed window; PHB_NNI_CHUNK_MOVES caps the chunk (tests run the multi-chunk loop on small trees with it)
 	const size_t per_move = 2 * C * P * S;
 	size_t chunk = 0;
 	double *d_vec = NULL;
-	int rc;
 	if (S != 4) {
 		size_t free_b = 0, total_b = 0;
 		PHBC_CHECK(cudaMemGetInfo(&free_b, &total_b));
@@ -360,7 +294,7 @@ extern "C" int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmove
 		if (chunk < 1) chunk = 1;
 		if (chunk > n) chunk = n;
 		if (chunk > 65535) chunk = 65535;
-		if ((rc = nni_alloc(ctx, &d_vec, chunk * per_move, false))) return rc;
+		if ((rc = phbc_alloc(ctx, &d_vec, chunk * per_move, false))) return rc;
 	}
 	auto launch = [&]() -> int {
 		int rc;
@@ -373,8 +307,8 @@ extern "C" int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmove
 		if (S == 4) {
 			for (int g0 = 0; g0 < ngroups; g0 += 65535) {
 				const int cnt = ngroups - g0 < 65535 ? ngroups - g0 : 65535;
-				k_nni_score<4><<<dim3((unsigned)tiles, (unsigned)cnt), NNI_THREADS, 0, ctx->stream>>>(b, d_groups + g0, d_moves, d_mats, ctx->d_freqs,
-				                                                                                    ctx->d_props, ctx->d_weights, o->scale, d_part);
+				k_nni_score<4><<<dim3((unsigned)tiles, (unsigned)cnt), NNI_THREADS, 0, ctx->stream>>>(b, d_groups + g0, d_moves, sc.mats, ctx->d_freqs,
+				                                                                                    ctx->d_props, ctx->d_weights, o->scale, sc.part);
 				ctx->launches++;
 			}
 		} else {
@@ -383,21 +317,16 @@ extern "C" int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmove
 			for (size_t m0 = 0; m0 < n; m0 += chunk) {
 				const size_t cnt = n - m0 < chunk ? n - m0 : chunk;
 				double *d_e = d_vec, *d_d = d_vec + cnt * C * P * S;
-				k_nni_operands<<<dim3((unsigned)((P + pblk - 1) / pblk), (unsigned)C, (unsigned)cnt), 256, osmem, ctx->stream>>>(b, d_moves + m0, d_mats,
+				k_nni_operands<<<dim3((unsigned)((P + pblk - 1) / pblk), (unsigned)C, (unsigned)cnt), 256, osmem, ctx->stream>>>(b, d_moves + m0, sc.mats,
 				                                                                                                              pblk, d_e, d_d);
-				k_nni_contract<<<dim3((unsigned)tiles, (unsigned)cnt), NNI_THREADS, csmem, ctx->stream>>>(b, d_moves + m0, d_mats, ctx->d_freqs,
+				k_nni_contract<<<dim3((unsigned)tiles, (unsigned)cnt), NNI_THREADS, csmem, ctx->stream>>>(b, d_moves + m0, sc.mats, ctx->d_freqs,
 				                                                                                        ctx->d_props, ctx->d_weights, o->scale, d_e,
-				                                                                                        d_d, d_part);
+				                                                                                        d_d, sc.part);
 				ctx->launches += 2;
 			}
 		}
 		if ((rc = phbc_time_end(ctx))) return rc;
-		k_branch_sum<<<(unsigned)(3 * n), 256, 0, ctx->stream>>>(d_part, (int)tiles, d_out);
-		ctx->launches++;
-		PHBC_CHECK(cudaGetLastError());
-		PHBC_CHECK(cudaMemcpyAsync(out_host, d_out, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-		PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
-		return 0;
+		return phbc_score_finish(ctx, sc, n, tiles, out_host);
 	};
 	rc = launch();
 	if (d_vec) {  // on every path: the stream is drained before the scratch goes

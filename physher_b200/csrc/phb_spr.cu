@@ -15,17 +15,11 @@
 // Both stage the five matrices of one (target, category) -- P_p, P_e, and P_s, P'_s, P"_s at the pendant length -- in shared memory,
 // take targets on grid.y (launches of at most 65,535) and write per-CTA sums [target][3][tile] that k_branch_sum (phb_branch.cu)
 // reduces in a fixed order: bit-identical from run to run, no floating-point atomics.
-#include "phb_ctx.cuh"
+#include "phb_score.cuh"
 
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
-
-// phb_branch.cu
-__global__ void k_branch_matrices(int S, int C, const double *__restrict__ evec, const double *__restrict__ eval, const double *__restrict__ ivec,
-                                  const double *__restrict__ bl, const double *__restrict__ rates, const double *__restrict__ ex_host,
-                                  double *__restrict__ mats);
-__global__ void k_branch_sum(const double *__restrict__ partial, int n, double *__restrict__ out);
 
 #define SPR_THREADS 128
 #define SPR_ANY_THREADS_MAX 512
@@ -44,21 +38,6 @@ __device__ __forceinline__ double spr_log_factor(const Bufs &b, int s, int e, in
 	if (e >= b.T) f += b.sf[(size_t)e * b.P + p];
 	if (s >= b.T) f += b.sf[(size_t)s * b.P + p];
 	return f;
-}
-
-// block reduction of the three per-pattern terms into partial [target][3][tiles]
-template <int WARPS>
-__device__ __forceinline__ void spr_block_sum(double (*red)[WARPS], const double *v, int k, double *partial) {
-	for (int q = 0; q < 3; q++) {
-		const double s = phb_warp_sum(v[q]);
-		if ((threadIdx.x & 31) == 0) red[q][threadIdx.x >> 5] = s;
-	}
-	__syncthreads();
-	if (threadIdx.x < 3) {
-		double s = 0.0;
-		for (int w = 0; w < (int)(blockDim.x >> 5); w++) s += red[threadIdx.x][w];
-		partial[((size_t)k * 3 + threadIdx.x) * gridDim.x + blockIdx.x] = s;
-	}
 }
 
 // grid (pattern tiles, targets k0 .. k0 + gridDim.y - 1)
@@ -137,12 +116,9 @@ __global__ void __launch_bounds__(SPR_THREADS) k_spr_score(Bufs b, int s, int pn
 		const double wt = weights[p];
 		double plk = log(L);
 		if (scale) plk += spr_log_factor(b, s, e, p);
-		const double r1 = dL / L;
-		v[0] = plk * wt;
-		v[1] = r1 * wt;
-		v[2] = (d2L / L - r1 * r1) * wt;
+		score_terms(plk, L, dL, d2L, wt, v);
 	}
-	spr_block_sum<SPR_THREADS / 32>(red, v, k, partial);
+	score_block_sum(red, v, 0, k, partial);
 }
 
 // any S: grid (pattern tiles, targets k0 ..), dynamic shared memory 5 S^2 doubles; row i of every product is formed where it is used
@@ -193,12 +169,9 @@ __global__ void __launch_bounds__(SPR_ANY_THREADS_MAX) k_spr_score_any(Bufs b, i
 		const double wt = weights[p];
 		double plk = log(L);
 		if (scale) plk += spr_log_factor(b, s, e, p);
-		const double r1 = dL / L;
-		v[0] = plk * wt;
-		v[1] = r1 * wt;
-		v[2] = (d2L / L - r1 * r1) * wt;
+		score_terms(plk, L, dL, d2L, wt, v);
 	}
-	spr_block_sum<SPR_ANY_THREADS_MAX / 32>(red, v, k, partial);
+	score_block_sum(red, v, 0, k, partial);
 }
 
 // threads per CTA of the score kernel: any S takes more where its five matrices leave room for one CTA per SM only
@@ -207,35 +180,26 @@ static int spr_threads(const phbc_ctx *ctx) {
 	return ctx->S == 4 ? SPR_THREADS : (smem > 48 * 1024 ? SPR_ANY_THREADS_MAX : SPR_THREADS);
 }
 
-// the scratch of one call, sized and allocated before the pruned pass overwrites anything, so that a state count the kernels cannot
-// stage (-1) or a device too small for the matrix table (-3) is reported with the object unchanged:
-//   bl [items] | results [n][3] | matrices [items][C][3][S*S] | partial [n][3][tiles] | host exponentials [items][C][S] | targets
-extern "C" int phbc_spr_reserve(phbc_ctx *ctx, int ntargets) {
-	PHBC_CHECK(cudaSetDevice(ctx->device));
-	const size_t S = ctx->S, C = ctx->C, P = ctx->P, N = ctx->N;
+// the scratch of one call (the layout of phb_score.cuh, descriptors = the targets), sized and allocated before the pruned pass
+// overwrites anything, so that a state count the kernels cannot stage (-1) or a device too small for the matrix table (-3) is reported
+// with the object unchanged
+static int spr_scratch(phbc_ctx *ctx, int ntargets, ScoreScratch *sc) {
+	const size_t S = ctx->S;
 	const size_t smem = 5 * S * S * sizeof(double);
 	if (S != 4 && smem > ctx->smem_optin) {
 		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "SPR scores: %zu states need %zu bytes of shared memory for five matrices (at most %zu)", S, smem,
 		         ctx->smem_optin);
 		return -1;
 	}
-	const size_t n = ntargets > 0 ? (size_t)ntargets : 1, items = N + n;
-	const size_t tiles = (P + spr_threads(ctx) - 1) / spr_threads(ctx);
-	const size_t need = (items * (1 + C * 3 * S * S + C * S) + n * (3 + 3 * tiles) + (n + 1) / 2) * sizeof(double);
-	if (need <= ctx->branch_bytes) return 0;
-	PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
-	if (ctx->d_branch) cudaFree(ctx->d_branch);
-	ctx->d_branch = NULL;
-	ctx->branch_bytes = 0;
-	const cudaError_t e = cudaMalloc((void **)&ctx->d_branch, need);
-	if (e == cudaErrorMemoryAllocation) {
-		(void)cudaGetLastError();
-		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "out of device memory: %.1f GB for the SPR matrix table and sums", need / 1e9);
-		return -3;
-	}
-	PHBC_CHECK(e);
-	ctx->branch_bytes = need;
-	return 0;
+	const size_t n = ntargets > 0 ? (size_t)ntargets : 1;
+	const size_t tiles = ((size_t)ctx->P + spr_threads(ctx) - 1) / spr_threads(ctx);
+	return phbc_score_scratch(ctx, ctx->N + n, n, tiles, n * sizeof(int), sc);
+}
+
+extern "C" int phbc_spr_reserve(phbc_ctx *ctx, int ntargets) {
+	PHBC_CHECK(cudaSetDevice(ctx->device));
+	ScoreScratch sc;
+	return spr_scratch(ctx, ntargets, &sc);
 }
 
 // out_host [ntargets][3]; bl_host [N + ntargets]: every node's length (root entry unused), then each target's pendant length; ex_host
@@ -243,7 +207,7 @@ extern "C" int phbc_spr_reserve(phbc_ctx *ctx, int ntargets) {
 extern "C" int phbc_spr_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int s, int p, int ntargets, const int *targets_host,
                                const double *bl_host, const double *ex_host, double *out_host) {
 	PHBC_CHECK(cudaSetDevice(ctx->device));
-	const size_t S = ctx->S, C = ctx->C, P = ctx->P, N = ctx->N;
+	const size_t S = ctx->S, P = ctx->P, N = ctx->N;
 	if (ntargets < 1) {
 		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "%d targets: at least one is needed", ntargets);
 		return -1;
@@ -252,45 +216,30 @@ extern "C" int phbc_spr_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int s, in
 		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "SPR scores need the eigen system (explicit matrices cannot be re-evaluated at a new length)");
 		return -4;
 	}
-	if (!ctx->d_upper || !ctx->d_lower || (o->scale && !ctx->d_sf) || (ctx->tip_kind != PHBC_TIP_STATES && !ctx->d_tip_partials)) {
-		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "upper / lower partials are not resident");
-		return -4;
-	}
 	int rc;
-	if ((rc = phbc_spr_reserve(ctx, ntargets))) return rc;  // nothing to do when the caller reserved first
+	if ((rc = phbc_score_resident(ctx, o))) return rc;
+	ScoreScratch sc;
+	if ((rc = spr_scratch(ctx, ntargets, &sc))) return rc;  // nothing to allocate when the caller reserved first
 	const size_t smem = 5 * S * S * sizeof(double);
 	const int threads = spr_threads(ctx);
-	const size_t n = (size_t)ntargets, items = N + n;
+	const size_t n = (size_t)ntargets;
 	const size_t tiles = (P + threads - 1) / threads;
-	double *d_bl = ctx->d_branch, *d_out = d_bl + items, *d_mats = d_out + 3 * n, *d_part = d_mats + items * C * 3 * S * S;
-	double *d_exbuf = d_part + n * 3 * tiles;
-	double *d_ex = ex_host ? d_exbuf : NULL;
-	int *d_targets = reinterpret_cast<int *>(d_exbuf + items * C * S);
-	PHBC_CHECK(cudaMemcpyAsync(d_bl, bl_host, items * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-	PHBC_CHECK(cudaMemcpyAsync(d_targets, targets_host, n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-	if (ex_host) PHBC_CHECK(cudaMemcpyAsync(d_ex, ex_host, items * C * S * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-	const int mthreads = S * S >= 256 ? 256 : (S * S >= 64 ? 64 : 32);
-	k_branch_matrices<<<dim3((unsigned)items, (unsigned)C), mthreads, 3 * S * sizeof(double), ctx->stream>>>((int)S, (int)C, ctx->d_evec, ctx->d_eval,
-	                                                                                                    ctx->d_ivec, d_bl, ctx->d_rates, d_ex, d_mats);
-	ctx->launches++;
+	const int *d_targets = static_cast<int *>(sc.desc);
+	PHBC_CHECK(cudaMemcpyAsync(sc.desc, targets_host, n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+	if ((rc = phbc_score_matrices(ctx, sc, N + n, bl_host, ex_host))) return rc;
 	if (S != 4 && smem > 48 * 1024) PHBC_CHECK(cudaFuncSetAttribute(k_spr_score_any, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 	Bufs b = phbc_make_bufs(ctx);
 	if ((rc = phbc_time_begin(ctx))) return rc;
 	for (size_t k0 = 0; k0 < n; k0 += 65535) {
 		const unsigned cnt = (unsigned)(n - k0 < 65535 ? n - k0 : 65535);
 		if (S == 4)
-			k_spr_score<4><<<dim3((unsigned)tiles, cnt), threads, 0, ctx->stream>>>(b, s, p, d_targets, (int)k0, d_mats, ctx->d_freqs, ctx->d_props,
-			                                                                     ctx->d_weights, o->scale, d_part);
+			k_spr_score<4><<<dim3((unsigned)tiles, cnt), threads, 0, ctx->stream>>>(b, s, p, d_targets, (int)k0, sc.mats, ctx->d_freqs, ctx->d_props,
+			                                                                     ctx->d_weights, o->scale, sc.part);
 		else
-			k_spr_score_any<<<dim3((unsigned)tiles, cnt), threads, smem, ctx->stream>>>(b, s, p, d_targets, (int)k0, d_mats, ctx->d_freqs, ctx->d_props,
-			                                                                          ctx->d_weights, o->scale, d_part);
+			k_spr_score_any<<<dim3((unsigned)tiles, cnt), threads, smem, ctx->stream>>>(b, s, p, d_targets, (int)k0, sc.mats, ctx->d_freqs, ctx->d_props,
+			                                                                          ctx->d_weights, o->scale, sc.part);
 		ctx->launches++;
 	}
 	if ((rc = phbc_time_end(ctx))) return rc;
-	k_branch_sum<<<(unsigned)(3 * n), 256, 0, ctx->stream>>>(d_part, (int)tiles, d_out);
-	ctx->launches++;
-	PHBC_CHECK(cudaGetLastError());
-	PHBC_CHECK(cudaMemcpyAsync(out_host, d_out, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-	PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
-	return 0;
+	return phbc_score_finish(ctx, sc, n, tiles, out_host);
 }

@@ -1052,23 +1052,24 @@ static void fill_opts(const phb_tlk *t, phbc_eval_opts *o, int want_gradient, in
  */
 static int wants_host_exp(const phb_tlk *t) { return t->host_exp && t->have_eigen && !t->have_matrices && t->h_eval && t->h_rates; }
 
-/* exp(eval_k * bl[b][n] * rate_c) for nbatch branch-length vectors, [nbatch][N][C][S], to the device */
+/* ex [n][C][S] = exp(eval_q * (bl[k] * rate_c)) for n lengths */
+static void host_exponentials(const phb_tlk *t, size_t n, const double *bl, double *ex) {
+	const int C = t->C, S = t->S;
+	for (size_t k = 0; k < n; k++)
+		for (int c = 0; c < C; c++)
+			for (int q = 0; q < S; q++) ex[(k * C + c) * S + q] = exp(t->h_eval[q] * (bl[k] * t->h_rates[c]));
+}
+
+/* the exponentials of nbatch branch-length vectors, [nbatch][N][C][S], to the device */
 static int upload_host_exponentials(phb_tlk *t, const double *bl, int nbatch) {
-	const int N = t->N, C = t->C, S = t->S;
-	const size_t need = (size_t)nbatch * N * C * S;
+	const size_t need = (size_t)nbatch * t->N * t->C * t->S;
 	if (need > t->ex_cap) {
 		double *nb = (double *)realloc(t->ex_buf, sizeof(double) * need);
 		if (!nb) return -3;
 		t->ex_buf = nb;
 		t->ex_cap = need;
 	}
-	for (int b = 0; b < nbatch; b++)
-		for (int n = 0; n < N; n++)
-			for (int c = 0; c < C; c++) {
-				const double tt = bl[(size_t)b * N + n] * t->h_rates[c];
-				double *dst = t->ex_buf + (((size_t)b * N + n) * C + c) * S;
-				for (int k = 0; k < S; k++) dst[k] = exp(t->h_eval[k] * tt);
-			}
+	host_exponentials(t, (size_t)nbatch * t->N, bl, t->ex_buf);
 	return phbc_upload_exponentials(t->ctx, t->ex_buf, nbatch);
 }
 
@@ -1123,6 +1124,14 @@ static void fill_opts_resident(const phb_tlk *t, phbc_eval_opts *o, int want_gra
 	fill_opts(t, o, want_gradient, 0);
 	o->kernels = ((t->S == 20 || (t->S >= 60 && t->S <= 63)) && t->kernels != PHB_KERNELS_GENERIC) ? PHB_KERNELS_AUTO : PHB_KERNELS_GENERIC;
 	o->materialize_uppers = 1;
+}
+
+/* PHB_OPT_INCREMENTAL on, for the calls that need resident partials */
+static void resident_on(phb_tlk *t) {
+	if (!t->incremental) {
+		t->incremental = 1;
+		t->resident = 0;
+	}
 }
 
 static void mark_clean(phb_tlk *t) {
@@ -1269,10 +1278,7 @@ static int resident_uppers(phb_tlk *t, int node, int irf) {
 
 /* SingleTreeLikelihood_update_uppers (treelikelihood.c:1530-1538): lnL, then every upper partial (root frequencies not folded in) */
 static int phb_tlk_update_uppers_impl(phb_tlk *t) {
-	if (!t->incremental) {
-		t->incremental = 1;
-		t->resident = 0;
-	}
+	resident_on(t);
 	double lnl;
 	int rc = resident_calculate(t, &lnl);
 	if (rc) return rc;
@@ -1288,9 +1294,7 @@ static int branch_items(phb_tlk *t, int nitems, const int *nodes, const double *
 	if (wants_host_exp(t)) { /* the item lengths get the host's exponentials like every other matrix of this model */
 		ex = (double *)malloc(sizeof(double) * (size_t)nitems * t->C * t->S);
 		if (!ex) return fail(PHB_ENOMEM, "out of memory");
-		for (int k = 0; k < nitems; k++)
-			for (int c = 0; c < t->C; c++)
-				for (int q = 0; q < t->S; q++) ex[((size_t)k * t->C + c) * t->S + q] = exp(t->h_eval[q] * (bl[k] * t->h_rates[c]));
+		host_exponentials(t, (size_t)nitems, bl, ex);
 	}
 	const int rc = phbc_branch_lnl(t->ctx, &o, nitems, nodes, bl, ex, out);
 	free(ex);
@@ -1304,10 +1308,7 @@ static int phb_tlk_calculate_branch_impl(phb_tlk *t, int node, int nbl, const do
 	if (t->have_matrices) return fail(PHB_ESTATE, "calculate_branch needs the eigen system: explicit matrices cannot be re-evaluated at a new length");
 	for (int k = 0; k < nbl; k++)
 		if (bl[k] < 0) return fail(PHB_EINVAL, "calculate_partials: node %d branch length = %E", node, bl[k]);
-	if (!t->incremental) {
-		t->incremental = 1;
-		t->resident = 0;
-	}
+	resident_on(t);
 	double cur;
 	int rc = resident_calculate(t, &cur);
 	if (rc) return rc;
@@ -1382,10 +1383,7 @@ static int phb_tlk_branch_hessian_diagonal_impl(phb_tlk *t, double *lnl, double 
 		}
 	}
 	if (!done) {
-		if (!t->incremental) {
-			t->incremental = 1;
-			t->resident = 0;
-		}
+		resident_on(t);
 		if ((rc = resident_calculate(t, &cur))) return rc; /* retries with rescaling on itself */
 		if (!isnan(cur) && !isinf(cur)) {
 			if ((rc = resident_uppers(t, -1, 0))) return rc;
@@ -1465,34 +1463,48 @@ static int phb_tlk_nni_moves_impl(phb_tlk *t, int *moves) {
 	return n;
 }
 
+/* the matrix table of a score pass: every node at its current length (the root's entry unused, 0), then one length per candidate --
+ * given[k], or the current length of node dflt[k * stride] */
+static void table_lengths(const phb_tlk *t, int ncand, const double *given, const int *dflt, int dflt_stride, double *bl) {
+	for (int n = 0; n < t->N; n++) bl[n] = n == t->root ? 0.0 : t->bl[n];
+	for (int k = 0; k < ncand; k++) bl[t->N + k] = given ? given[k] : t->bl[dflt[(size_t)k * dflt_stride]];
+}
+
 /* launch order of the 4-state kernel's work items: by parent of v, so that the groups of two siblings are neighbours (U_p from L2) */
-static _Thread_local const phb_tlk *g_nni_tlk;
-static _Thread_local const int *g_nni_moves;
+typedef struct NniKey {
+	int pv, v, x, k; /* parent of v, v, x, move index */
+} NniKey;
 static int nni_order(const void *pa, const void *pb) {
-	const int a = *(const int *)pa, b = *(const int *)pb;
-	const phb_tlk *t = g_nni_tlk;
-	const int va = t->parent[g_nni_moves[2 * a + 1]], vb = t->parent[g_nni_moves[2 * b + 1]];
-	const int ka[4] = {t->parent[va], va, g_nni_moves[2 * a], a}, kb[4] = {t->parent[vb], vb, g_nni_moves[2 * b], b};
+	const NniKey *a = (const NniKey *)pa, *b = (const NniKey *)pb;
+	const int ka[4] = {a->pv, a->v, a->x, a->k}, kb[4] = {b->pv, b->v, b->x, b->k};
 	for (int i = 0; i < 4; i++)
 		if (ka[i] != kb[i]) return ka[i] < kb[i] ? -1 : 1;
 	return 0;
 }
 
-/* one pass of the scores on resident partials: the move descriptors, the (v, x) pairs, the matrix table and its lengths */
-static int nni_pass(phb_tlk *t, int nmoves, const int *moves, const double *t_central, double *out) {
-	const int N = t->N, C = t->C, S = t->S;
+/* one pass of the scores on resident partials: every upper partial, the move descriptors, the (v, x) pairs, the matrix table and its
+ * lengths */
+typedef struct NniArgs {
+	int nmoves;
+	const int *moves;
+	const double *t_central;
+} NniArgs;
+static int nni_pass(phb_tlk *t, const void *arg, double *out) {
+	const NniArgs *a = (const NniArgs *)arg;
+	const int N = t->N, C = t->C, S = t->S, nmoves = a->nmoves;
+	const int *moves = a->moves;
+	int rc = resident_uppers(t, -1, 0);
+	if (rc) return rc;
 	const size_t items = (size_t)N + nmoves;
 	phbc_nni_move *desc = (phbc_nni_move *)malloc(sizeof(phbc_nni_move) * (size_t)nmoves);
-	int *order = (int *)malloc(sizeof(int) * (size_t)nmoves);
+	NniKey *order = (NniKey *)malloc(sizeof(NniKey) * (size_t)nmoves);
 	int *groups = (int *)malloc(sizeof(int) * 2 * (size_t)nmoves);
 	double *bl = (double *)malloc(sizeof(double) * items);
 	double *ex = wants_host_exp(t) ? (double *)malloc(sizeof(double) * items * C * S) : NULL;
-	int rc = PHB_OK;
 	if (!desc || !order || !groups || !bl || (wants_host_exp(t) && !ex)) {
 		rc = fail(PHB_ENOMEM, "out of memory");
 		goto done;
 	}
-	for (int n = 0; n < N; n++) bl[n] = n == t->root ? 0.0 : t->bl[n];
 	for (int k = 0; k < nmoves; k++) {
 		const int x = moves[2 * k], y = moves[2 * k + 1], v = t->parent[y];
 		phbc_nni_move *m = &desc[k];
@@ -1505,22 +1517,18 @@ static int nni_pass(phb_tlk *t, int nmoves, const int *moves, const double *t_ce
 			m->a = m->a_mat = sibling_of(t, x);
 		}
 		m->cmat = N + k, m->out = k;
-		bl[N + k] = t_central ? t_central[k] : t->bl[v];
-		order[k] = k;
+		order[k] = (NniKey){t->parent[v], v, x, k};
 	}
-	g_nni_tlk = t, g_nni_moves = moves;
-	qsort(order, (size_t)nmoves, sizeof(int), nni_order);
+	table_lengths(t, nmoves, a->t_central, &order[0].v, sizeof(NniKey) / sizeof(int), bl); /* the central branch is v's */
+	qsort(order, (size_t)nmoves, sizeof(NniKey), nni_order);
 	int ngroups = 0;
 	for (int i = 0; i < nmoves; ngroups++) {
-		const int a = order[i], b = i + 1 < nmoves ? order[i + 1] : -1;
-		const int pair = b >= 0 && moves[2 * a] == moves[2 * b] && t->parent[moves[2 * a + 1]] == t->parent[moves[2 * b + 1]];
-		groups[2 * ngroups] = a, groups[2 * ngroups + 1] = pair ? b : -1;
+		const NniKey *ka = &order[i], *kb = i + 1 < nmoves ? &order[i + 1] : NULL;
+		const int pair = kb && ka->x == kb->x && ka->v == kb->v;
+		groups[2 * ngroups] = ka->k, groups[2 * ngroups + 1] = pair ? kb->k : -1;
 		i += pair ? 2 : 1;
 	}
-	if (ex)
-		for (size_t k = 0; k < items; k++)
-			for (int c = 0; c < C; c++)
-				for (int q = 0; q < S; q++) ex[(k * C + c) * S + q] = exp(t->h_eval[q] * (bl[k] * t->h_rates[c]));
+	if (ex) host_exponentials(t, items, bl, ex);
 	phbc_eval_opts o;
 	fill_opts_resident(t, &o, 1);
 	if ((rc = phbc_nni_scores(t->ctx, &o, nmoves, desc, ngroups, groups, bl, ex, out))) rc = dev_fail(rc);
@@ -1530,11 +1538,35 @@ done:
 }
 
 /*
- * lnL and central-branch derivatives of every listed NNI neighbour from resident partials: lowers and uppers made resident
- * (PHB_OPT_INCREMENTAL on, as phb_tlk_branch_hessian_diagonal's resident route), then one pass over them (phb_nni.cu).  NaN / inf as
- * treelikelihood.c:1496-1519: an infinite lnL of the current tree, or a move whose unscaled site likelihood underflows, switches
- * rescaling on and recomputes once.
+ * The score calls on resident partials (NNI, SPR): reserve the resident buffers (-3 with the object unchanged), make the lowers resident
+ * (PHB_OPT_INCREMENTAL on), then one pass writing out [n][3].  NaN / inf as treelikelihood.c:1496-1519: an infinite lnL of the current
+ * tree, or an output that is not finite while rescaling is off, switches rescaling on and scores once more; a current lnL still NaN or
+ * infinite NaN-fills out.
  */
+static int resident_scores(phb_tlk *t, int n, double *lnl, double *out, int (*pass)(phb_tlk *, const void *, double *), const void *arg) {
+	phbc_eval_opts o;
+	fill_opts(t, &o, 1, 0);
+	int rc = phbc_generic_buffers(t->ctx, &o);
+	if (rc) return dev_fail(rc);
+	resident_on(t);
+	double cur = 0.0;
+	for (int attempt = 0; attempt < 2; attempt++) {
+		if ((rc = resident_calculate(t, &cur))) return rc; /* retries with rescaling on itself */
+		if (isnan(cur) || isinf(cur)) break;
+		if ((rc = pass(t, arg, out))) return rc;
+		int finite = 1;
+		for (int k = 0; k < 3 * n; k++) finite &= isfinite(out[k]) != 0;
+		if (finite || t->scale) break;
+		t->scale = 1; /* something underflowed unscaled: rescale everything and score again */
+		t->all_dirty = 1;
+	}
+	if (lnl) *lnl = cur;
+	if (isnan(cur) || isinf(cur))
+		for (int k = 0; k < 3 * n; k++) out[k] = NAN;
+	return PHB_OK;
+}
+
+/* lnL and central-branch derivatives of every listed NNI neighbour from resident partials (phb_nni.cu) */
 static int phb_tlk_nni_scores_impl(phb_tlk *t, int nmoves, const int *moves, const double *t_central, double *lnl, double *out) {
 	if (!moves || !out) return fail(PHB_EINVAL, "nni_scores: moves and out are required");
 	if (nmoves < 1) return fail(PHB_EINVAL, "nni_scores: %d moves (at least one is needed)", nmoves);
@@ -1548,27 +1580,8 @@ static int phb_tlk_nni_scores_impl(phb_tlk *t, int nmoves, const int *moves, con
 	if (t->have_matrices) return fail(PHB_ESTATE, "nni_scores needs the eigen system: explicit matrices cannot be re-evaluated at a new length");
 	int rc = check_ready(t);
 	if (rc) return rc;
-	if ((rc = phbc_nni_reserve(t->ctx, t->scale))) return dev_fail(rc);
-	if (!t->incremental) {
-		t->incremental = 1;
-		t->resident = 0;
-	}
-	double cur = 0.0;
-	for (int attempt = 0; attempt < 2; attempt++) {
-		if ((rc = resident_calculate(t, &cur))) return rc; /* retries with rescaling on itself */
-		if (isnan(cur) || isinf(cur)) break;
-		if ((rc = resident_uppers(t, -1, 0))) return rc;
-		if ((rc = nni_pass(t, nmoves, moves, t_central, out))) return rc;
-		int finite = 1;
-		for (int k = 0; k < 3 * nmoves; k++) finite &= isfinite(out[k]) != 0;
-		if (finite || t->scale) break;
-		t->scale = 1; /* a move's site likelihood underflowed unscaled: rescale everything and score again */
-		t->all_dirty = 1;
-	}
-	if (lnl) *lnl = cur;
-	if (isnan(cur) || isinf(cur))
-		for (int k = 0; k < 3 * nmoves; k++) out[k] = NAN;
-	return PHB_OK;
+	const NniArgs a = {nmoves, moves, t_central};
+	return resident_scores(t, nmoves, lnl, out, nni_pass, &a);
 }
 
 /*
@@ -1628,7 +1641,14 @@ static int phb_tlk_spr_targets_impl(phb_tlk *t, int s, int *targets) {
  * ancestors below the root (lower_stale: the next evaluation recomputes them, and the cached lnL stays that of the current tree) and
  * upper_ok of every node it wrote; the uppers of p and of the subtree of s are untouched.
  */
-static int spr_pass(phb_tlk *t, int s, int ntargets, const int *targets, const double *t_pendant, double *out) {
+typedef struct SprArgs {
+	int s, ntargets;
+	const int *targets;
+	const double *t_pendant;
+} SprArgs;
+static int spr_pass(phb_tlk *t, const void *arg, double *out) {
+	const SprArgs *a = (const SprArgs *)arg;
+	const int s = a->s, ntargets = a->ntargets;
 	const int N = t->N, C = t->C, S = t->S, root = t->root;
 	const int p = t->parent[s], g = t->parent[p], b = sibling_of(t, s);
 	const size_t items = (size_t)N + ntargets;
@@ -1695,25 +1715,17 @@ static int spr_pass(phb_tlk *t, int s, int ntargets, const int *targets, const d
 		rc = dev_fail(rc);
 		goto done;
 	}
-	/* the matrix table: every node at its current length, then each target's pendant length */
-	for (int n = 0; n < N; n++) bl[n] = n == root ? 0.0 : t->bl[n];
-	for (int k = 0; k < ntargets; k++) bl[N + k] = t_pendant ? t_pendant[k] : t->bl[s];
-	if (ex)
-		for (size_t k = 0; k < items; k++)
-			for (int c = 0; c < C; c++)
-				for (int q = 0; q < S; q++) ex[(k * C + c) * S + q] = exp(t->h_eval[q] * (bl[k] * t->h_rates[c]));
+	table_lengths(t, ntargets, a->t_pendant, &s, 0, bl); /* the pendant branch is s's */
+	if (ex) host_exponentials(t, items, bl, ex);
 	fill_opts_resident(t, &o, 1);
-	if ((rc = phbc_spr_scores(t->ctx, &o, s, p, ntargets, targets, bl, ex, out))) rc = dev_fail(rc);
+	if ((rc = phbc_spr_scores(t->ctx, &o, s, p, ntargets, a->targets, bl, ex, out))) rc = dev_fail(rc);
 done:
 	free(queue), free(depth), free(bl), free(ex);
 	return rc;
 }
 
-/*
- * lnL and pendant-branch derivatives of the subtree of s regrafted on each listed target, from one pass over the pruned tree: lowers
- * made resident (PHB_OPT_INCREMENTAL on), then spr_pass.  NaN / inf as phb_tlk_nni_scores: an infinite lnL of the current tree, or a
- * target whose unscaled site likelihood underflows, switches rescaling on and scores once more.
- */
+/* lnL and pendant-branch derivatives of the subtree of s regrafted on each listed target, from one pass over the pruned tree (phb_spr.cu);
+ * the matrix table is reserved with the resident buffers, before the pruned pass changes anything */
 static int phb_tlk_spr_scores_impl(phb_tlk *t, int s, int ntargets, const int *targets, const double *t_pendant, double *lnl, double *out) {
 	int rc = spr_check_prune(t, "spr_scores", s);
 	if (rc) return rc;
@@ -1738,26 +1750,9 @@ static int phb_tlk_spr_scores_impl(phb_tlk *t, int s, int ntargets, const int *t
 	if (rc) return rc;
 	if (t->have_matrices) return fail(PHB_ESTATE, "spr_scores needs the eigen system: explicit matrices cannot be re-evaluated at a new length");
 	if ((rc = check_ready(t))) return rc;
-	if ((rc = phbc_nni_reserve(t->ctx, t->scale)) || (rc = phbc_spr_reserve(t->ctx, ntargets))) return dev_fail(rc);
-	if (!t->incremental) {
-		t->incremental = 1;
-		t->resident = 0;
-	}
-	double cur = 0.0;
-	for (int attempt = 0; attempt < 2; attempt++) {
-		if ((rc = resident_calculate(t, &cur))) return rc; /* retries with rescaling on itself */
-		if (isnan(cur) || isinf(cur)) break;
-		if ((rc = spr_pass(t, s, ntargets, targets, t_pendant, out))) return rc;
-		int finite = 1;
-		for (int k = 0; k < 3 * ntargets; k++) finite &= isfinite(out[k]) != 0;
-		if (finite || t->scale) break;
-		t->scale = 1; /* a target's site likelihood underflowed unscaled: rescale everything and score again */
-		t->all_dirty = 1;
-	}
-	if (lnl) *lnl = cur;
-	if (isnan(cur) || isinf(cur))
-		for (int k = 0; k < 3 * ntargets; k++) out[k] = NAN;
-	return PHB_OK;
+	if ((rc = phbc_spr_reserve(t->ctx, ntargets))) return dev_fail(rc);
+	const SprArgs a = {s, ntargets, targets, t_pendant};
+	return resident_scores(t, ntargets, lnl, out, spr_pass, &a);
 }
 
 /*
@@ -1775,10 +1770,7 @@ static int phb_tlk_update_partials_impl(phb_tlk *t, int out, int p1, int m1, int
 	if (out < T || out >= 2 * N || p1 < 0 || p1 >= 2 * N || m1 < 0 || m1 >= N || p2 >= 2 * N || (p2 >= 0 && (m2 < 0 || m2 >= N)))
 		return fail(PHB_EINVAL, "update_partials(%d, %d, %d, %d, %d): index out of range", out, p1, m1, p2, m2);
 	if (t->have_matrices) return fail(PHB_ESTATE, "update_partials needs the eigen system: explicit matrices belong to one set of branch lengths");
-	if (!t->incremental) {
-		t->incremental = 1;
-		t->resident = 0;
-	}
+	resident_on(t);
 	double cur;
 	int rc = resident_calculate(t, &cur);
 	if (rc) return rc;

@@ -184,6 +184,30 @@ def test_branch_under_rescaling(S, C):
 
 
 @gpu
+def test_branch_candidates_past_one_launch():
+    """70,000 candidate lengths in one call: the values of the same lengths scored in slices of at most 65,535, and one more score
+    launch than a call whose items fit one grid.y"""
+    pb = synthetic_problem(4, 8, 64, 2, 55)
+    tlk = phb.SingleTreeLikelihood.from_problem(pb)
+    n = next(i for i in range(pb.nnodes) if i != pb.root and pb.left[i] >= 0)
+    cands = pb.bl[n] * np.linspace(0.2, 3.0, 70000)
+    tlk.calculate_branch(n, cands[:2])
+
+    def run(c):
+        before = tlk.launch_count()
+        out = np.stack(tlk.calculate_branch(n, c), 1)
+        return tlk.launch_count() - before, out
+
+    one, head = run(cands[:65535])
+    two, out = run(cands)
+    assert two == one + 1
+    _, tail = run(cands[65535:])
+    assert np.array_equal(out, np.concatenate([head, tail]))
+    assert deriv_err(out[::997], O.branch_derivatives(pb, n, cands[::997])) < RTOL
+    tlk.close()
+
+
+@gpu
 def test_branch_errors():
     pb = synthetic_problem(4, 6, 50, 1, 3)
     tlk = phb.SingleTreeLikelihood.from_problem(pb)
