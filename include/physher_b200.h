@@ -69,6 +69,16 @@ extern "C" {
                                             cherries by pairs of tip states always / never (default: from 4 (S + 1)^2 patterns on), 22 = rescaled
                                             evaluations on the node-at-a-time tensor-core kernels instead of the message form */
 
+/* State-count limits.  phb_tlk_create accepts 2 <= nstate <= 255, but the node-at-a-time and score kernels stage whole S x S matrices of
+ * doubles in the shared memory of one CTA, so each call has a largest state count, set by the device's opt-in shared memory per block
+ * (cudaDevAttrMaxSharedMemoryPerBlockOptin; 227 KB on B200 gives the numbers in brackets):
+ *   evaluation, gradient, matrix gradient on the node-at-a-time kernels   2 S^2 x 8 bytes   [S <= 120]
+ *   phb_tlk_calculate_branch, phb_tlk_branch_hessian_diagonal (resident)  3 S^2 x 8 bytes   [S <= 98]
+ *   phb_tlk_nni_scores (S != 4)                                           4 S^2 x 8 bytes   [S <= 85]
+ *   phb_tlk_spr_scores (S != 4)                                           5 S^2 x 8 bytes   [S <= 76]
+ * Past its limit a call returns PHB_EINVAL, with a message naming the state count and the bytes it needs, before it launches its kernels;
+ * the object stays usable for the calls whose limit it is within. */
+
 #define PHB_KERNELS_AUTO 0    /* by state count, like the function-pointer dispatch at treelikelihood.c:1067-1165 */
 #define PHB_KERNELS_GENERIC 1 /* node-at-a-time kernels, any state count, materialised upper partials */
 #define PHB_KERNELS_FUSED 2   /* whole-tree walk kernels (4 states; 20 states on the tensor cores) / level-batched tensor-core kernels (60 ... 63 states) */

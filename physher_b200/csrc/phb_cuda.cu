@@ -596,8 +596,8 @@ __global__ void k_sum_blocks(const double *__restrict__ in, int n, double *__res
 #define GEN_PGRAD 256
 
 // calculate_branch_partials + gradient_cat_branch_lengths (treelikelihoodX.c:878-1001, treelikelihood.c:2793-2941,
-// 2715-2789); grid (ceil(P/256), N-1 non-root nodes), one thread per pattern                           -- K9, K10
-__global__ void k_generic_branch_gradient(Bufs b, int root, const double *__restrict__ Pm, const double *__restrict__ dPm,
+// 2715-2789); grid (ceil(P/256), non-root nodes y0 .. y0 + gridDim.y - 1), one thread per pattern       -- K9, K10
+__global__ void k_generic_branch_gradient(Bufs b, int root, int y0, const double *__restrict__ Pm, const double *__restrict__ dPm,
                                           const double *__restrict__ freqs, const double *__restrict__ props,
                                           const double *__restrict__ weights, const double *__restrict__ pattern_lnl,
                                           int scale, int compat, int include_root_freqs, double *__restrict__ partial /* [N][C][tiles] */) {
@@ -605,7 +605,7 @@ __global__ void k_generic_branch_gradient(Bufs b, int root, const double *__rest
 	__shared__ double red[GEN_PGRAD / 32];
 	const int S = b.S, SS = S * S;
 	double *dM = sm, *M = sm + SS;
-	int node = blockIdx.y;
+	int node = y0 + blockIdx.y;
 	if (node >= root) node++;  // skip the root
 	const int p = blockIdx.x * blockDim.x + threadIdx.x;
 	const bool live = p < b.P;
@@ -714,6 +714,14 @@ static int phbc_launch_transition_matrices(phbc_ctx *ctx, int batch_index) {
 	return 0;
 }
 
+extern "C" int phbc_smem_check(const phbc_ctx *ctx, const char *what, int nmat) {
+	const size_t need = (size_t)nmat * ctx->S * ctx->S * sizeof(double);
+	if (need <= ctx->smem_optin) return 0;
+	snprintf(phbc_errbuf, sizeof(phbc_errbuf), "%s: %d states need %zu bytes of shared memory for %d matrices (at most %zu)", what, ctx->S, need, nmat,
+	         ctx->smem_optin);
+	return -1;
+}
+
 int phbc_alloc(phbc_ctx *ctx, double **p, size_t count, bool zero) {
 	const cudaError_t e = cudaMalloc((void **)p, count * sizeof(double));
 	if (e == cudaErrorMemoryAllocation) {
@@ -795,23 +803,29 @@ int phbc_gradient_from_partials(phbc_ctx *ctx, int tiles, double *result) {
 	return 0;
 }
 
-int phbc_generic_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, double *result) {
-	Bufs b = phbc_make_bufs(ctx);
-	const size_t S = ctx->S, C = ctx->C, P = ctx->P, N = ctx->N;
+// k_generic_branch_gradient with dPm in the place of dP/dt over every non-root node into the [N][C][tiles] scratch: the nodes on grid.y,
+// in launches of at most 65,535
+static int gen_branch_gradient(phbc_ctx *ctx, const double *dPm, int scale, int compat, int include_root_freqs) {
+	const size_t S = ctx->S, gtiles = ((size_t)ctx->P + GEN_PGRAD - 1) / GEN_PGRAD;
 	const size_t smem = 2 * S * S * sizeof(double);
 	if (smem > 48 * 1024) PHBC_CHECK(cudaFuncSetAttribute(k_generic_branch_gradient, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+	Bufs b = phbc_make_bufs(ctx);
+	for (int y0 = 0; y0 < ctx->N - 1; y0 += 65535) {
+		const int cnt = ctx->N - 1 - y0 < 65535 ? ctx->N - 1 - y0 : 65535;
+		k_generic_branch_gradient<<<dim3((unsigned)gtiles, (unsigned)cnt), GEN_PGRAD, smem, ctx->stream>>>(
+		    b, ctx->root, y0, ctx->d_P, dPm, ctx->d_freqs, ctx->d_props, ctx->d_weights, ctx->d_pattern_lnl, scale, compat, include_root_freqs,
+		    ctx->d_scratch);
+		ctx->launches++;
+	}
+	return 0;
+}
+
+int phbc_generic_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, double *result) {
+	const size_t C = ctx->C, P = ctx->P, N = ctx->N;
 	const size_t gtiles = (P + GEN_PGRAD - 1) / GEN_PGRAD;
 	int rc;
 	if ((rc = phbc_ensure_scratch(ctx, N * C * gtiles * sizeof(double)))) return rc;
-	if (N - 1 > 65535) {
-		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "generic gradient kernel supports at most 65535 branches");
-		return -1;
-	}
-	// blockIdx.y enumerates the non-root nodes
-	k_generic_branch_gradient<<<dim3((unsigned)gtiles, (unsigned)(N - 1)), GEN_PGRAD, smem, ctx->stream>>>(
-	    b, ctx->root, ctx->d_P, ctx->d_dP, ctx->d_freqs, ctx->d_props, ctx->d_weights, ctx->d_pattern_lnl, o->scale,
-	    o->compat_scaled_gradient, o->include_root_freqs, ctx->d_scratch);
-	ctx->launches++;
+	if ((rc = gen_branch_gradient(ctx, ctx->d_dP, o->scale, o->compat_scaled_gradient, o->include_root_freqs))) return rc;
 	return phbc_gradient_from_partials(ctx, (int)gtiles, result);
 }
 
@@ -822,6 +836,7 @@ int phbc_generic_evaluate(phbc_ctx *ctx, const phbc_eval_opts *o) {
 		return -1;
 	}
 	int rc;
+	if ((rc = phbc_smem_check(ctx, "generic kernels", 2))) return rc;
 	if ((rc = phbc_generic_prepare(ctx, o))) return rc;
 	ctx->lower_is_message = false;
 	ctx->node_evals++;
@@ -907,8 +922,10 @@ extern "C" int phbc_matrix_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, int 
 		if (frc != 1) return frc;
 	}
 	const bool tensor = phbc_dmma_supported(ctx, &e) && e.kernels != 1;
+	int rc;
+	if (!tensor && (rc = phbc_smem_check(ctx, "generic kernels", 2))) return rc;
 	ctx->last_family = tensor ? 3 : 1;
-	int rc = 0;
+	rc = 0;
 	const size_t set = N * C * S * S;
 	double *d_M = NULL, *d_cat = NULL, *d_out = NULL;
 	cudaError_t err = cudaMalloc((void **)&d_M, (size_t)nsets * set * sizeof(double));
@@ -941,16 +958,13 @@ extern "C" int phbc_matrix_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, int 
 	const size_t gtiles = (P + GEN_PGRAD - 1) / GEN_PGRAD;
 	if (err == cudaSuccess) {
 		rc = phbc_ensure_scratch(ctx, N * C * gtiles * sizeof(double));
-		const size_t smem = 2 * S * S * sizeof(double);
-		if (!rc && smem > 48 * 1024) err = cudaFuncSetAttribute(k_generic_branch_gradient, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-		Bufs b = phbc_make_bufs(ctx);
 		for (int k = 0; k < nsets && !rc && err == cudaSuccess; k++) {
-			k_generic_branch_gradient<<<dim3((unsigned)gtiles, (unsigned)(N - 1)), GEN_PGRAD, smem, ctx->stream>>>(
-			    b, ctx->root, ctx->d_P, d_M + (size_t)k * set, ctx->d_freqs, ctx->d_props, ctx->d_weights, ctx->d_pattern_lnl, e.scale,
-			    0 /* one site denominator: dlikelihood / likelihood, :2464-2474 */, e.include_root_freqs, ctx->d_scratch);
+			rc = gen_branch_gradient(ctx, d_M + (size_t)k * set, e.scale, 0 /* one site denominator: dlikelihood / likelihood, :2464-2474 */,
+			                         e.include_root_freqs);
+			if (rc) break;
 			k_generic_gradient_reduce<<<(unsigned)(((size_t)N * C * 32 + 127) / 128), 128, 0, ctx->stream>>>((int)N, (int)C, ctx->root, (int)gtiles, ctx->d_scratch,
 			                                                                                 d_cat + (size_t)k * N * C);
-			ctx->launches += 2;
+			ctx->launches++;
 		}
 		if (!rc && err == cudaSuccess) {
 			k_matrix_gradient_sum<<<nsets, 256, 0, ctx->stream>>>((int)N, (int)C, ctx->root, skip_node, d_cat, ctx->d_props, d_out);
@@ -981,6 +995,7 @@ extern "C" int phbc_run_ops(phbc_ctx *ctx, const phbc_eval_opts *o, int nops, co
 	PHBC_CHECK(cudaSetDevice(ctx->device));
 	const size_t S = ctx->S, C = ctx->C, P = ctx->P, N = ctx->N;
 	int rc;
+	if ((rc = phbc_smem_check(ctx, "generic kernels", 2))) return rc;
 	phbc_eval_opts e = *o;
 	e.batch_index = 0;
 	e.batch_count = 1;

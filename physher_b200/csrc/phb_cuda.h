@@ -198,6 +198,10 @@ int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmoves, const ph
 /* the call's matrix table and sums, allocated before the pruned pass changes anything: -1 when the state count needs more shared
  * memory than a CTA may have, -3 when the device cannot hold them */
 int phbc_spr_reserve(phbc_ctx *ctx, int ntargets);
+/* -1, with a message naming the state count and the bytes, unless one CTA can stage nmat S x S matrices of doubles in shared memory (the
+ * device's opt-in limit): 2 for the node-at-a-time kernels, 3 the single-branch pass, 4 NNI (any S), 5 SPR (any S).  Checked before
+ * the first launch of a call, so that a state count past the limit is refused as such and the object stays usable. */
+int phbc_smem_check(const phbc_ctx *ctx, const char *what, int nmat);
 int phbc_spr_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int s, int p, int ntargets, const int *targets, const double *bl, const double *ex,
                     double *out);
 int phbc_matrix_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, int nsets, const double *M_host, int skip_node, double *lnl, double *out_host);

@@ -184,13 +184,8 @@ static int spr_threads(const phbc_ctx *ctx) {
 // overwrites anything, so that a state count the kernels cannot stage (-1) or a device too small for the matrix table (-3) is reported
 // with the object unchanged
 static int spr_scratch(phbc_ctx *ctx, int ntargets, ScoreScratch *sc) {
-	const size_t S = ctx->S;
-	const size_t smem = 5 * S * S * sizeof(double);
-	if (S != 4 && smem > ctx->smem_optin) {
-		snprintf(phbc_errbuf, sizeof(phbc_errbuf), "SPR scores: %zu states need %zu bytes of shared memory for five matrices (at most %zu)", S, smem,
-		         ctx->smem_optin);
-		return -1;
-	}
+	int rc;
+	if (ctx->S != 4 && (rc = phbc_smem_check(ctx, "SPR scores", 5))) return rc;
 	const size_t n = ntargets > 0 ? (size_t)ntargets : 1;
 	const size_t tiles = ((size_t)ctx->P + spr_threads(ctx) - 1) / spr_threads(ctx);
 	return phbc_score_scratch(ctx, ctx->N + n, n, tiles, n * sizeof(int), sc);
@@ -227,7 +222,9 @@ extern "C" int phbc_spr_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int s, in
 	const int *d_targets = static_cast<int *>(sc.desc);
 	PHBC_CHECK(cudaMemcpyAsync(sc.desc, targets_host, n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
 	if ((rc = phbc_score_matrices(ctx, sc, N + n, bl_host, ex_host))) return rc;
-	if (S != 4 && smem > 48 * 1024) PHBC_CHECK(cudaFuncSetAttribute(k_spr_score_any, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+	// any S: the dynamic size is always declared -- the block-sum array's static bytes count toward the 48 KiB default too (35 states:
+	// 49,000 dynamic + 384 static bytes)
+	if (S != 4) PHBC_CHECK(cudaFuncSetAttribute(k_spr_score_any, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 	Bufs b = phbc_make_bufs(ctx);
 	if ((rc = phbc_time_begin(ctx))) return rc;
 	for (size_t k0 = 0; k0 < n; k0 += 65535) {

@@ -1308,10 +1308,11 @@ static int phb_tlk_calculate_branch_impl(phb_tlk *t, int node, int nbl, const do
 	if (t->have_matrices) return fail(PHB_ESTATE, "calculate_branch needs the eigen system: explicit matrices cannot be re-evaluated at a new length");
 	for (int k = 0; k < nbl; k++)
 		if (bl[k] < 0) return fail(PHB_EINVAL, "calculate_partials: node %d branch length = %E", node, bl[k]);
+	int rc = phbc_smem_check(t->ctx, "calculate_branch", 3);
+	if (rc) return dev_fail(rc);
 	resident_on(t);
 	double cur;
-	int rc = resident_calculate(t, &cur);
-	if (rc) return rc;
+	if ((rc = resident_calculate(t, &cur))) return rc;
 	if (isnan(cur) || isinf(cur)) {
 		for (int k = 0; k < nbl; k++) {
 			if (lnl) lnl[k] = cur;
@@ -1383,6 +1384,7 @@ static int phb_tlk_branch_hessian_diagonal_impl(phb_tlk *t, double *lnl, double 
 		}
 	}
 	if (!done) {
+		if ((rc = phbc_smem_check(t->ctx, "branch_hessian_diagonal", 3))) return dev_fail(rc);
 		resident_on(t);
 		if ((rc = resident_calculate(t, &cur))) return rc; /* retries with rescaling on itself */
 		if (!isnan(cur) && !isinf(cur)) {
@@ -1580,6 +1582,7 @@ static int phb_tlk_nni_scores_impl(phb_tlk *t, int nmoves, const int *moves, con
 	if (t->have_matrices) return fail(PHB_ESTATE, "nni_scores needs the eigen system: explicit matrices cannot be re-evaluated at a new length");
 	int rc = check_ready(t);
 	if (rc) return rc;
+	if (t->S != 4 && (rc = phbc_smem_check(t->ctx, "nni_scores", 4))) return dev_fail(rc);
 	const NniArgs a = {nmoves, moves, t_central};
 	return resident_scores(t, nmoves, lnl, out, nni_pass, &a);
 }
