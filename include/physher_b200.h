@@ -76,6 +76,8 @@ extern "C" {
  *   phb_tlk_calculate_branch, phb_tlk_branch_hessian_diagonal (resident)  3 S^2 x 8 bytes   [S <= 98]
  *   phb_tlk_nni_scores (S != 4)                                           4 S^2 x 8 bytes   [S <= 85]
  *   phb_tlk_spr_scores (S != 4)                                           5 S^2 x 8 bytes   [S <= 76]
+ *   phb_tlk_spr_tripod_scores: the pruned pass on the node-at-a-time      2 S^2 x 8 bytes   [S <= 120]
+ *     kernels (its contraction stages its nine matrices in chunks of rows of at most 48 KiB and adds no lower limit)
  * Past its limit a call returns PHB_EINVAL, with a message naming the state count and the bytes it needs, before it launches its kernels;
  * the object stays usable for the calls whose limit it is within. */
 
@@ -282,6 +284,29 @@ int phb_tlk_nni_scores(phb_tlk *tlk, int nmoves, const int *moves /* [nmoves][2]
 int phb_tlk_spr_targets(phb_tlk *tlk, int s, int *targets /* [count] or NULL */);
 int phb_tlk_spr_scores(phb_tlk *tlk, int s, int ntargets, const int *targets, const double *t_pendant /* [ntargets] or NULL */,
                        double *lnl, double *out /* [ntargets][3] */);
+
+/*
+ * phb_tlk_spr_tripod_scores: the SPR scores with the three branches that meet at the regraft point at lengths of their own -- what the
+ * reference's SPR driver optimises after each regraft (the tripod, spropt.c:1578-1608).  Names as above.
+ *   pruned tree      b's branch is joined: l_b = t_b + t_p, or *t_join when t_join is not NULL; no other length changes.
+ *   regrafted tree   on target e, with h e's parent in the pruned tree: node p's branch (h - p) is t_up, node e's branch (p - e) t_down and
+ *                    node s's branch t_pend, from t_tripod[k] = {t_up, t_down, t_pend}; NULL: t_up = t_down = l_e / 2 with l_e e's length
+ *                    in the pruned tree (l_b for e = b) and t_pend = t_s.  Every other branch keeps its length, b keeps l_b unless e = b.
+ *   out[k]           {lnL, g_up, g_down, g_pend, H_uu, H_dd, H_pp, H_ud, H_up, H_dp} of the tree regrafted on targets[k].
+ * With the pruned tree's U~_e and L~_e (as above):
+ *   A = P(t_up) U~_e      B = P(t_down) L~_e      Z = P(t_pend) L_s      L_k = sum_c prop_c sum_i pi_i A_i B_i Z_i
+ * A first derivative replaces one factor's matrix by r_c P', a diagonal second derivative by r_c^2 P", a mixed one puts r_c P' in two
+ * factors; the sums are g_a = sum w L_a / L and H_ab = sum w (L_ab / L - L_a L_b / L^2).  The derivatives are the exact ones:
+ * PHB_OPT_INCLUDE_ROOT_FREQS, PHB_OPT_COMPAT_SCALED_GRADIENT and the unrooted zeroing do not apply.  With t_join = t_b and t_tripod[k] =
+ * {t_p, t_e, t_s}, lnL, g_pend and H_pp are those of phb_tlk_spr_scores; target b with t_up = t_p, t_down = t_b and the default join is
+ * the current tree.
+ * Everything else is as phb_tlk_spr_scores: *lnl, PHB_OPT_INCREMENTAL, what is marked invalid, the rescaling retry, the refusals (plus
+ * PHB_EINVAL for a negative or NaN length in t_tripod or *t_join), PHB_ESTATE, PHB_ENOMEM.  The joined length reaches the pruned pass
+ * through b's transition matrix, which the call rebuilds at l_b and then, with every other matrix, at the current lengths again: after
+ * the call, phb_tlk_calculate, phb_tlk_gradient, phb_tlk_branch_hessian_diagonal and phb_tlk_spr_scores return what they returned before.
+ */
+int phb_tlk_spr_tripod_scores(phb_tlk *tlk, int s, int ntargets, const int *targets, const double *t_tripod /* [ntargets][3] or NULL */,
+                              const double *t_join /* or NULL */, double *lnl, double *out /* [ntargets][10] */);
 
 /*
  * phb_tlk_update_partials == the struct slot tlk->update_partials(tlk, out, p1, m1, p2, m2) (treelikelihood.h:91), for the callers

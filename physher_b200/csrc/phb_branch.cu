@@ -139,9 +139,9 @@ int phbc_score_resident(const phbc_ctx *ctx, const phbc_eval_opts *o) {
 }
 
 // grows ctx->d_branch to the pass's layout (the stream is drained before the old buffer goes) and carves it
-int phbc_score_scratch(phbc_ctx *ctx, size_t items, size_t nout, size_t tiles, size_t desc_bytes, ScoreScratch *sc) {
-	const size_t S = ctx->S, C = ctx->C;
-	const size_t need = (items * (1 + C * 3 * S * S + C * S) + nout * (3 + 3 * tiles) + (desc_bytes + 7) / 8) * sizeof(double);
+int phbc_score_scratch(phbc_ctx *ctx, size_t items, size_t nout, int nterms, size_t tiles, size_t desc_bytes, ScoreScratch *sc) {
+	const size_t S = ctx->S, C = ctx->C, nt = (size_t)nterms;
+	const size_t need = (items * (1 + C * 3 * S * S + C * S) + nout * (nt + nt * tiles) + (desc_bytes + 7) / 8) * sizeof(double);
 	if (need > ctx->branch_bytes) {
 		PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
 		if (ctx->d_branch) cudaFree(ctx->d_branch);
@@ -153,9 +153,9 @@ int phbc_score_scratch(phbc_ctx *ctx, size_t items, size_t nout, size_t tiles, s
 	}
 	sc->bl = ctx->d_branch;
 	sc->out = sc->bl + items;
-	sc->mats = sc->out + 3 * nout;
+	sc->mats = sc->out + nt * nout;
 	sc->part = sc->mats + items * C * 3 * S * S;
-	sc->ex = sc->part + nout * 3 * tiles;
+	sc->ex = sc->part + nout * nt * tiles;
 	sc->desc = sc->ex + items * C * S;
 	return 0;
 }
@@ -172,12 +172,12 @@ int phbc_score_matrices(phbc_ctx *ctx, const ScoreScratch &sc, size_t items, con
 	return 0;
 }
 
-// out_host [nout][3] = the per-CTA sums [nout][3][tiles] summed in a fixed order; synchronous
-int phbc_score_finish(phbc_ctx *ctx, const ScoreScratch &sc, size_t nout, size_t tiles, double *out_host) {
-	k_branch_sum<<<(unsigned)(3 * nout), 256, 0, ctx->stream>>>(sc.part, (int)tiles, sc.out);
+// out_host [nout][nterms] = the per-CTA sums [nout][nterms][tiles] summed in a fixed order; synchronous
+int phbc_score_finish(phbc_ctx *ctx, const ScoreScratch &sc, size_t nout, int nterms, size_t tiles, double *out_host) {
+	k_branch_sum<<<(unsigned)(nterms * nout), 256, 0, ctx->stream>>>(sc.part, (int)tiles, sc.out);
 	ctx->launches++;
 	PHBC_CHECK(cudaGetLastError());
-	PHBC_CHECK(cudaMemcpyAsync(out_host, sc.out, 3 * nout * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+	PHBC_CHECK(cudaMemcpyAsync(out_host, sc.out, nterms * nout * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
 	PHBC_CHECK(cudaStreamSynchronize(ctx->stream));
 	return 0;
 }
@@ -207,7 +207,7 @@ extern "C" int phbc_branch_lnl(phbc_ctx *ctx, const phbc_eval_opts *o, int nitem
 	const size_t S = ctx->S, C = ctx->C, n = (size_t)nitems;
 	const size_t tiles = ((size_t)ctx->P + BR_THREADS - 1) / BR_THREADS;
 	ScoreScratch sc;
-	if ((rc = phbc_score_scratch(ctx, n, n, tiles, n * sizeof(int), &sc))) return rc;
+	if ((rc = phbc_score_scratch(ctx, n, n, 3, tiles, n * sizeof(int), &sc))) return rc;
 	const int *d_nodes = static_cast<int *>(sc.desc);
 	PHBC_CHECK(cudaMemcpyAsync(sc.desc, nodes_host, n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
 	if ((rc = phbc_score_matrices(ctx, sc, n, bl_host, ex_host))) return rc;
@@ -222,5 +222,5 @@ extern "C" int phbc_branch_lnl(phbc_ctx *ctx, const phbc_eval_opts *o, int nitem
 		ctx->launches++;
 	}
 	if ((rc = phbc_time_end(ctx))) return rc;
-	return phbc_score_finish(ctx, sc, n, tiles, out_host);
+	return phbc_score_finish(ctx, sc, n, 3, tiles, out_host);
 }

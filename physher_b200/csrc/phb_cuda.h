@@ -204,6 +204,14 @@ int phbc_spr_reserve(phbc_ctx *ctx, int ntargets);
 int phbc_smem_check(const phbc_ctx *ctx, const char *what, int nmat);
 int phbc_spr_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int s, int p, int ntargets, const int *targets, const double *bl, const double *ex,
                     double *out);
+/* SPR tripod scores (phb_spr.cu): out [ntargets][10] = lnL, the gradient in (t_up, t_down, t_pend) and the Hessian entries uu, dd, pp,
+ * ud, up, dp of the subtree of s regrafted on each target with the three branches at the regraft point at lengths of their own, from the
+ * pruned tree's partials the caller left in the resident buffers; bl [N + 3 ntargets] the matrix table's lengths (node n = entry n,
+ * target k's t_up, t_down, t_pend = entries N + 3k, N + 3k + 1, N + 3k + 2), ex (may be NULL) their exponentials.  The reserve sizes the
+ * table before the pruned pass (-1 past the pruned pass's state-count limit, -3 when the device cannot hold it). */
+int phbc_spr_tripod_reserve(phbc_ctx *ctx, int ntargets);
+int phbc_spr_tripod_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int s, int ntargets, const int *targets, const double *bl, const double *ex,
+                           double *out);
 int phbc_matrix_gradient(phbc_ctx *ctx, const phbc_eval_opts *o, int nsets, const double *M_host, int skip_node, double *lnl, double *out_host);
 /* time-tree chain, batched (phb_timetree.cu) */
 int phbc_set_time_tree(phbc_ctx *ctx, const double *lowers, const int *parent, const int *preorder, const int *postorder);

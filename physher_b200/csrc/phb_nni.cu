@@ -272,7 +272,7 @@ extern "C" int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmove
 	const size_t n = (size_t)nmoves, items = N + n;
 	const size_t tiles = (P + NNI_THREADS - 1) / NNI_THREADS;
 	ScoreScratch sc;
-	if ((rc = phbc_score_scratch(ctx, items, n, tiles, 2 * (size_t)ngroups * sizeof(int) + n * sizeof(phbc_nni_move), &sc))) return rc;
+	if ((rc = phbc_score_scratch(ctx, items, n, 3, tiles, 2 * (size_t)ngroups * sizeof(int) + n * sizeof(phbc_nni_move), &sc))) return rc;
 	int2 *d_groups = static_cast<int2 *>(sc.desc);  // the 32-byte descriptors follow
 	phbc_nni_move *d_moves = reinterpret_cast<phbc_nni_move *>(d_groups + ngroups);
 	PHBC_CHECK(cudaMemcpyAsync(d_moves, moves_host, n * sizeof(phbc_nni_move), cudaMemcpyHostToDevice, ctx->stream));
@@ -326,7 +326,7 @@ extern "C" int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmove
 			}
 		}
 		if ((rc = phbc_time_end(ctx))) return rc;
-		return phbc_score_finish(ctx, sc, n, tiles, out_host);
+		return phbc_score_finish(ctx, sc, n, 3, tiles, out_host);
 	};
 	rc = launch();
 	if (d_vec) {  // on every path: the stream is drained before the scratch goes

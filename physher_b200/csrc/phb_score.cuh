@@ -1,13 +1,14 @@
 // phb_score.cuh -- the score passes on resident partials (internal): the single-branch path and the Hessian diagonal (phb_branch.cu),
-// NNI scores (phb_nni.cu) and SPR scores (phb_spr.cu).
+// NNI scores (phb_nni.cu), SPR scores and SPR tripod scores (phb_spr.cu).
 //
-// Every pass has the same frame around its own score kernel:
-//   phbc_score_scratch   ctx->d_branch carved as  bl [items] | out [nout][3] | mats [items][C][3][S*S] | part [nout][3][tiles] |
-//                        ex [items][C][S] | the pass's descriptors
+// Every pass has the same frame around its own score kernel; nterms is the number of terms per output row (3: lnL and one branch's
+// first and second derivatives; 10 for the tripod: lnL, three first derivatives, the six entries of a symmetric 3 x 3 Hessian):
+//   phbc_score_scratch   ctx->d_branch carved as  bl [items] | out [nout][nterms] | mats [items][C][3][S*S] |
+//                        part [nout][nterms][tiles] | ex [items][C][S] | the pass's descriptors
 //   phbc_score_matrices  the lengths (and host exponentials) up, one k_branch_matrices launch: P, r P', r^2 P" of every table item
-//   score kernel(s)      per-pattern terms (score_terms), block sums into part [row][3][tile] (score_block_sum)
+//   score kernel(s)      per-pattern terms (score_terms), block sums into part [row][nterms][tile] (score_block_sum)
 //   phbc_score_finish    k_branch_sum over the tiles in a fixed order (bit-identical from run to run, no floating-point atomics) and
-//                        the [nout][3] results down
+//                        the [nout][nterms] results down
 #pragma once
 
 #include "phb_ctx.cuh"
@@ -22,9 +23,9 @@ struct ScoreScratch {
 	double *bl, *out, *mats, *part, *ex;
 	void *desc;  // 8-byte aligned
 };
-int phbc_score_scratch(phbc_ctx *ctx, size_t items, size_t nout, size_t tiles, size_t desc_bytes, ScoreScratch *sc);
+int phbc_score_scratch(phbc_ctx *ctx, size_t items, size_t nout, int nterms, size_t tiles, size_t desc_bytes, ScoreScratch *sc);
 int phbc_score_matrices(phbc_ctx *ctx, const ScoreScratch &sc, size_t items, const double *bl_host, const double *ex_host);
-int phbc_score_finish(phbc_ctx *ctx, const ScoreScratch &sc, size_t nout, size_t tiles, double *out_host);
+int phbc_score_finish(phbc_ctx *ctx, const ScoreScratch &sc, size_t nout, int nterms, size_t tiles, double *out_host);
 // -4 unless the resident buffers the score kernels read are there: uppers, lowers, scale factors under rescaling, tip partials
 int phbc_score_resident(const phbc_ctx *ctx, const phbc_eval_opts *o);
 
@@ -39,18 +40,18 @@ __device__ __forceinline__ void score_terms(double plk, double L, double dL, dou
 	v[2] = (d2L / L - r1 * r1) * w;
 }
 
-// Block sum of the three terms into partial [row][3][tiles]: red is shared [3][WARPS]; nwarps the warps of the block (<= WARPS), 0 for
+// Block sum of the NT terms into partial [row][NT][tiles]: red is shared [NT][WARPS]; nwarps the warps of the block (<= WARPS), 0 for
 // blockDim.x / 32.
-template <int WARPS>
-__device__ __forceinline__ void score_block_sum(double (*red)[WARPS], const double *v, int nwarps, int row, double *partial) {
-	for (int q = 0; q < 3; q++) {
+template <int NT, int WARPS>
+__device__ __forceinline__ void score_block_sum(double (&red)[NT][WARPS], const double *v, int nwarps, int row, double *partial) {
+	for (int q = 0; q < NT; q++) {
 		const double s = phb_warp_sum(v[q]);
 		if ((threadIdx.x & 31) == 0) red[q][threadIdx.x >> 5] = s;
 	}
 	__syncthreads();
-	if (threadIdx.x < 3) {
+	if (threadIdx.x < NT) {
 		double s = 0.0;
 		for (int w = 0; w < (nwarps ? nwarps : (int)(blockDim.x >> 5)); w++) s += red[threadIdx.x][w];
-		partial[((size_t)row * 3 + threadIdx.x) * gridDim.x + blockIdx.x] = s;
+		partial[((size_t)row * NT + threadIdx.x) * gridDim.x + blockIdx.x] = s;
 	}
 }

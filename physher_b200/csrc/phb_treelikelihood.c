@@ -1073,12 +1073,15 @@ static int upload_host_exponentials(phb_tlk *t, const double *bl, int nbatch) {
 	return phbc_upload_exponentials(t->ctx, t->ex_buf, nbatch);
 }
 
-static int upload_bl(phb_tlk *t) {
-	int rc = phbc_upload_branch_lengths(t->ctx, t->bl, 1);
+/* one branch-length vector [N] (and its host exponentials) to the device: the next matrix rebuild uses it */
+static int upload_lengths(phb_tlk *t, const double *bl) {
+	int rc = phbc_upload_branch_lengths(t->ctx, bl, 1);
 	if (rc) return rc;
-	if (wants_host_exp(t)) rc = upload_host_exponentials(t, t->bl, 1);
+	if (wants_host_exp(t)) rc = upload_host_exponentials(t, bl, 1);
 	return rc;
 }
+
+static int upload_bl(phb_tlk *t) { return upload_lengths(t, t->bl); }
 
 /* one full evaluation with the reference's NaN / inf handling (treelikelihood.c:1489-1519) */
 static int evaluate_once(phb_tlk *t, int want_gradient, double *lnl, double *grad_out) {
@@ -1541,11 +1544,12 @@ done:
 
 /*
  * The score calls on resident partials (NNI, SPR): reserve the resident buffers (-3 with the object unchanged), make the lowers resident
- * (PHB_OPT_INCREMENTAL on), then one pass writing out [n][3].  NaN / inf as treelikelihood.c:1496-1519: an infinite lnL of the current
+ * (PHB_OPT_INCREMENTAL on), then one pass writing out [n][nterms].  NaN / inf as treelikelihood.c:1496-1519: an infinite lnL of the current
  * tree, or an output that is not finite while rescaling is off, switches rescaling on and scores once more; a current lnL still NaN or
  * infinite NaN-fills out.
  */
-static int resident_scores(phb_tlk *t, int n, double *lnl, double *out, int (*pass)(phb_tlk *, const void *, double *), const void *arg) {
+static int resident_scores(phb_tlk *t, int n, int nterms, double *lnl, double *out, int (*pass)(phb_tlk *, const void *, double *),
+                           const void *arg) {
 	phbc_eval_opts o;
 	fill_opts(t, &o, 1, 0);
 	int rc = phbc_generic_buffers(t->ctx, &o);
@@ -1557,14 +1561,14 @@ static int resident_scores(phb_tlk *t, int n, double *lnl, double *out, int (*pa
 		if (isnan(cur) || isinf(cur)) break;
 		if ((rc = pass(t, arg, out))) return rc;
 		int finite = 1;
-		for (int k = 0; k < 3 * n; k++) finite &= isfinite(out[k]) != 0;
+		for (int k = 0; k < nterms * n; k++) finite &= isfinite(out[k]) != 0;
 		if (finite || t->scale) break;
 		t->scale = 1; /* something underflowed unscaled: rescale everything and score again */
 		t->all_dirty = 1;
 	}
 	if (lnl) *lnl = cur;
 	if (isnan(cur) || isinf(cur))
-		for (int k = 0; k < 3 * n; k++) out[k] = NAN;
+		for (int k = 0; k < nterms * n; k++) out[k] = NAN;
 	return PHB_OK;
 }
 
@@ -1584,7 +1588,7 @@ static int phb_tlk_nni_scores_impl(phb_tlk *t, int nmoves, const int *moves, con
 	if (rc) return rc;
 	if (t->S != 4 && (rc = phbc_smem_check(t->ctx, "nni_scores", 4))) return dev_fail(rc);
 	const NniArgs a = {nmoves, moves, t_central};
-	return resident_scores(t, nmoves, lnl, out, nni_pass, &a);
+	return resident_scores(t, nmoves, 3, lnl, out, nni_pass, &a);
 }
 
 /*
@@ -1640,21 +1644,42 @@ static int phb_tlk_spr_targets_impl(phb_tlk *t, int s, int *targets) {
  *   lowers  g's op becomes (b, b) o (q, q) on the side p had, every ancestor of g below the root takes its usual op (nothing when g is
  *           the root; the root's own lower partial is never written);
  *   uppers  the pruned tree's upper op of every node outside {p} and the subtree of s, grouped by their depth in the pruned tree.
- * Current matrices (no rebuild), no root integration.  The validity maps lose exactly what the pass overwrites: lower_ok of g and its
- * ancestors below the root (lower_stale: the next evaluation recomputes them, and the cached lnL stays that of the current tree) and
- * upper_ok of every node it wrote; the uppers of p and of the subtree of s are untouched.
+ * Current matrices, no root integration.  b's branch in the pruned tree has the length `join`: where that differs from t_b (the tripod
+ * scores join b's and p's branches), b's matrix slot -- read by the pruned pass exactly where the pruned tree uses b's branch -- is
+ * rebuilt at that length first, and every matrix is rebuilt from the current lengths once the pruned partials are written, so that
+ * nothing after the call sees it.  The validity maps lose exactly what the pass overwrites: lower_ok of g and its ancestors below the
+ * root (lower_stale: the next evaluation recomputes them, and the cached lnL stays that of the current tree) and upper_ok of every node
+ * it wrote; the uppers of p and of the subtree of s are untouched.
  */
 typedef struct SprArgs {
 	int s, ntargets;
 	const int *targets;
-	const double *t_pendant;
+	const double *t_pendant; /* spr_scores: [ntargets] or NULL */
+	const double *t_tripod;  /* spr_tripod_scores: [ntargets][3] or NULL */
+	double join;             /* b's length in the pruned tree */
+	int tripod;
 } SprArgs;
+
+/* the tripod's matrix table: every node at its current length (the root's entry unused, 0), then t_up, t_down, t_pend of each target --
+ * given[3k ..], or half of e's length in the pruned tree (join for e = b) twice and t_s */
+static void tripod_lengths(const phb_tlk *t, int ntargets, const int *targets, const double *given, int s, int b, double join, double *bl) {
+	table_lengths(t, 0, NULL, NULL, 0, bl);
+	for (int k = 0; k < ntargets; k++) {
+		const double half = (targets[k] == b ? join : t->bl[targets[k]]) / 2;
+		double *row = bl + t->N + 3 * (size_t)k;
+		row[0] = given ? given[3 * k] : half;
+		row[1] = given ? given[3 * k + 1] : half;
+		row[2] = given ? given[3 * k + 2] : t->bl[s];
+	}
+}
+
 static int spr_pass(phb_tlk *t, const void *arg, double *out) {
 	const SprArgs *a = (const SprArgs *)arg;
 	const int s = a->s, ntargets = a->ntargets;
 	const int N = t->N, C = t->C, S = t->S, root = t->root;
 	const int p = t->parent[s], g = t->parent[p], b = sibling_of(t, s);
-	const size_t items = (size_t)N + ntargets;
+	int joined = a->join != t->bl[b];
+	const size_t items = (size_t)N + (a->tripod ? 3 : 1) * (size_t)ntargets;
 	int *queue = (int *)malloc(sizeof(int) * N);
 	int *depth = (int *)malloc(sizeof(int) * N);
 	double *bl = (double *)malloc(sizeof(double) * items);
@@ -1666,6 +1691,14 @@ static int spr_pass(phb_tlk *t, const void *arg, double *out) {
 	}
 	t->sweep_valid = 0;
 	phbc_eval_opts o;
+	if (joined) { /* b's matrix at the joined length; the rebuild comes with the lower ops below */
+		memcpy(bl, t->bl, sizeof(double) * N);
+		bl[b] = a->join;
+		if ((rc = upload_lengths(t, bl))) {
+			rc = dev_fail(rc);
+			goto done;
+		}
+	}
 	int nops = 0;
 	for (int x = g; x != root; x = t->parent[x]) { /* one level each, children before parents */
 		int l = t->left[x], r = t->right[x];
@@ -1677,10 +1710,10 @@ static int spr_pass(phb_tlk *t, const void *arg, double *out) {
 		t->lower_ok[x] = 0;
 	}
 	t->sub_level_off[nops] = nops;
-	if (nops) {
-		t->lower_stale = 1;
+	if (nops) t->lower_stale = 1;
+	if (nops || joined) {
 		fill_opts_resident(t, &o, 0);
-		if ((rc = phbc_run_ops(t->ctx, &o, nops, t->sub_ops, nops, t->sub_level_off, 0, 0, NULL))) {
+		if ((rc = phbc_run_ops(t->ctx, &o, nops, t->sub_ops, nops, t->sub_level_off, joined, 0, NULL))) {
 			rc = dev_fail(rc);
 			goto done;
 		}
@@ -1718,22 +1751,42 @@ static int spr_pass(phb_tlk *t, const void *arg, double *out) {
 		rc = dev_fail(rc);
 		goto done;
 	}
-	table_lengths(t, ntargets, a->t_pendant, &s, 0, bl); /* the pendant branch is s's */
+	if (joined) { /* every matrix back at the current lengths: the same inputs give the same bits */
+		if ((rc = upload_bl(t))) {
+			rc = dev_fail(rc);
+			goto done;
+		}
+		fill_opts_resident(t, &o, 0);
+		if ((rc = phbc_run_ops(t->ctx, &o, 0, NULL, 0, t->sub_level_off, 1, 0, NULL))) {
+			rc = dev_fail(rc);
+			goto done;
+		}
+		joined = 0;
+	}
+	if (a->tripod)
+		tripod_lengths(t, ntargets, a->targets, a->t_tripod, s, b, a->join, bl);
+	else
+		table_lengths(t, ntargets, a->t_pendant, &s, 0, bl); /* the pendant branch is s's */
 	if (ex) host_exponentials(t, items, bl, ex);
 	fill_opts_resident(t, &o, 1);
-	if ((rc = phbc_spr_scores(t->ctx, &o, s, p, ntargets, a->targets, bl, ex, out))) rc = dev_fail(rc);
+	if (a->tripod)
+		rc = phbc_spr_tripod_scores(t->ctx, &o, s, ntargets, a->targets, bl, ex, out);
+	else
+		rc = phbc_spr_scores(t->ctx, &o, s, p, ntargets, a->targets, bl, ex, out);
+	if (rc) rc = dev_fail(rc);
 done:
+	if (joined) t->all_dirty = 1; /* the matrices may still hold the joined length: the next evaluation is a full one */
 	free(queue), free(depth), free(bl), free(ex);
 	return rc;
 }
 
-/* lnL and pendant-branch derivatives of the subtree of s regrafted on each listed target, from one pass over the pruned tree (phb_spr.cu);
- * the matrix table is reserved with the resident buffers, before the pruned pass changes anything */
-static int phb_tlk_spr_scores_impl(phb_tlk *t, int s, int ntargets, const int *targets, const double *t_pendant, double *lnl, double *out) {
-	int rc = spr_check_prune(t, "spr_scores", s);
+/* the checks both SPR score calls share: s, out, the targets, and their lengths lens [ntargets][nlen] (may be NULL) */
+static int spr_check(phb_tlk *t, const char *fn, int s, int ntargets, const int *targets, const double *lens, int nlen, const char *lname,
+                     const double *out) {
+	int rc = spr_check_prune(t, fn, s);
 	if (rc) return rc;
-	if (!targets || !out) return fail(PHB_EINVAL, "spr_scores: targets and out are required");
-	if (ntargets < 1) return fail(PHB_EINVAL, "spr_scores: %d targets (at least one is needed)", ntargets);
+	if (!targets || !out) return fail(PHB_EINVAL, "%s: targets and out are required", fn);
+	if (ntargets < 1) return fail(PHB_EINVAL, "%s: %d targets (at least one is needed)", fn, ntargets);
 	unsigned char *mark = (unsigned char *)malloc(t->N);
 	int *stack = (int *)malloc(sizeof(int) * t->N);
 	if (!mark || !stack) {
@@ -1745,17 +1798,37 @@ static int phb_tlk_spr_scores_impl(phb_tlk *t, int s, int ntargets, const int *t
 	for (int k = 0; k < ntargets && !rc; k++) {
 		const int e = targets[k];
 		if (e < 0 || e >= t->N || e == t->root || e == p || mark[e])
-			rc = fail(PHB_EINVAL, "spr_scores: target %d (node %d) is not a regraft position of the subtree of %d", k, e, s);
-		else if (t_pendant && !(t_pendant[k] >= 0))
-			rc = fail(PHB_EINVAL, "spr_scores: target %d pendant branch length = %E", k, t_pendant[k]);
+			rc = fail(PHB_EINVAL, "%s: target %d (node %d) is not a regraft position of the subtree of %d", fn, k, e, s);
+		for (int j = 0; lens && j < nlen && !rc; j++)
+			if (!(lens[(size_t)k * nlen + j] >= 0)) rc = fail(PHB_EINVAL, "%s: target %d %s = %E", fn, k, lname, lens[(size_t)k * nlen + j]);
 	}
 	free(mark), free(stack);
 	if (rc) return rc;
-	if (t->have_matrices) return fail(PHB_ESTATE, "spr_scores needs the eigen system: explicit matrices cannot be re-evaluated at a new length");
-	if ((rc = check_ready(t))) return rc;
+	if (t->have_matrices) return fail(PHB_ESTATE, "%s needs the eigen system: explicit matrices cannot be re-evaluated at a new length", fn);
+	return check_ready(t);
+}
+
+/* lnL and pendant-branch derivatives of the subtree of s regrafted on each listed target, from one pass over the pruned tree (phb_spr.cu);
+ * the matrix table is reserved with the resident buffers, before the pruned pass changes anything */
+static int phb_tlk_spr_scores_impl(phb_tlk *t, int s, int ntargets, const int *targets, const double *t_pendant, double *lnl, double *out) {
+	int rc = spr_check(t, "spr_scores", s, ntargets, targets, t_pendant, 1, "pendant branch length", out);
+	if (rc) return rc;
 	if ((rc = phbc_spr_reserve(t->ctx, ntargets))) return dev_fail(rc);
-	const SprArgs a = {s, ntargets, targets, t_pendant};
-	return resident_scores(t, ntargets, lnl, out, spr_pass, &a);
+	const SprArgs a = {s, ntargets, targets, t_pendant, NULL, t->bl[sibling_of(t, s)], 0};
+	return resident_scores(t, ntargets, 3, lnl, out, spr_pass, &a);
+}
+
+/* lnL, gradient and Hessian in the three branches at the regraft point (spropt.c:1578-1608 optimises them after each regraft) of the
+ * subtree of s regrafted on each listed target, b's branch joined with p's in the pruned tree; one pass, as the SPR scores */
+static int phb_tlk_spr_tripod_scores_impl(phb_tlk *t, int s, int ntargets, const int *targets, const double *t_tripod, const double *t_join,
+                                          double *lnl, double *out) {
+	int rc = spr_check(t, "spr_tripod_scores", s, ntargets, targets, t_tripod, 3, "tripod branch length", out);
+	if (rc) return rc;
+	if (t_join && !(*t_join >= 0)) return fail(PHB_EINVAL, "spr_tripod_scores: joined branch length = %E", *t_join);
+	if ((rc = phbc_spr_tripod_reserve(t->ctx, ntargets))) return dev_fail(rc);
+	const int p = t->parent[s], b = sibling_of(t, s);
+	const SprArgs a = {s, ntargets, targets, NULL, t_tripod, t_join ? *t_join : t->bl[b] + t->bl[p], 1};
+	return resident_scores(t, ntargets, 10, lnl, out, spr_pass, &a);
 }
 
 /*
@@ -2420,6 +2493,14 @@ int phb_tlk_spr_targets(phb_tlk *t, int s, int *targets) { return phb_tlk_spr_ta
 int phb_tlk_spr_scores(phb_tlk *t, int s, int ntargets, const int *targets, const double *t_pendant, double *lnl, double *out) {
 	nvtxRangePushA("phb_tlk_spr_scores");
 	const int rc = phb_tlk_spr_scores_impl(t, s, ntargets, targets, t_pendant, lnl, out);
+	nvtxRangePop();
+	return rc;
+}
+
+int phb_tlk_spr_tripod_scores(phb_tlk *t, int s, int ntargets, const int *targets, const double *t_tripod, const double *t_join, double *lnl,
+                              double *out) {
+	nvtxRangePushA("phb_tlk_spr_tripod_scores");
+	const int rc = phb_tlk_spr_tripod_scores_impl(t, s, ntargets, targets, t_tripod, t_join, lnl, out);
 	nvtxRangePop();
 	return rc;
 }

@@ -75,6 +75,7 @@ SYMBOLS = [
     ("phb_tlk_nni_scores", C.c_int, [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp]),
     ("phb_tlk_spr_targets", C.c_int, [C.c_void_p, C.c_int, _ip]),
     ("phb_tlk_spr_scores", C.c_int, [C.c_void_p, C.c_int, C.c_int, _ip, _dp, _dp, _dp]),
+    ("phb_tlk_spr_tripod_scores", C.c_int, [C.c_void_p, C.c_int, C.c_int, _ip, _dp, _dp, _dp, _dp]),
     ("phb_tlk_update_partials", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _dp]),
     ("phb_tlk_get_partials", C.c_int, [C.c_void_p, C.c_int, _dp]),
     ("phb_tlk_get_matrices", C.c_int, [C.c_void_p, _dp, _dp]),
@@ -515,6 +516,24 @@ class SingleTreeLikelihood:
         self._check(self.lib.phb_tlk_spr_scores(self.h, int(s), int(tg.shape[0]), tg.ctypes.data_as(_ip),
                                                 None if tp is None else tp.ctypes.data_as(_dp), C.byref(lnl), out.ctypes.data_as(_dp)))
         return lnl.value, out
+
+    def spr_tripod_scores(self, s, targets=None, t_tripod=None, t_join=None):
+        """lnL, gradient and Hessian in (t_up, t_down, t_pend), the three branches at the regraft point, of the tree the subtree of s
+        (pruned with its parent, b's branch joined at t_join, None: t_b + t_p) regrafted on the branch above each target gives, the
+        tripod at t_tripod[k] (None: half of the target's pruned length twice and t_s), in one call on resident partials:
+        (lnl[n] of each regrafted tree, grad[n, 3], hess[n, 3, 3]); calculate() gives the current tree's.  targets=None scores every
+        target of spr_targets(s)."""
+        tg = self.spr_targets(s) if targets is None else np.ascontiguousarray(targets, dtype=np.int32).reshape(-1)
+        tt = None if t_tripod is None else np.ascontiguousarray(t_tripod, dtype=np.float64).reshape(-1)
+        if tt is not None and tt.shape[0] != 3 * tg.shape[0]:
+            raise ValueError("t_tripod needs three lengths per target")
+        tj = None if t_join is None else C.c_double(float(t_join))
+        out = np.zeros((tg.shape[0], 10))
+        self._check(self.lib.phb_tlk_spr_tripod_scores(self.h, int(s), int(tg.shape[0]), tg.ctypes.data_as(_ip),
+                                                       None if tt is None else tt.ctypes.data_as(_dp),
+                                                       None if tj is None else C.cast(C.byref(tj), _dp), None, out.ctypes.data_as(_dp)))
+        hess = out[:, [4, 7, 8, 7, 5, 9, 8, 9, 6]].reshape(-1, 3, 3)
+        return out[:, 0].copy(), out[:, 1:4].copy(), hess
 
     def update_partials(self, out, p1, m1, p2=-1, m2=-1, mirror=True):
         """tlk->update_partials(tlk, out, p1, m1, p2, m2) (treelikelihood.h:91) on the resident device buffers; returns the result."""
