@@ -78,6 +78,8 @@ extern "C" {
  *   phb_tlk_spr_scores (S != 4)                                           5 S^2 x 8 bytes   [S <= 76]
  *   phb_tlk_spr_tripod_scores: the pruned pass on the node-at-a-time      2 S^2 x 8 bytes   [S <= 120]
  *     kernels (its contraction stages its nine matrices in chunks of rows of at most 48 KiB and adds no lower limit)
+ *   phb_tlk_nni_quintet_scores: the resident partials on the node-at-   2 S^2 x 8 bytes   [S <= 120]
+ *     a-time kernels (its any-S contraction keeps 12 S-vectors per pattern in shared memory, at most 92 KiB, and adds no lower limit)
  * Past its limit a call returns PHB_EINVAL, with a message naming the state count and the bytes it needs, before it launches its kernels;
  * the object stays usable for the calls whose limit it is within. */
 
@@ -249,6 +251,28 @@ int phb_tlk_branch_hessian_diagonal(phb_tlk *tlk, double *lnl, double *grad /* [
 int phb_tlk_nni_moves(phb_tlk *tlk, int *moves /* [count][2] or NULL */);
 int phb_tlk_nni_scores(phb_tlk *tlk, int nmoves, const int *moves /* [nmoves][2] */, const double *t_central /* [nmoves] or NULL */,
                        double *lnl, double *out /* [nmoves][3] */);
+
+/*
+ * phb_tlk_nni_quintet_scores: the NNI scores with the central branch and the four branches around it at lengths of their own -- the
+ * Newton terms a driver needs to re-fit a move's neighbourhood before it accepts it (an exchange leaves the four branches at lengths
+ * fitted to the old topology).  Names as above; in the exchanged tree the central edge joins v's end, where keep and x hang, and the far
+ * end, where y and a fourth branch o meet:
+ *   kind R   o is node p's own branch (p = parent[v]); there is no o when p is the root (every entry that involves o is 0)
+ *   kind C   o is keep_w's branch; w's branch keeps its length (in the unrooted tree it is one edge with v's branch)
+ * The five branches c = v, k = keep, x, y, o take t_five[k] = {t_c, t_k, t_x, t_y, t_o} (NULL: every branch at its current length by
+ * node id); every other branch keeps its length.  With M = P L:
+ *   (R)  L_k = sum_c prop_c sum_i pi_i [(P_o U_p) o (P_y L_y)]_i (P_c ((P_k L_k) o (P_x L_x)))_i
+ *   (C)  the far side is P_w ((P_o L_o) o (P_y L_y)), P_w at w's current length
+ * A first derivative replaces one branch's matrix by r_c P', a diagonal second derivative by r_c^2 P", a mixed one puts r_c P' in two
+ * factors; the sums are g_a = sum w L_a / L and H_ab = sum w (L_ab / L - L_a L_b / L^2).  out[k] = {lnL, g_c, g_k, g_x, g_y, g_o, then
+ * the upper triangle of H row by row: cc ck cx cy co kk kx ky ko xx xy xo yy yo oo}, 21 numbers.  The derivatives are the exact ones:
+ * PHB_OPT_INCLUDE_ROOT_FREQS, PHB_OPT_COMPAT_SCALED_GRADIENT and the unrooted zeroing do not apply.  With t_five = NULL, lnL, g_c and
+ * H_cc are those of phb_tlk_nni_scores.  Under rescaling the per-pattern log factor is that of phb_tlk_nni_scores.
+ * Everything else is as phb_tlk_nni_scores: *lnl, PHB_OPT_INCREMENTAL with every partial left resident, the cached lnL unchanged, the
+ * rescaling retry and the NaN fill, the refusals (a negative or NaN length in t_five is PHB_EINVAL), PHB_ESTATE, PHB_ENOMEM.
+ */
+int phb_tlk_nni_quintet_scores(phb_tlk *tlk, int nmoves, const int *moves /* [nmoves][2] */, const double *t_five /* [nmoves][5] or NULL */,
+                               double *lnl, double *out /* [nmoves][21] */);
 
 /*
  * Subtree prune and regraft (the SPR moves the tree-search drivers score, spropt.c:1548-1615).  s is the root of the subtree to prune;

@@ -191,6 +191,12 @@ typedef struct phbc_nni_move {
  * (the 4-state kernel's work items) */
 int phbc_nni_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmoves, const phbc_nni_move *moves, int ngroups, const int *groups,
                     const double *bl, const double *ex, double *out);
+/* NNI quintet scores (phb_nni.cu): out [nmoves][21] = lnL, the gradient in (t_c, t_k, t_x, t_y, t_o) and the upper triangle of the
+ * Hessian, row by row, of each exchanged tree with its five branches at lengths of their own.  moves in launch order, with cmat the first
+ * of five consecutive table entries c, k, x, y, o and out the output row; bl [N + 5 nmoves] the matrix table's lengths, ex (may be NULL)
+ * their exponentials [N + 5 nmoves][C][S]. */
+int phbc_nni_quintet_scores(phbc_ctx *ctx, const phbc_eval_opts *o, int nmoves, const phbc_nni_move *moves, const double *bl, const double *ex,
+                            double *out);
 /* Subtree prune and regraft (phb_spr.cu): out [ntargets][3] = lnL, d lnL/dt_s, d2 lnL/dt_s2 of the subtree of s (p = parent[s])
  * regrafted on the branch above each target node, from the pruned tree's partials the caller left in the resident buffers (U~_e at
  * N + e, L~_e at e); bl [N + ntargets] the matrix table's lengths (node n = entry n, target k's pendant length = entry N + k), ex (may

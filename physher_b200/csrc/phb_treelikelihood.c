@@ -1592,6 +1592,88 @@ static int phb_tlk_nni_scores_impl(phb_tlk *t, int nmoves, const int *moves, con
 }
 
 /*
+ * NNI quintet scores: every move with the central branch c = v and the four around it free -- k = keep and x at v's end, y and o at the
+ * far end (kind R: o is p's own branch, none when p is the root; kind C: o is keep_w's branch, w's branch keeps its length).  The matrix
+ * table holds every node at its current length, then c, k, x, y, o of each move: t_five[5k ..], or the current lengths by node id.  The
+ * descriptors go in the launch order of the NNI scores, by (parent of v, v, x), so that neighbouring moves read the same operands.
+ */
+typedef struct QuintetArgs {
+	int nmoves;
+	const int *moves;
+	const double *t_five;
+} QuintetArgs;
+static int quintet_pass(phb_tlk *t, const void *arg, double *out) {
+	const QuintetArgs *a = (const QuintetArgs *)arg;
+	const int N = t->N, C = t->C, S = t->S, nmoves = a->nmoves;
+	const int *moves = a->moves;
+	int rc = resident_uppers(t, -1, 0);
+	if (rc) return rc;
+	const size_t items = (size_t)N + 5 * (size_t)nmoves;
+	phbc_nni_move *desc = (phbc_nni_move *)malloc(sizeof(phbc_nni_move) * (size_t)nmoves);
+	NniKey *order = (NniKey *)malloc(sizeof(NniKey) * (size_t)nmoves);
+	double *bl = (double *)malloc(sizeof(double) * items);
+	double *ex = wants_host_exp(t) ? (double *)malloc(sizeof(double) * items * C * S) : NULL;
+	if (!desc || !order || !bl || (wants_host_exp(t) && !ex)) {
+		rc = fail(PHB_ENOMEM, "out of memory");
+		goto done;
+	}
+	table_lengths(t, 0, NULL, NULL, 0, bl);
+	for (int k = 0; k < nmoves; k++) {
+		const int x = moves[2 * k], y = moves[2 * k + 1], v = t->parent[y];
+		order[k] = (NniKey){t->parent[v], v, x, k};
+	}
+	qsort(order, (size_t)nmoves, sizeof(NniKey), nni_order);
+	for (int i = 0; i < nmoves; i++) {
+		const int k = order[i].k, x = moves[2 * k], y = moves[2 * k + 1], v = t->parent[y], keep = sibling_of(t, y);
+		phbc_nni_move *m = &desc[i];
+		int o;
+		m->x = x, m->y = y, m->keep = keep;
+		if (nni_kind(t, x, y) == 0) {
+			const int p = t->parent[v];
+			o = p;
+			m->a = p == t->root ? -1 : N + p, m->a_mat = -1, m->w = -1;
+		} else {
+			m->w = t->parent[x];
+			m->a = o = sibling_of(t, x);
+			m->a_mat = -1;
+		}
+		m->cmat = N + 5 * k, m->out = k;
+		const int owner[5] = {v, keep, x, y, o};
+		double *row = bl + N + 5 * (size_t)k;
+		for (int j = 0; j < 5; j++) row[j] = a->t_five ? a->t_five[5 * (size_t)k + j] : (owner[j] == t->root ? 0.0 : t->bl[owner[j]]);
+	}
+	if (ex) host_exponentials(t, items, bl, ex);
+	phbc_eval_opts o;
+	fill_opts_resident(t, &o, 1);
+	if ((rc = phbc_nni_quintet_scores(t->ctx, &o, nmoves, desc, bl, ex, out))) rc = dev_fail(rc);
+done:
+	free(desc), free(order), free(bl), free(ex);
+	return rc;
+}
+
+/* lnL, gradient and Hessian in the five branches of every listed NNI neighbour from resident partials (phb_nni.cu); the checks of the
+ * NNI scores, plus the state-count limit of the node-at-a-time kernels for every S */
+static int phb_tlk_nni_quintet_scores_impl(phb_tlk *t, int nmoves, const int *moves, const double *t_five, double *lnl, double *out) {
+	if (!moves || !out) return fail(PHB_EINVAL, "nni_quintet_scores: moves and out are required");
+	if (nmoves < 1) return fail(PHB_EINVAL, "nni_quintet_scores: %d moves (at least one is needed)", nmoves);
+	for (int k = 0; k < nmoves; k++) {
+		if (nni_kind(t, moves[2 * k], moves[2 * k + 1]) < 0)
+			return fail(PHB_EINVAL, "nni_quintet_scores: move %d (%d, %d) is not a nearest-neighbour interchange of the current tree", k,
+			            moves[2 * k], moves[2 * k + 1]);
+		for (int j = 0; t_five && j < 5; j++)
+			if (!(t_five[5 * (size_t)k + j] >= 0))
+				return fail(PHB_EINVAL, "nni_quintet_scores: move %d branch length %d = %E", k, j, t_five[5 * (size_t)k + j]);
+	}
+	if (t->have_matrices)
+		return fail(PHB_ESTATE, "nni_quintet_scores needs the eigen system: explicit matrices cannot be re-evaluated at a new length");
+	int rc = check_ready(t);
+	if (rc) return rc;
+	if ((rc = phbc_smem_check(t->ctx, "nni_quintet_scores", 2))) return dev_fail(rc);
+	const QuintetArgs a = {nmoves, moves, t_five};
+	return resident_scores(t, nmoves, 21, lnl, out, quintet_pass, &a);
+}
+
+/*
  * Subtree prune and regraft (spropt.c:1548-1615): the subtree of s is pruned together with p = parent[s] -- the sibling b of s takes
  * p's slot under g = parent[p] -- and regrafted on the branch above a target e of the pruned tree: p takes e's slot, e the slot of p
  * that is not s's.  s may be neither the root nor a child of the root; a target is any node outside the subtree of s other than p and
@@ -2484,6 +2566,13 @@ int phb_tlk_nni_moves(phb_tlk *t, int *moves) { return phb_tlk_nni_moves_impl(t,
 int phb_tlk_nni_scores(phb_tlk *t, int nmoves, const int *moves, const double *t_central, double *lnl, double *out) {
 	nvtxRangePushA("phb_tlk_nni_scores");
 	const int rc = phb_tlk_nni_scores_impl(t, nmoves, moves, t_central, lnl, out);
+	nvtxRangePop();
+	return rc;
+}
+
+int phb_tlk_nni_quintet_scores(phb_tlk *t, int nmoves, const int *moves, const double *t_five, double *lnl, double *out) {
+	nvtxRangePushA("phb_tlk_nni_quintet_scores");
+	const int rc = phb_tlk_nni_quintet_scores_impl(t, nmoves, moves, t_five, lnl, out);
 	nvtxRangePop();
 	return rc;
 }

@@ -76,6 +76,7 @@ SYMBOLS = [
     ("phb_tlk_spr_targets", C.c_int, [C.c_void_p, C.c_int, _ip]),
     ("phb_tlk_spr_scores", C.c_int, [C.c_void_p, C.c_int, C.c_int, _ip, _dp, _dp, _dp]),
     ("phb_tlk_spr_tripod_scores", C.c_int, [C.c_void_p, C.c_int, C.c_int, _ip, _dp, _dp, _dp, _dp]),
+    ("phb_tlk_nni_quintet_scores", C.c_int, [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp]),
     ("phb_tlk_update_partials", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _dp]),
     ("phb_tlk_get_partials", C.c_int, [C.c_void_p, C.c_int, _dp]),
     ("phb_tlk_get_matrices", C.c_int, [C.c_void_p, _dp, _dp]),
@@ -491,6 +492,24 @@ class SingleTreeLikelihood:
         self._check(self.lib.phb_tlk_nni_scores(self.h, int(m.shape[0]), m.ctypes.data_as(_ip), None if tc is None else tc.ctypes.data_as(_dp),
                                                 C.byref(lnl), out.ctypes.data_as(_dp)))
         return lnl.value, out
+
+    def nni_quintet_scores(self, moves=None, t_five=None):
+        """lnL, gradient and Hessian in (t_c, t_k, t_x, t_y, t_o) -- the central branch, keep and x at v's end, y and the fourth branch o
+        at the far end -- of the tree each move (x, y) produces, the five at t_five[k] (None: their current lengths by node id), in one
+        call on resident partials (see phb_tlk_nni_quintet_scores): (lnl[n] of each exchanged tree, grad[n, 5], hess[n, 5, 5]);
+        calculate() gives the current tree's.  moves=None scores the whole neighbourhood, nni_moves()."""
+        m = self.nni_moves() if moves is None else np.ascontiguousarray(moves, dtype=np.int32).reshape(-1, 2)
+        tf = None if t_five is None else np.ascontiguousarray(t_five, dtype=np.float64).reshape(-1)
+        if tf is not None and tf.shape[0] != 5 * m.shape[0]:
+            raise ValueError("t_five needs five lengths per move")
+        out = np.zeros((m.shape[0], 21))
+        self._check(self.lib.phb_tlk_nni_quintet_scores(self.h, int(m.shape[0]), m.ctypes.data_as(_ip),
+                                                        None if tf is None else tf.ctypes.data_as(_dp), None, out.ctypes.data_as(_dp)))
+        iu = np.triu_indices(5)
+        hess = np.zeros((m.shape[0], 5, 5))
+        hess[:, iu[0], iu[1]] = out[:, 6:]
+        hess[:, iu[1], iu[0]] = out[:, 6:]
+        return out[:, 0].copy(), out[:, 1:6].copy(), hess
 
     def spr_targets(self, s):
         """The regraft targets of the subtree of s, int32 [n] (see phb_tlk_spr_targets; PHB_OPT_UNROOTED decides whether targets that
